@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload c2|c3|c4|c1|c5b8..c5b64] [--mode parity|econ8|econ|fast|mixed|fp32] [--c5]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic RGB-D: the whole focal stack
 [N,3,S,H,W] of the workload, in ONE kernel launch.  Metric: Mpix*slices/s = N*S*H*W / t / 1e6
@@ -19,6 +20,12 @@ sharding.render_stack_sharded (tile-row partition), checked bit-for-bit against 
 `--impl reference` runs the UNMODIFIED reference (baseline/_ref, see baseline/make_ref.py) through its own
 public API, PSFNet.render, on the host CPU: same metric, workload and inputs; nothing of this repo's
 product is imported by that arm.  Prints ONE JSON line (rank 0).
+
+`--dump-outputs DIR` writes the focal stack of the last timed step as DIR/render_stack.npy (float32, [N,3,S,H,W]) so
+that two builds run with the same arguments (hence the same seeded inputs) can be compared element for element.  A
+stack larger than 64 MB is replaced by a fixed, seeded sample of its elements: render_stack.npy holds the values and
+render_stack_index.npy (float64) their flat indices.  Under torchrun every rank writes render_stack_rank<r>*.npy of
+its own stack within 64 MB / ranks.
 """
 import argparse
 import json
@@ -65,6 +72,23 @@ MODE_ACCURACY = {
     "econ": "max-abs vs the reference's goldens 3.1e-5 / 3.4e-5 / 2.2e-6, tested at 6e-5; worst case over a hand-built image 2.0e-4 (not certified)",
     "mixed": "2.2e-4 on the goldens (reduced precision)", "fast": "6e-3 max / 6e-5 mean on the goldens (reduced precision)",
     "fp32": "1.3e-6 on the goldens (CUDA cores, operation-exact)"}
+
+
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs: all files of all ranks together
+
+
+def dump_output(out, path, name, budget):
+    """out -> path/<name>.npy (float32).  Over `budget` bytes: a sample of elements at seeded random flat indices
+    (sorted, repeats possible), written with those indices as path/<name>_index.npy (float64, exact below 2^53)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = out.detach()
+    room = budget - 4096                                   # .npy headers
+    if out.numel() * 4 > room:
+        idx = torch.randint(out.numel(), (room // (4 + 8),), generator=torch.Generator().manual_seed(0)).sort().values
+        np.save(os.path.join(path, f"{name}_index.npy"), idx.double().numpy())
+        out = out.reshape(-1)[idx.to(out.device)]
+    np.save(os.path.join(path, f"{name}.npy"), out.float().cpu().numpy())
 
 
 def flops_per_pixel(ks):
@@ -204,6 +228,7 @@ def reference_renderer(name, device):
         return (lambda img, depth, foc: lens.render(img, depth, foc)), "reference"
     from oracle import focal_stack_oracle as orc
     Ws, bs = weights_for(ks, product=False)
+    Ws, bs = [w.to(device) for w in Ws], [b.to(device) for b in bs]
     return (lambda img, depth, foc: orc.render_reference_ops(Ws, bs, img, depth, foc, ks)), "port"
 
 
@@ -526,6 +551,9 @@ def run_ours(args):
     t_wall1 = time.perf_counter()
     launches = nat.lib.aadff_launch_count() - launches0 - args.warmup
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs:
+        dump_output(out, args.dump_outputs, "render_stack" if world == 1 else f"render_stack_rank{rank}",
+                    DUMP_BYTES // world)
     total_ms = torch.tensor([sum(times)], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -665,7 +693,13 @@ def main():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--c5", default="", help="comma-separated batch sizes of the end-to-end AiF training step, e.g. 8,16,32,64")
     ap.add_argument("--ref-device", default="cpu", choices=["cpu", "cuda"], help="reference arm only (cuda = eager baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the focal stack of the last timed step to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

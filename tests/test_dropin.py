@@ -1,4 +1,5 @@
-"""The drop-in boundary, driven the way the reference's own scripts drive it (CPU; needs /root/reference).
+"""The drop-in boundary, driven the way the reference's own scripts drive it (CPU; needs a checkout of the reference,
+singer-yang/Aberration-Aware-Depth-from-Focus, named by the environment variable AADFF_REFERENCE).
 
 Two integration modes (INTEGRATION.md):
   shadow  -- this repo's site directory in front of the reference checkout on sys.path: the import block of
@@ -18,9 +19,9 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHADOW = os.path.join(ROOT, "aberration-aware-depth-from-focus_b200")
-REF = "/root/reference"
+REF = os.environ.get("AADFF_REFERENCE", "")
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout only exists in the build container")
+pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="needs a reference checkout (set AADFF_REFERENCE)")
 
 STUBS = textwrap.dedent("""
     import sys, types
@@ -37,7 +38,8 @@ STUBS = textwrap.dedent("""
 
 
 def run_child(body, path):
-    code = STUBS + f"\nimport os\nos.chdir({REF!r})\nsys.path[:0] = {path!r}\n" + textwrap.dedent(body)
+    code = STUBS + f"\nimport os\nos.chdir({REF!r})\nREF_ROOT = os.path.realpath({REF!r}) + os.sep\nsys.path[:0] = {path!r}\n" + \
+        textwrap.dedent(body)
     env = dict(os.environ, PYTHONPATH="")
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, timeout=600)
     assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
@@ -53,10 +55,10 @@ def test_shadow_runs_the_training_scripts_import_block_and_get_lens():
         from dff import *
         import deeplens, dff, deeplens.utils, deeplens.psfnet, dff.utils, dff.AiFNet, dff.dataset
         here = lambda m: os.path.realpath(m.__file__)
-        assert here(deeplens.utils).startswith('/root/reference/'), here(deeplens.utils)
-        assert here(dff.AiFNet).startswith('/root/reference/') and here(dff.dataset).startswith('/root/reference/')
-        assert not here(deeplens.psfnet).startswith('/root/reference/')
-        assert not here(dff.utils).startswith('/root/reference/')
+        assert here(deeplens.utils).startswith(REF_ROOT), here(deeplens.utils)
+        assert here(dff.AiFNet).startswith(REF_ROOT) and here(dff.dataset).startswith(REF_ROOT)
+        assert not here(deeplens.psfnet).startswith(REF_ROOT)
+        assert not here(dff.utils).startswith(REF_ROOT)
         assert PSFNet.__module__ == 'aadff_lens' and ThinLens.__module__ == 'aadff_lens'
         assert select_focus_dist.__module__ == 'aadff_focus' and get_lens.__module__ == 'aadff_factory'
         AiFDepthNet, get_dataset, Middlebury, mask_mae, local_psf_render          # names the scripts use
@@ -94,7 +96,7 @@ def test_install_patches_an_already_imported_reference():
         import deeplens.render_psf
         ref_render = sys.modules['deeplens.render_psf']   # (the attribute deeplens.render_psf is a function there)
         import dff.utils as ref_dff_utils
-        assert os.path.realpath(ref_psfnet.__file__).startswith('/root/reference/')
+        assert os.path.realpath(ref_psfnet.__file__).startswith(REF_ROOT)
         ref_render_fn, ref_gather, ref_select = ref_psfnet.PSFNet.render, ref_render.local_psf_render, ref_dff_utils.select_focus_dist
         sys.path.insert(0, %r)
         import aadff_b200

@@ -237,6 +237,27 @@ def test_sharded_render_gathers_to_single_rank_result_gloo(tmp_path):
         assert "ok" in o
 
 
+def test_bench_dump_outputs_whole_or_seeded_sample(tmp_path):
+    """bench.py --dump-outputs: a stack within the budget is written whole, a larger one as the same seeded sample of
+    values + flat indices on every run, all files together within the budget."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    out = torch.rand(2, 3, 5, 40, 56, generator=torch.Generator().manual_seed(1))
+    bench.dump_output(out, str(tmp_path / "whole"), "render_stack", bench.DUMP_BYTES)
+    whole = np.load(tmp_path / "whole" / "render_stack.npy")
+    assert whole.dtype == np.float32 and np.array_equal(whole, out.numpy())
+    budget = 40000
+    for run in ("a", "b"):
+        bench.dump_output(out, str(tmp_path / run), "render_stack", budget)
+        assert sum(f.stat().st_size for f in (tmp_path / run).iterdir()) <= budget
+    vals, idx = np.load(tmp_path / "a" / "render_stack.npy"), np.load(tmp_path / "a" / "render_stack_index.npy")
+    assert vals.dtype == np.float32 and idx.dtype == np.float64 and len(vals) == len(idx) > 1000
+    assert np.array_equal(vals, out.numpy().reshape(-1)[idx.astype(np.int64)])
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "render_stack_index.npy"))
+
+
 def test_bench_reference_arm_prints_contract_line():
     """`bench.py --impl reference` (the CPU arm) must emit one JSON line with the contract keys."""
     import json
