@@ -552,6 +552,10 @@ int aadff_psfnet_create(const float* const* weights, const float* const* biases,
 #undef AADFF_SET_ATTR
         CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 14>, attr, so));      // econ8: no cluster variant
         CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, true, 14>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<true, false, 0, false, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 12, false, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 13, false, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 14, false, true>, attr, so));
     }
 #undef CREATE_TRY
     *out = h;
@@ -763,6 +767,32 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     // 2-CTA clusters sharing the weight stream by multicast (fused_tc_kernel.cuh, CL2).  Built, bit-exact, and measured
     // NOT to pay (profiles/NOTES_r02.md: -7 % at c2, +-1 % where power-capped), so it is off unless debug flag 8 asks for it.
     const bool cl2 = P.probes == nullptr && P.trace == nullptr && uni != 0 && uni != 14 && (P.dbg & 8u) && h->num_sms >= 2;
+    // A operands in tensor memory (fused_tc_kernel.cuh, TA): render launches of the 2-/3-term specialisations with one
+    // head block of N <= 192 (ks <= 13) and at least two hidden layers, 4-stage ring.  Its shared memory holds no
+    // activations: ring, raw head values of the tile being gathered, two halo slots.  Debug flag 1 << 20 keeps such
+    // launches on the shared-memory path (equality tests, A/B timing).
+    bool all2 = true;
+    for (int i = 0; i < h->n_groups; ++i) all2 &= (P.g[i].terms >= 2);
+    const uint32_t head_n = h->groups[h->n_hidden].N;
+    uint32_t smem_launch = smem;
+    const bool ta = P.probes == nullptr && !cl2 && !(P.dbg & (1u << 20)) && h->n_groups == h->n_hidden + 1 &&
+                    h->n_hidden >= 2 && head_n <= (uint32_t)TC_TA_L1_COL && P.kslab == 1 && P.n_stages == 4 && all2 &&
+                    (uni == 12 || uni == 13 || uni == 14 || P.trace != nullptr);
+    if (ta) {
+        const uint32_t stg_bytes = ((head_n + 31u) & ~31u) * TC_M * 4;      // the gather reads 32-column blocks
+        P.halo_bytes = halo_bytes;
+        P.off_stage = 0;
+        P.off_stg = 4 * TC_STAGE_BYTES;
+        P.off_bias = P.off_stg + stg_bytes;
+        P.off_w0 = P.off_bias + bias_bytes;
+        P.off_halo = (P.off_w0 + 320 * 4 + 15u) & ~15u;
+        P.off_red = P.off_halo + 2 * halo_bytes;
+        P.off_bar = P.off_red + TC_M * 5 * 4;
+        P.off_ones = (P.off_bar + TC_BAR_BYTES + 15u) & ~15u;
+        P.off_bslab = P.off_ones + ones_bytes;
+        smem_launch = P.off_bslab + bslab_bytes;
+        if (smem_launch > (uint32_t)h->smem_optin) return fail(AADFF_E_UNSUPPORTED, "shared memory budget exceeded (TA)");
+    }
     if (cl2) {
         grid = (int)std::min<long long>((P.n_tiles + 1) & ~1ll, (long long)(h->num_sms & ~1));
         cudaLaunchConfig_t cfg{};
@@ -785,7 +815,14 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
         }
         if (le != cudaSuccess) return fail(AADFF_E_CUDA, std::string("cluster launch: ") + cudaGetErrorString(le));
     } else if (P.trace != nullptr && P.probes == nullptr) {
-        fused_psfnet_render_kernel<true, false, 0><<<grid, TC_NT, smem, st>>>(P);
+        if (ta) fused_psfnet_render_kernel<true, false, 0, false, true><<<grid, TC_NT, smem_launch, st>>>(P);
+        else fused_psfnet_render_kernel<true, false, 0><<<grid, TC_NT, smem, st>>>(P);
+    } else if (ta) {
+        switch (uni) {
+            case 12: fused_psfnet_render_kernel<false, false, 12, false, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
+            case 13: fused_psfnet_render_kernel<false, false, 13, false, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
+            default: fused_psfnet_render_kernel<false, false, 14, false, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
+        }
     } else {
 #define AADFF_LAUNCH(U)                                                                                   \
         case U:                                                                                           \

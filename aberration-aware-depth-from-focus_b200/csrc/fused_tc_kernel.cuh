@@ -61,6 +61,11 @@ constexpr int TC_MIXED_FIRST_GROUP = 3;  // mixed: groups 0..2 (L1..L3) three te
 constexpr int TC_ECON_FIRST_GROUP = 4;   // econ: groups 0..3 (L1..L4) three terms, L5.. and the head two (econ_calib.h)
 constexpr int TC_ECON8_FIRST_GROUP = 7;  // econ8: groups 0..6 (L1..L7) three terms, L8, L9 and the head two -- the earliest
                                          // start whose adversarial worst case stays under 1e-4 (DESIGN.md section 5)
+// TA (A operands in tensor memory): L1's A (K = 64) is written by layer 0 into the last 64 columns of the head's
+// accumulator buffer, behind the head's N <= 192 columns; its hand-off uses a_ready barriers 5 and 6, which the 3-term
+// barrier map leaves unused, so that layer 0 of the next tile may arrive before the head has consumed barriers 0 and 1
+constexpr int TC_TA_L1_COL = TC_HID - 64;
+constexpr int TC_TA_L1_BAR = 5;
 
 struct TcGroup {            // one accumulation group: one layer, or one <=256-column block of the head
     uint32_t w_off;         // byte offset of its first slab in the packed weights
@@ -90,6 +95,8 @@ struct TcParams {
     // shared-memory byte offsets
     uint32_t off_stage, off_bias, off_w0, off_halo, off_red, off_bar, off_ones;
     uint32_t off_bslab;     // bias-slab slot: [256 x 8] halves (K columns 0..7) + a shared [256 x 8] block of zeros (K 8..15)
+    uint32_t off_stg;       // TA: raw head accumulator of the tile being gathered, [head columns / 4][128 rows] float4
+    uint32_t halo_bytes;    // TA: one of the two halo slots (tile t is gathered while tile t+1's halo is fetched)
     uint32_t dbg;           // what-if timing switches (results invalid): 1 = no weight copies, 2 = no A stores
     // pred mode (kernel instantiated with PRED = true): probes [M,4] in, L1-normalised PSFs [M, ks*ks] out
     const float* probes;
@@ -185,6 +192,32 @@ __device__ __forceinline__ void epi_group8(const uint32_t* acc, uint32_t a_hi, u
     st_shared_v4(a_lo + off, l[0], l[1], l[2], l[3]);
 }
 
+// TA: one K=16 step of a tensor-memory A operand, written over the 16 accumulator columns it was made from:
+// 8 columns of fp16x2 hi, then 8 of lo (the same conversions as epi_group8 with need_lo)
+__device__ __forceinline__ void epi_ta16(const uint32_t* acc, uint32_t taddr) {
+    uint32_t o[16];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+        const float a0 = __uint_as_float(acc[2 * u]), a1 = __uint_as_float(acc[2 * u + 1]);
+        o[u] = pack_half2_relu_rz(a0, a1);
+        const float2 f = __half22float2(*reinterpret_cast<__half2*>(&o[u]));
+        o[8 + u] = pack_half2_relu(a0 - f.x, a1 - f.y);
+    }
+    tmem_st16(taddr, o);
+}
+
+// TA: the same for 16 fp32 values from registers (layer 0; the conversions of store_split8 with need_lo)
+__device__ __forceinline__ void split_ta16(const float (&v)[16], uint32_t taddr) {
+    uint32_t o[16];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+        o[u] = pack_half2(v[2 * u], v[2 * u + 1]);
+        const float2 f = __half22float2(*reinterpret_cast<__half2*>(&o[u]));
+        o[8 + u] = pack_half2(v[2 * u] - f.x, v[2 * u + 1] - f.y);
+    }
+    tmem_st16(taddr, o);
+}
+
 // Warp roles.  The hardware warp arbiter favours the HIGHEST warp id on a scheduler, so the two
 // single-thread roles that must react quickly (weight producer, MMA issuer) are the LAST warps of
 // the CTA; with low ids they were starved by the ALU-heavy epilogue warps sharing their scheduler
@@ -205,9 +238,18 @@ constexpr int TC_WARP_MMA = TC_EPI_WARPS + 1;        // warp 9
 // refilled only after BOTH CTAs' MMAs have released it (the release commits are multicast too, the "empty" barriers
 // count two arrivals).  Everything else -- activations, accumulators, MMAs, epilogue -- stays per CTA.  Both CTAs of a
 // pair run the same number of tile iterations; the one without a tile left computes a dummy tile and stores nothing.
-template <bool TRACE, bool PRED, int UNI, bool CL2 = false>
+//
+// TA: the activations never touch shared memory.  Each layer's epilogue turns its accumulator into the next layer's A
+// operand in the same TMEM columns (epi_ta16), and the MMAs read A from tensor memory.  A group's A therefore lives in
+// the other accumulator buffer, so before a group's first MMA the MMA warp also waits for the previous group's
+// accumulator: every MMA that read the A in its destination buffer has retired.  Layer 0 of tile t+1 runs under tile
+// t's head MMAs, and tile t's head values are copied raw to shared memory (off_stg) so that its sigmoid / gather runs
+// after tile t+1's L1 epilogue, under L2's MMAs.  Render kernels with one head block of N <= 192, at least two hidden
+// layers and only 2-/3-term groups (host-checked).
+template <bool TRACE, bool PRED, int UNI, bool CL2 = false, bool TA = false>
 __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __grid_constant__ TcParams P) {
     static_assert(!(CL2 && (PRED || TRACE)), "the cluster variant exists for the render kernels only");
+    static_assert(!(TA && (CL2 || PRED)), "tensor-memory A operands exist for the one-CTA render kernels only");
     constexpr int UM = UNI % 10;
     const uint32_t cta_rank = CL2 ? cluster_ctarank() : 0u;
     // tile iterations of this CTA: with CL2 both CTAs of a pair take the count of the even one
@@ -256,7 +298,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
             // 3-term modes: barrier 0, 1 = 32-column chunks 0, 1 (all 8 warps, 16-column steps); barrier 2 = chunks
             // 2+3 and barrier 4 = chunks 4..7 (the MMA warp is slower than the epilogue by then, so it only
             // checks at K-steps 0, 1, 2 and 4: every spared wait is ~90 cycles of idle tensor pipe)
-            mbar_init(bar_aready(j), (kslab_c == 2 || j < 4) ? TC_EPI_WARPS : 2 * TC_EPI_WARPS);
+            mbar_init(bar_aready(j), (kslab_c == 2 || j < 4 || (TA && (j == TC_TA_L1_BAR || j == TC_TA_L1_BAR + 1)))
+                                         ? TC_EPI_WARPS : 2 * TC_EPI_WARPS);
         for (int b = 0; b < 2; ++b) { mbar_init(bar_accfull(b), 1); mbar_init(bar_accfree(b), TC_EPI_WARPS); }
         mbar_init(bar_bfull(), 1);
         mbar_init(bar_bempty(), 1);
@@ -352,6 +395,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
         int stage = 0;
         uint32_t fbits = 0, aphase = 0, frphase = 0;      // bit s / j / b = parity to wait for next on that barrier
         uint32_t bphase = 0;                               // bias-slab slot
+        uint32_t afbits = 0;                               // TA: bit b = parity of accfull(b) to wait for next
         uint32_t gcount = 0;
         TcTrace<TRACE> tr; tr.init(lane == 0 ? P.trace : nullptr, 1);
         // descriptors: everything but the 14-bit start-address field (16-byte units) is loop invariant
@@ -377,9 +421,16 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     mbar_wait(bar_accfree(buf), (frphase >> buf) & 1);
                     frphase ^= 1u << buf;
                 }
+                if (TA && gcount >= 1) {     // write-after-read: the MMAs of group gcount-1 read their A from buffer `buf`
+                    mbar_wait(bar_accfull(buf ^ 1), (afbits >> (buf ^ 1)) & 1);
+                    afbits ^= 1u << (buf ^ 1);
+                }
                 tc_fence_after_sync();
                 tr.ev(0x200 + gi);                               // group start (accumulator free)
                 const uint32_t d_tmem = tmem_base + buf * 256;
+                // TA: this group's A = the previous group's accumulator, converted in place (L1: layer 0's, see TC_TA_L1_COL)
+                const uint32_t a_tmem = tmem_base + (buf ^ 1) * 256 + (gi == 0 ? TC_TA_L1_COL : 0);
+                const int abar0 = (TA && gi == 0) ? TC_TA_L1_BAR : 0;
                 const uint32_t idesc = umma_idesc_f16_f32(TC_M, gN);
                 const uint32_t kstep_b = (2 * gN * 16) >> 4;     // one K=16 step of B: 2 * LBO_B
                 const uint64_t db0 = umma_smem_desc(stage0, gN * 16, 128);
@@ -409,6 +460,11 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     const int kc = it * kslab;                   // first K=32 slab of this step
                     const uint64_t ah = da_hi + (uint32_t)kc * (2 * KSTEP_A);
                     const uint64_t al = da_lo + (uint32_t)kc * (2 * KSTEP_A);
+                    // one MMA with the hi (lo = false) or lo part of A's K=16 step k16 of this slab
+                    auto mma_a = [&](bool lo, int k16, uint64_t b, uint32_t acc) {
+                        if constexpr (TA) umma_f16_ts(d_tmem, a_tmem + (uint32_t)(kc * 32 + k16 * 16 + (lo ? 8 : 0)), b, idesc, acc);
+                        else umma_f16_ss(d_tmem, (lo ? al : ah) + (uint32_t)k16 * KSTEP_A, b, idesc, acc);
+                    };
                     if (ALIGNED) stage = (three ? 2 * it : it) & 3;   // groups start at ring position 0 (host-checked)
                     if (!pre_waited) {
                         tr.ev(0x500 + kc);
@@ -416,8 +472,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                         tr.ev(0x600 + kc);
                         // A chunk: 64 columns per barrier in fast mode; barriers 0, 1, 2 (= chunks 2+3), 4 (= 4..7) else
                         if (new_a && (kslab == 2 || it < 3 || it == 4)) {
-                            mbar_wait(bar_aready(it), (aphase >> it) & 1);
-                            aphase ^= 1u << it;
+                            mbar_wait(bar_aready(abar0 + it), (aphase >> (abar0 + it)) & 1);
+                            aphase ^= 1u << (abar0 + it);
                             tr.ev(0x400 + kc);
                         }
                     }
@@ -432,10 +488,10 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                         const bool merged = three && (ALIGNED || P.n_stages >= 4);       // lo bytes arrived with the pair barrier
                         if (elect_one_sync()) {
                             const uint64_t db = (db0 & ~0x3FFFull) | ((stage_addr(hi_stage) & 0x3FFFFu) >> 4);
-                            umma_f16_ss(d_tmem, ah, db, idesc, has_bias || it != 0);
-                            umma_f16_ss(d_tmem, ah + KSTEP_A, db + kstep_b, idesc, 1);
-                            umma_f16_ss(d_tmem, al, db, idesc, 1);
-                            umma_f16_ss(d_tmem, al + KSTEP_A, db + kstep_b, idesc, 1);
+                            mma_a(false, 0, db, has_bias || it != 0);
+                            mma_a(false, 1, db + kstep_b, 1);
+                            mma_a(true, 0, db, 1);
+                            mma_a(true, 1, db + kstep_b, 1);
                             if (!three) {
                                 if (last) umma_commit(bar_accfull(buf));
                                 release(bar_empty(hi_stage));
@@ -443,8 +499,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                                 release(bar_empty(hi_stage));           // release the hi stage early (64 KB ring)
                                 if (merged) {
                                     const uint64_t dl = (db0 & ~0x3FFFull) | ((stage_addr(stage) & 0x3FFFFu) >> 4);
-                                    umma_f16_ss(d_tmem, ah, dl, idesc, 1);              // Ah*Wl
-                                    umma_f16_ss(d_tmem, ah + KSTEP_A, dl + kstep_b, idesc, 1);
+                                    mma_a(false, 0, dl, 1);              // Ah*Wl
+                                    mma_a(false, 1, dl + kstep_b, 1);
                                     if (last) umma_commit(bar_accfull(buf));
                                     release(bar_empty(stage));
                                 }
@@ -459,8 +515,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                                 tc_fence_after_sync();
                                 if (elect_one_sync()) {
                                     const uint64_t dl = (db0 & ~0x3FFFull) | ((stage_addr(stage) & 0x3FFFFu) >> 4);
-                                    umma_f16_ss(d_tmem, ah, dl, idesc, 1);
-                                    umma_f16_ss(d_tmem, ah + KSTEP_A, dl + kstep_b, idesc, 1);
+                                    mma_a(false, 0, dl, 1);
+                                    mma_a(false, 1, dl + kstep_b, 1);
                                     if (last) umma_commit(bar_accfull(buf));
                                     release(bar_empty(stage));
                                 }
@@ -473,11 +529,11 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     // ---- 1-term groups (fast / the tail of mixed)
                     if (elect_one_sync()) {
                         const uint64_t db = (db0 & ~0x3FFFull) | ((stage_addr(hi_stage) & 0x3FFFFu) >> 4);
-                        umma_f16_ss(d_tmem, ah, db, idesc, has_bias || it != 0);
-                        umma_f16_ss(d_tmem, ah + KSTEP_A, db + kstep_b, idesc, 1);
+                        mma_a(false, 0, db, has_bias || it != 0);
+                        mma_a(false, 1, db + kstep_b, 1);
                         if (kslab == 2) {
-                            umma_f16_ss(d_tmem, ah + 2 * KSTEP_A, db + STAGE_STEP, idesc, 1);
-                            umma_f16_ss(d_tmem, ah + 3 * KSTEP_A, db + STAGE_STEP + kstep_b, idesc, 1);
+                            mma_a(false, 2, db + STAGE_STEP, 1);
+                            mma_a(false, 3, db + STAGE_STEP + kstep_b, 1);
                         }
                     }
                     __syncwarp();
@@ -488,8 +544,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                         tr.ev(0x500 + kc + kslab);
                         { mbar_wait(bar_full(stage), (fbits >> stage) & 1); fbits ^= 1u << stage; }
                         if (new_a && (kslab == 2 || it + 1 < 3 || it + 1 == 4)) {     // same barrier map as above
-                            mbar_wait(bar_aready(it + 1), (aphase >> (it + 1)) & 1);
-                            aphase ^= 1u << (it + 1);
+                            mbar_wait(bar_aready(abar0 + it + 1), (aphase >> (abar0 + it + 1)) & 1);
+                            aphase ^= 1u << (abar0 + it + 1);
                         }
                         tr.ev(0x400 + kc + kslab);
                         pre_waited = true;
@@ -569,7 +625,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
         // ---- layer 0 (4 -> 64) in fp32 for tile `t`: (x, y, z, foc_z) -> 64 features -> A operand of L1.
         //      Runs one tile AHEAD: right after the previous tile's last head block has retired (the A buffer is
         //      free again) and BEFORE that tile's gather, so the L1 MMAs of tile t overlap the gather of tile t-1.
-        auto layer0 = [&](long long t) {
+        //      TA: L1's A goes to columns [TC_TA_L1_COL, +64) of accumulator buffer `ta_buf` (the previous tile's head).
+        auto layer0 = [&](long long t, uint32_t ta_buf) {
             float x, y, z, fz;
             if constexpr (PRED) {
                 x = nx_in.x; y = nx_in.y; z = nx_in.z; fz = nx_in.w;
@@ -580,6 +637,28 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                 y = coord_y(min(h0 + ty, ra.H - 1), ra.H, ra.step_y);
                 z = depth_to_z(nx_depth, ra.d_min, ra.d_range);
                 fz = depth_to_z(nx_foc, ra.d_min, ra.d_range);
+            }
+            if constexpr (TA) {
+                // K=16 steps hh and 2 + hh of L1's A: the features of the fine shared-memory hand-off below
+#pragma unroll
+                for (int st = 0; st < 2; ++st) {
+                    const int k16 = 2 * st + hh;
+                    float v[16];
+#pragma unroll
+                    for (int u = 0; u < 16; ++u) {
+                        const int f = k16 * 16 + u;
+                        const float4 wv = *reinterpret_cast<const float4*>(s_w0 + f * 4);
+                        float a = s_w0[256 + f];
+                        a = fmaf(wv.x, x, a); a = fmaf(wv.y, y, a); a = fmaf(wv.z, z, a); a = fmaf(wv.w, fz, a);
+                        v[u] = fmaxf(a, 0.f);
+                    }
+                    split_ta16(v, t_lane + ta_buf * 256 + TC_TA_L1_COL + k16 * 16);
+                }
+                tmem_st_wait();
+                tc_fence_before_sync();
+                __syncwarp();
+                if (lane == 0) { mbar_arrive(bar_aready(TC_TA_L1_BAR)); mbar_arrive(bar_aready(TC_TA_L1_BAR + 1)); }
+                return;
             }
             const bool need_lo = terms_of(0) >= 2;
 #pragma unroll
@@ -606,7 +685,87 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                 else mbar_arrive(bar_aready(0));
             }
         };
-        if (my_iters > 0) layer0(blockIdx.x);
+        if (my_iters > 0) layer0(blockIdx.x, 1u);
+
+        // ---- 32 head columns of this thread's pixel, taps tap_first.. (bias_c: their -log2(e) * bias): sigmoid, gather
+        //      from the halo tile (render_psf.py:103-105), accumulated into ssum / cacc
+        auto gather32 = [&](const uint32_t (&rr)[32], int tap_first, const float* bias_c, const float4* hbase, float& ssum,
+                            float (&cacc)[TC_MAX_C]) {
+            int i = tap_first / ks, j = tap_first - i * ks;
+            int off = i * TC_HALO_PITCH + j;
+            const int nvalid = kk - tap_first;     // >= 32 for every group but the padded last one
+            if (nvalid >= 32) {
+                // branch-free so that the MUFU / LDS latencies of different taps overlap
+#pragma unroll
+                for (int u = 0; u < 32; ++u) {
+                    const float sg = rcp_approx(1.0f + ex2_approx(fmaf(__uint_as_float(rr[u]), NEG_LOG2E, bias_c[u])));
+                    const float4 px = hbase[off];
+                    ssum += sg;
+                    cacc[0] = fmaf(sg, px.x, cacc[0]);
+                    cacc[1] = fmaf(sg, px.y, cacc[1]);
+                    cacc[2] = fmaf(sg, px.z, cacc[2]);
+                    cacc[3] = fmaf(sg, px.w, cacc[3]);
+                    ++off;
+                    if (++j == ks) { j = 0; off += TC_HALO_PITCH - ks; }
+                }
+            } else {
+#pragma unroll
+                for (int u = 0; u < 32; ++u) {
+                    const bool ok = u < nvalid;    // padding columns contribute nothing and read slot 0
+                    float sg = rcp_approx(1.0f + ex2_approx(fmaf(__uint_as_float(rr[u]), NEG_LOG2E, bias_c[u])));
+                    sg = ok ? sg : 0.f;
+                    const float4 px = hbase[ok ? off : 0];
+                    ssum += sg;
+                    cacc[0] = fmaf(sg, px.x, cacc[0]);
+                    cacc[1] = fmaf(sg, px.y, cacc[1]);
+                    cacc[2] = fmaf(sg, px.z, cacc[2]);
+                    cacc[3] = fmaf(sg, px.w, cacc[3]);
+                    ++off;
+                    if (++j == ks) { j = 0; off += TC_HALO_PITCH - ks; }
+                }
+            }
+        };
+        // ---- combine the two column-halves of each pixel, normalise (F.normalize p=1), store
+        auto store_px = [&](float ssum, const float (&cacc)[TC_MAX_C], int n, int s, int h, int w, bool valid) {
+            if (hh == 1) {
+                s_red[row * 5 + 0] = ssum;
+#pragma unroll
+                for (int c = 0; c < TC_MAX_C; ++c) s_red[row * 5 + 1 + c] = cacc[c];
+            }
+            tr.ev(0xD00);                                // gather done
+            named_bar_sync(2 + q, 64);
+            if (hh == 0 && valid) {
+                const float inv = 1.0f / fmaxf(ssum + s_red[row * 5], 1e-12f);
+                float* o = ra.out + n * ra.os_n + ra.c0 * ra.os_c + s * ra.os_s + h * ra.os_h + w * ra.os_w;
+#pragma unroll
+                for (int c = 0; c < TC_MAX_C; ++c)
+                    if (c < ra.C) o[c * ra.os_c] = (cacc[c] + s_red[row * 5 + 1 + c]) * inv;
+            }
+        };
+
+        // ---- TA: gather of this CTA's tile number `piter` from its raw head values (off_stg) and its halo slot
+        const int halo_f4 = (int)(P.halo_bytes / 16);
+        auto gather_ta = [&](long long piter) {
+            int pn, ps, h0, w0;
+            tile_coords(blockIdx.x + piter * gridDim.x, pn, ps, h0, w0);
+            float ssum = 0.f, cacc[TC_MAX_C] = {0.f, 0.f, 0.f, 0.f};
+            const float4* hbase = s_halo + (piter & 1) * halo_f4 + ty * TC_HALO_PITCH + tx;
+            const float4* stg = reinterpret_cast<const float4*>(smem + P.off_stg) + row;
+            const int gi = P.n_hidden;
+            const float* bias = s_bias + (P.g[gi].bias_off - P.bias_skip);
+#pragma unroll 1
+            for (int c32 = hh * 32; c32 < P.g[gi].N; c32 += 64) {
+                uint32_t rr[32];
+#pragma unroll
+                for (int k = 0; k < 8; ++k) {
+                    const float4 v = stg[(c32 / 4 + k) * TC_M];
+                    rr[4 * k] = __float_as_uint(v.x); rr[4 * k + 1] = __float_as_uint(v.y);
+                    rr[4 * k + 2] = __float_as_uint(v.z); rr[4 * k + 3] = __float_as_uint(v.w);
+                }
+                gather32(rr, P.g[gi].tap0 + c32, bias + c32, hbase, ssum, cacc);
+            }
+            store_px(ssum, cacc, pn, ps, h0 + ty, w0 + tx, (h0 + ty < ra.H) && (w0 + tx < ra.W));
+        };
 
         long long tile = blockIdx.x;
         for (long long iter = 0; iter < my_iters; ++iter, tile += gridDim.x) {
@@ -622,7 +781,10 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
             // The halo tile (replicate-clamped, render_psf.py:96) is only needed by the gather at the end of the
             // tile: its pixels are fetched one per thread per hidden layer -- the global loads are issued before
             // the accumulator wait and stored to smem after the layer's epilogue, so they cost no time.
-            named_bar_sync(1, TC_EPI_THREADS);           // previous tile's gather is done with halo/red
+            // (TA: two halo slots; the slot of this tile was last read by the gather of tile iter-2, which every
+            // thread finished before the "halo tile complete" barrier of tile iter-1)
+            if (!TA) named_bar_sync(1, TC_EPI_THREADS);  // previous tile's gather is done with halo/red
+            float4* const s_halo_t = s_halo + (TA ? (int)(iter & 1) * halo_f4 : 0);
             const float* img_n = ra.img + ((long long)n * ra.Ctot + ra.c0) * ra.H * ra.W;
             const long long cstride = (long long)ra.H * ra.W;
             auto halo_fetch = [&](int idx, float4& v) -> int {       // returns the smem slot or -1
@@ -651,55 +813,121 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                 const bool need_lo = terms_of(gi + 1) >= 2;
                 const uint32_t t_acc = t_lane + buf * 256;
                 uint32_t rr[2][32], rf[2][16];
-                if (fine) {
-                    tmem_ld16(t_acc + hh * 16, rf[0]);          // my 16 columns of chunk 0 ...
-                    tmem_ld16(t_acc + 32 + hh * 16, rf[1]);     // ... and of chunk 1
+                if constexpr (TA) {
+                    // the same column map and hand-offs, converted in place: 16 accumulator columns -> one K=16 step of
+                    // the next layer's A (8 columns hi, 8 lo); only this thread's lane is read and written
+                    tmem_ld16(t_acc + hh * 16, rf[0]);
+                    tmem_ld16(t_acc + 32 + hh * 16, rf[1]);
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        tmem_ld_wait();
+                        if (j < 3) tmem_ld32(t_acc + (j + 1) * 64 + hh * 32, rr[(j + 1) & 1]);
+                        if (j == 0) {
+#pragma unroll
+                            for (int c = 0; c < 2; ++c) {
+                                epi_ta16(rf[c], t_acc + c * 32 + hh * 16);
+                                tmem_st_wait();
+                                tc_fence_before_sync();
+                                __syncwarp();
+                                if (lane == 0) mbar_arrive(bar_aready(c));
+                            }
+                        } else {
+                            const int col = j * 64 + hh * 32;
+                            epi_ta16(&rr[j & 1][0], t_acc + col);
+                            epi_ta16(&rr[j & 1][16], t_acc + col + 16);
+                            tmem_st_wait();
+                            tc_fence_before_sync();
+                            __syncwarp();
+                            if (lane == 0) mbar_arrive(bar_aready(j == 1 ? 2 : 4));
+                        }
+                        tr.ev(0xC00 + j);
+                    }
                 } else {
-                    tmem_ld32(t_acc + hh * 32, rr[0]);
-                }
+                    if (fine) {
+                        tmem_ld16(t_acc + hh * 16, rf[0]);          // my 16 columns of chunk 0 ...
+                        tmem_ld16(t_acc + 32 + hh * 16, rf[1]);     // ... and of chunk 1
+                    } else {
+                        tmem_ld32(t_acc + hh * 32, rr[0]);
+                    }
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    tmem_ld_wait();
-                    if (j < 3) tmem_ld32(t_acc + (j + 1) * 64 + hh * 32, rr[(j + 1) & 1]);
-                    if (j == 0 && fine) {
+                    for (int j = 0; j < 4; ++j) {
+                        tmem_ld_wait();
+                        if (j < 3) tmem_ld32(t_acc + (j + 1) * 64 + hh * 32, rr[(j + 1) & 1]);
+                        if (j == 0 && fine) {
 #pragma unroll
-                        for (int c = 0; c < 2; ++c) {
-                            const int col = c * 32 + hh * 16;
+                            for (int c = 0; c < 2; ++c) {
+                                const int col = c * 32 + hh * 16;
 #pragma unroll
-                            for (int i = 0; i < 2; ++i)
-                                epi_group8(&rf[c][i * 8], a_hi, a_lo, col / 8 + i, a_row, need_lo);
+                                for (int i = 0; i < 2; ++i)
+                                    epi_group8(&rf[c][i * 8], a_hi, a_lo, col / 8 + i, a_row, need_lo);
+                                fence_proxy_async_smem();
+                                __syncwarp();
+                                if (lane == 0) mbar_arrive(bar_aready(c));
+                            }
+                        } else {
+                            const int col = j * 64 + hh * 32;
+#pragma unroll
+                            for (int i = 0; i < 4; ++i)
+                                epi_group8(&rr[j & 1][i * 8], a_hi, a_lo, col / 8 + i, a_row, need_lo);
                             fence_proxy_async_smem();
                             __syncwarp();
-                            if (lane == 0) mbar_arrive(bar_aready(c));
+                            if (lane == 0) mbar_arrive(bar_aready(fine ? (j == 1 ? 2 : 4) : j));
                         }
-                    } else {
-                        const int col = j * 64 + hh * 32;
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            epi_group8(&rr[j & 1][i * 8], a_hi, a_lo, col / 8 + i, a_row, need_lo);
-                        fence_proxy_async_smem();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(bar_aready(fine ? (j == 1 ? 2 : 4) : j));
+                        tr.ev(0xC00 + j);                        // columns of 64-group j handed to the MMA warp
                     }
-                    tr.ev(0xC00 + j);                        // columns of 64-group j handed to the MMA warp
                 }
                 tc_fence_before_sync();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_accfree(buf));
-                if (hslot >= 0) s_halo[hslot] = hv;
+                if (hslot >= 0) s_halo_t[hslot] = hv;
                 ++gcount;
+                if constexpr (TA) {
+                    if (gi == 0 && iter > 0) gather_ta(iter - 1);       // under L2's MMAs
+                    if (gi == P.n_hidden - 1 && iter + 1 < my_iters) {
+                        // under the head's MMAs: the last MMA that read the columns layer 0 writes (L9's) has retired
+                        layer0(tile + gridDim.x, (uint32_t)(gcount & 1));
+                        tr.ev(0x900);
+                    }
+                }
             }
             for (int idx = P.n_hidden * TC_EPI_THREADS + et; !PRED && !dummy && idx < HH * HW; idx += TC_EPI_THREADS) {   // remainder
                 float4 hv;
                 const int hslot = halo_fetch(idx, hv);
-                s_halo[hslot] = hv;
+                s_halo_t[hslot] = hv;
             }
             named_bar_sync(1, TC_EPI_THREADS);           // halo tile complete (all warps stored their share)
+
+            if constexpr (TA) {
+                // ---- head: raw accumulator -> off_stg, buffer released at once; sigmoid and gather follow tile
+                //      t+1's L1 epilogue (gather_ta).  Each thread later reads back only what it wrote here.
+                const int buf = (int)(gcount & 1), gi = P.n_hidden;
+                tr.ev(0xA00 + gi);
+                mbar_wait(bar_accfull(buf), (afphase >> buf) & 1);
+                afphase ^= 1u << buf;
+                tc_fence_after_sync();
+                tr.ev(0xB00 + gi);
+                float4* stg = reinterpret_cast<float4*>(smem + P.off_stg) + row;
+#pragma unroll 1
+                for (int c32 = hh * 32; c32 < P.g[gi].N; c32 += 64) {
+                    uint32_t rr[32];
+                    tmem_ld32(t_lane + buf * 256 + c32, rr);
+                    tmem_ld_wait();
+#pragma unroll
+                    for (int k = 0; k < 8; ++k)
+                        stg[(c32 / 4 + k) * TC_M] = make_float4(__uint_as_float(rr[4 * k]), __uint_as_float(rr[4 * k + 1]),
+                                                                __uint_as_float(rr[4 * k + 2]), __uint_as_float(rr[4 * k + 3]));
+                }
+                tc_fence_before_sync();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(bar_accfree(buf));
+                ++gcount;
+                continue;
+            }
 
             // ---- head blocks: sigmoid, gather from the halo tile (render_psf.py:103-105)
             //      The bias table holds -log2(e) * bias for the head, so exp(-(acc + b)) is one FFMA + EX2.
             float ssum = 0.f, cacc[TC_MAX_C] = {0.f, 0.f, 0.f, 0.f};
-            const float4* hbase = s_halo + ty * TC_HALO_PITCH + tx;
+            const float4* hbase = s_halo_t + ty * TC_HALO_PITCH + tx;
             for (int gi = P.n_hidden; gi < P.n_groups; ++gi) {
                 const int buf = (int)(gcount & 1);
                 tr.ev(0xA00 + gi);
@@ -708,7 +936,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                 tc_fence_after_sync();
                 tr.ev(0xB00 + gi);
                 if (gi == P.n_groups - 1 && iter + 1 < my_iters) {
-                    layer0(tile + gridDim.x);            // every MMA that read this tile's A operand has retired
+                    layer0(tile + gridDim.x, 0u);        // every MMA that read this tile's A operand has retired
                     tr.ev(0x900);
                 }
                 const int gN = P.g[gi].N, gtap0 = P.g[gi].tap0;
@@ -780,14 +1008,12 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     uint32_t rr[32];
                     tmem_ld32(t_lane + buf * 256 + c32, rr);
                     const int tap_first = gtap0 + c32;
-                    int i = tap_first / ks, j = tap_first - i * ks;
-                    int off = i * TC_HALO_PITCH + j;
-                    const int nvalid = kk - tap_first;     // >= 32 for every group but the padded last one
                     tmem_ld_wait();
                     if constexpr (PRED) {
                         // several head blocks (ks >= 13): the un-normalised sigmoid values go out now -- transposed
                         // through the halo area like above, so that a store instruction covers 4 rows x 32 B instead
                         // of 32 rows -- and are rescaled below
+                        const int nvalid = kk - tap_first;
                         float sgv[32];
 #pragma unroll
                         for (int u = 0; u < 32; ++u) {
@@ -814,35 +1040,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                             }
                             __syncwarp();
                         }
-                    } else if (nvalid >= 32) {
-                        // branch-free so that the MUFU / LDS latencies of different taps overlap
-#pragma unroll
-                        for (int u = 0; u < 32; ++u) {
-                            const float sg = rcp_approx(1.0f + ex2_approx(fmaf(__uint_as_float(rr[u]), NEG_LOG2E, bias[c32 + u])));
-                            const float4 px = hbase[off];
-                            ssum += sg;
-                            cacc[0] = fmaf(sg, px.x, cacc[0]);
-                            cacc[1] = fmaf(sg, px.y, cacc[1]);
-                            cacc[2] = fmaf(sg, px.z, cacc[2]);
-                            cacc[3] = fmaf(sg, px.w, cacc[3]);
-                            ++off;
-                            if (++j == ks) { j = 0; off += TC_HALO_PITCH - ks; }
-                        }
                     } else {
-#pragma unroll
-                        for (int u = 0; u < 32; ++u) {
-                            const bool ok = u < nvalid;    // padding columns contribute nothing and read slot 0
-                            float sg = rcp_approx(1.0f + ex2_approx(fmaf(__uint_as_float(rr[u]), NEG_LOG2E, bias[c32 + u])));
-                            sg = ok ? sg : 0.f;
-                            const float4 px = hbase[ok ? off : 0];
-                            ssum += sg;
-                            cacc[0] = fmaf(sg, px.x, cacc[0]);
-                            cacc[1] = fmaf(sg, px.y, cacc[1]);
-                            cacc[2] = fmaf(sg, px.z, cacc[2]);
-                            cacc[3] = fmaf(sg, px.w, cacc[3]);
-                            ++off;
-                            if (++j == ks) { j = 0; off += TC_HALO_PITCH - ks; }
-                        }
+                        gather32(rr, tap_first, bias + c32, hbase, ssum, cacc);
                     }
                 }
                 tc_fence_before_sync();
@@ -866,21 +1065,10 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                 }
                 continue;
             }
-            // ---- combine the two column-halves of each pixel, normalise (F.normalize p=1), store
-            if (hh == 1) {
-                s_red[row * 5 + 0] = ssum;
-#pragma unroll
-                for (int c = 0; c < TC_MAX_C; ++c) s_red[row * 5 + 1 + c] = cacc[c];
-            }
-            tr.ev(0xD00);                                // gather done
-            named_bar_sync(2 + q, 64);
-            if (hh == 0 && valid) {
-                const float inv = 1.0f / fmaxf(ssum + s_red[row * 5], 1e-12f);
-                float* o = ra.out + n * ra.os_n + ra.c0 * ra.os_c + s * ra.os_s + h * ra.os_h + w * ra.os_w;
-#pragma unroll
-                for (int c = 0; c < TC_MAX_C; ++c)
-                    if (c < ra.C) o[c * ra.os_c] = (cacc[c] + s_red[row * 5 + 1 + c]) * inv;
-            }
+            store_px(ssum, cacc, n, s, h, w, valid);
+        }
+        if constexpr (TA) {
+            if (my_iters > 0) gather_ta(my_iters - 1);
         }
     }
 

@@ -142,6 +142,18 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
 __device__ __forceinline__ void tmem_ld_wait() {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
+// 16 registers per thread -> 32 lanes x 16 consecutive 32-bit columns (thread = lane)
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+        "{%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
+        "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
+        "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+        : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() {
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+}
 
 // ----------------------------------------------------------------------------- UMMA descriptors
 // Shared-memory matrix descriptor, K-major, SWIZZLE_NONE ("interleaved" canonical layout):
@@ -175,6 +187,20 @@ __device__ __forceinline__ void umma_f16_ss(uint32_t d_tmem, uint64_t adesc, uin
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
         "}" ::"r"(d_tmem),
         "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+
+// The same with A in tensor memory (UTCHMMA tmem A operand): lane m = row m, a K=16 step of fp16 A is 8 consecutive
+// 32-bit columns from a_tmem, column c holding K elements 2c (low half) and 2c + 1 (high half).
+__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc,
+                                            uint32_t accumulate) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t"
+        "}" ::"r"(d_tmem),
+        "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
 
