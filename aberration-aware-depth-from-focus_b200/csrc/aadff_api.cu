@@ -13,7 +13,6 @@
 
 #include "../../include/aadff.h"
 #include "fused_tc_kernel.cuh"
-#include "fused_fast2_kernel.cuh"
 #include "gather_kernel.cuh"
 #include "gather_coalesced_kernel.cuh"
 #include "gather_strip_kernel.cuh"
@@ -143,21 +142,7 @@ bool launch_psf_conv(int ks, int grid, cudaStream_t st, const PsfConvArgs& a) {
     }
 }
 
-template <int KS>
-bool launch_thinlens(int ks, int grid, int smem, cudaStream_t st, const ThinLensArgs& a, const CUtensorMap& map) {
-    if constexpr (KS > 31) {
-        return false;
-    } else {
-        if (ks == KS) {
-            if (smem > 48 * 1024)      // per-device attribute
-                cudaFuncSetAttribute(thinlens_render_kernel<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            thinlens_render_kernel<KS><<<grid, TL_NT, smem, st>>>(a, map);
-            return true;
-        }
-        return launch_thinlens<KS + 2>(ks, grid, smem, st, a, map);
-    }
-}
-// two pixels per thread (thinlens_render2_kernel): tile geometry by kernel size
+// thinlens_render2_kernel: tile geometry by kernel size
 template <int KS>
 bool thinlens2_geometry(int ks, int cn, int* box_w, int* box_h, int* smem) {
     if constexpr (KS > 31) {
@@ -546,16 +531,14 @@ int aadff_psfnet_create(const float* const* weights, const float* const* biases,
         CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<true, false, 0>, attr, so));
 #define AADFF_SET_ATTR(U)                                                                        \
         CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, U>, attr, so));   \
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, U, true>, attr, so));   \
         CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, true, U>, attr, so));
-        AADFF_SET_ATTR(0) AADFF_SET_ATTR(1) AADFF_SET_ATTR(3) AADFF_SET_ATTR(13) AADFF_SET_ATTR(12) AADFF_SET_ATTR(15)
+        AADFF_SET_ATTR(0) AADFF_SET_ATTR(1) AADFF_SET_ATTR(3) AADFF_SET_ATTR(13) AADFF_SET_ATTR(12) AADFF_SET_ATTR(14)
+        AADFF_SET_ATTR(15)
 #undef AADFF_SET_ATTR
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 14>, attr, so));      // econ8: no cluster variant
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, true, 14>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<true, false, 0, false, true>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 12, false, true>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 13, false, true>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 14, false, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<true, false, 0, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 12, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 13, true>, attr, so));
+        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 14, true>, attr, so));
     }
 #undef CREATE_TRY
     *out = h;
@@ -615,53 +598,6 @@ static int ensure_econ(aadff_psfnet_t h) {
     return AADFF_OK;
 }
 
-// AADFF_MODE_FAST with two tiles in flight per CTA (fused_fast2_kernel.cuh).  Built, bit-identical to the one-tile kernel
-// and measured SLOWER (0.80-0.91x, profiles/NOTES_r02.md: the second tile's activations leave a 64 KB weight ring, too
-// shallow to cover the L2 latency at fast mode's 64 B/clk per SM), so it only runs when debug flag 32 asks for it.
-// Returns 1 if the launch does not qualify (flag not set, several head blocks, shared-memory budget).
-static int launch_fast2(aadff_psfnet_t h, const RenderArgs& ra, cudaStream_t st, long long tile_row0, long long tile_row1) {
-    if (!h->tc_ok || h->n_groups != h->n_hidden + 1 || !(g_dbg_flags.load() & 32)) return 1;
-    F2Params P{};
-    P.ra = ra;
-    P.wpack = h->d_wpack;
-    P.bias = h->d_bias_tc;
-    P.w0b0 = h->d_w0b0;
-    P.n_groups = h->n_groups;
-    P.n_hidden = h->n_hidden;
-    P.n_bias = h->n_bias;
-    P.bias_skip = h->head_bias0;
-    P.kk = h->kk;
-    for (int i = 0; i < h->n_groups; ++i) { P.g[i] = h->groups[i]; P.g[i].terms = 1; }
-    P.tiles_x = (ra.W + TC_TILE_W - 1) / TC_TILE_W;
-    P.tiles_y = (ra.H + TC_TILE_H - 1) / TC_TILE_H;
-    P.n_tiles = (long long)P.tiles_x * P.tiles_y * ra.N * ra.S;
-    if (tile_row1 >= 0) {
-        P.tile0 = tile_row0 * P.tiles_x;
-        P.n_tiles = (tile_row1 - tile_row0) * P.tiles_x;
-        if (P.n_tiles <= 0) return AADFF_OK;
-    }
-    P.halo_pitch = TC_TILE_W + ra.ks - 1;
-    P.halo_bytes = (uint32_t)(TC_TILE_H + ra.ks - 1) * P.halo_pitch * 16;
-    const uint32_t bias_bytes = (uint32_t)(h->n_bias - h->head_bias0) * 4;
-    P.off_stage = 2 * TC_A_PART_BYTES;
-    P.off_bias = P.off_stage + F2_STAGES * TC_STAGE_BYTES;
-    P.off_w0 = P.off_bias + bias_bytes;
-    P.off_halo = (P.off_w0 + 320 * 4 + 15u) & ~15u;
-    P.off_red = P.off_halo + 2 * P.halo_bytes;
-    P.off_bar = P.off_red + 2 * TC_M * 5 * 4;
-    P.off_ones = (P.off_bar + TC_BAR_BYTES + 15u) & ~15u;
-    P.off_bslab = P.off_ones + 2 * TC_A_LBO;
-    const uint32_t smem = P.off_bslab + 2 * TC_BSLAB_BYTES;
-    if (smem > (uint32_t)h->smem_optin) return 1;
-    const long long units = (P.n_tiles + 1) / 2;
-    const int grid = (int)std::min<long long>(units, h->num_sms);
-    cudaFuncSetAttribute(fused_fast2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin);
-    fused_fast2_kernel<<<grid, TC_NT, smem, st>>>(P);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
-}
-
 static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st, long long tile_row0 = 0,
                      long long tile_row1 = -1, const float* probes = nullptr, float* psf_out = nullptr,
                      long long n_probes = 0) {
@@ -670,10 +606,6 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     if (econ_like) {
         const int rc = ensure_econ(h);
         if (rc) return rc;
-    }
-    if (mode == AADFF_MODE_FAST && probes == nullptr && g_trace.load() == nullptr) {
-        const int rc = launch_fast2(h, ra, st, tile_row0, tile_row1);
-        if (rc <= 0) return rc;                                   // launched (0) or failed (< 0); 1 = not eligible
     }
     TcParams P{};
     P.ra = ra;
@@ -743,7 +675,7 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     // 32 KB stages (two packed K=32 slabs each) so that every issue iteration queues four MMAs
     P.kslab = (!any_lo && stages == 4) ? 2 : 1;
     P.n_stages = (P.kslab == 2) ? 4 : stages;
-    int grid = (int)std::min<long long>(P.n_tiles, h->num_sms);
+    const int grid = (int)std::min<long long>(P.n_tiles, h->num_sms);
     // kernel specialisation (fused_tc_kernel.cuh, template UNI): pattern 3 = all groups three-term (parity), 1 = all
     // single-term with the long ring (fast), 2 = econ, 5 = mixed, 0 = per-group terms at run time; +10 when the ring has
     // four stages and every group consumes a multiple of four of them (ring position of a K-step = compile-time)
@@ -764,9 +696,6 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     else if (econ_pat && aligned) uni = 12;
     else if (econ8_pat && aligned && h->n_groups > TC_ECON8_FIRST_GROUP) uni = 14;
     else if (mixed_pat && aligned) uni = 15;
-    // 2-CTA clusters sharing the weight stream by multicast (fused_tc_kernel.cuh, CL2).  Built, bit-exact, and measured
-    // NOT to pay (profiles/NOTES_r02.md: -7 % at c2, +-1 % where power-capped), so it is off unless debug flag 8 asks for it.
-    const bool cl2 = P.probes == nullptr && P.trace == nullptr && uni != 0 && uni != 14 && (P.dbg & 8u) && h->num_sms >= 2;
     // A operands in tensor memory (fused_tc_kernel.cuh, TA): render launches of the 2-/3-term specialisations with one
     // head block of N <= 192 (ks <= 13) and at least two hidden layers, 4-stage ring.  Its shared memory holds no
     // activations: ring, raw head values of the tile being gathered, two halo slots.  Debug flag 1 << 20 keeps such
@@ -775,7 +704,7 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     for (int i = 0; i < h->n_groups; ++i) all2 &= (P.g[i].terms >= 2);
     const uint32_t head_n = h->groups[h->n_hidden].N;
     uint32_t smem_launch = smem;
-    const bool ta = P.probes == nullptr && !cl2 && !(P.dbg & (1u << 20)) && h->n_groups == h->n_hidden + 1 &&
+    const bool ta = P.probes == nullptr && !(P.dbg & (1u << 20)) && h->n_groups == h->n_hidden + 1 &&
                     h->n_hidden >= 2 && head_n <= (uint32_t)TC_TA_L1_COL && P.kslab == 1 && P.n_stages == 4 && all2 &&
                     (uni == 12 || uni == 13 || uni == 14 || P.trace != nullptr);
     if (ta) {
@@ -793,35 +722,14 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
         smem_launch = P.off_bslab + bslab_bytes;
         if (smem_launch > (uint32_t)h->smem_optin) return fail(AADFF_E_UNSUPPORTED, "shared memory budget exceeded (TA)");
     }
-    if (cl2) {
-        grid = (int)std::min<long long>((P.n_tiles + 1) & ~1ll, (long long)(h->num_sms & ~1));
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)grid);
-        cfg.blockDim = dim3(TC_NT);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = st;
-        cudaLaunchAttribute la[1];
-        la[0].id = cudaLaunchAttributeClusterDimension;
-        la[0].val.clusterDim.x = 2; la[0].val.clusterDim.y = 1; la[0].val.clusterDim.z = 1;
-        cfg.attrs = la;
-        cfg.numAttrs = 1;
-        cudaError_t le = cudaSuccess;
-        switch (uni) {
-            case 1: le = cudaLaunchKernelEx(&cfg, fused_psfnet_render_kernel<false, false, 1, true>, P); break;
-            case 3: le = cudaLaunchKernelEx(&cfg, fused_psfnet_render_kernel<false, false, 3, true>, P); break;
-            case 13: le = cudaLaunchKernelEx(&cfg, fused_psfnet_render_kernel<false, false, 13, true>, P); break;
-            case 12: le = cudaLaunchKernelEx(&cfg, fused_psfnet_render_kernel<false, false, 12, true>, P); break;
-            default: le = cudaLaunchKernelEx(&cfg, fused_psfnet_render_kernel<false, false, 15, true>, P); break;
-        }
-        if (le != cudaSuccess) return fail(AADFF_E_CUDA, std::string("cluster launch: ") + cudaGetErrorString(le));
-    } else if (P.trace != nullptr && P.probes == nullptr) {
-        if (ta) fused_psfnet_render_kernel<true, false, 0, false, true><<<grid, TC_NT, smem_launch, st>>>(P);
+    if (P.trace != nullptr && P.probes == nullptr) {
+        if (ta) fused_psfnet_render_kernel<true, false, 0, true><<<grid, TC_NT, smem_launch, st>>>(P);
         else fused_psfnet_render_kernel<true, false, 0><<<grid, TC_NT, smem, st>>>(P);
     } else if (ta) {
         switch (uni) {
-            case 12: fused_psfnet_render_kernel<false, false, 12, false, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
-            case 13: fused_psfnet_render_kernel<false, false, 13, false, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
-            default: fused_psfnet_render_kernel<false, false, 14, false, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
+            case 12: fused_psfnet_render_kernel<false, false, 12, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
+            case 13: fused_psfnet_render_kernel<false, false, 13, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
+            default: fused_psfnet_render_kernel<false, false, 14, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
         }
     } else {
 #define AADFF_LAUNCH(U)                                                                                   \
@@ -1005,7 +913,7 @@ int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, i
     CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int dbg = g_dbg_flags.load();
-    if (ks >= 3 && ks <= STRIP_MAX_KS && !(dbg & (128 | 512)) && W % 4 == 0 && reinterpret_cast<uintptr_t>(psf) % 16 == 0 &&
+    if (ks >= 3 && ks <= STRIP_MAX_KS && !(dbg & 512) && W % 4 == 0 && reinterpret_cast<uintptr_t>(psf) % 16 == 0 &&
         reinterpret_cast<uintptr_t>(out) % 8 == 0 && (long long)N * H * ((W + 31) / 32) < (1ll << 40)) {
         // strip-walking kernel (gather_strip_kernel.cuh): bulk-copied PSF rows, per-warp pipelines
         int c0 = 0;
@@ -1019,7 +927,7 @@ int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, i
         }
         return AADFF_OK;
     }
-    if (ks >= 3 && ks <= 31 && !(g_dbg_flags.load() & 128)) {
+    if (ks >= 3 && ks <= 31) {
         // register-streaming kernel (gather_coalesced_kernel.cuh): any W, any alignment
         const long long tiles = (long long)N * ((H + GC_WARPS - 1) / GC_WARPS) * ((W + GC_TW - 1) / GC_TW);
         if (tiles >= (1ll << 31)) return fail(AADFF_E_INVALID, "image batch too large for one launch");
@@ -1035,42 +943,7 @@ int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, i
         }
         return AADFF_OK;
     }
-    const int kk = ks * ks;
-    int P = 32;
-    while (P > 4 && P * kk * 4 > GS_BUF_BYTES) P >>= 1;
-    const bool stream_ok = (W % 4 == 0) && (reinterpret_cast<uintptr_t>(psf) % 16 == 0) && (P * kk * 4 <= GS_BUF_BYTES);
-    if (stream_ok) {
-        // HBM-streaming path: cp.async.bulk PSF chunks, smem halo tile.  One 16 KB chunk buffer per warp, 8 warps.
-        // (Two buffers per warp only fit with 6 warps and measured 20 % slower: the kernel is limited by the
-        //  arithmetic/latency of its 8 warps, not by exposed copy latency -- debug flag 64 selects that variant.)
-        const int nbuf = (P == 32 && (g_dbg_flags.load() & 64)) ? 2 : 1;
-        const int nw = (nbuf == 2) ? GS_TILE_H_2BUF : GS_TILE_H_1BUF;
-        const int buf_bytes = (P * kk * 4 + 127) / 128 * 128;
-        const int HH = nw + ks - 1, pitch = (GS_TILE_W + ks - 1) | 1;
-        const int smem = nw * nbuf * buf_bytes + GS_MAXC * HH * pitch * 4 + 16 * nw;
-        if (smem > 48 * 1024) {    // per-device attribute: set on every launch that needs the opt-in
-            if (nw == GS_TILE_H_1BUF)
-                CUDA_TRY(cudaFuncSetAttribute(local_psf_stream_kernel<GS_TILE_H_1BUF>,
-                                              cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            else
-                CUDA_TRY(cudaFuncSetAttribute(local_psf_stream_kernel<GS_TILE_H_2BUF>,
-                                              cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        }
-        const long long tiles = (long long)N * ((H + nw - 1) / nw) * ((W + GS_TILE_W - 1) / GS_TILE_W);
-        const int grid = (int)std::min<long long>(tiles, sms);
-        for (int c0 = 0; c0 < C; c0 += GS_MAXC) {
-            const int cn = std::min(GS_MAXC, C - c0);
-            if (nw == GS_TILE_H_1BUF)
-                local_psf_stream_kernel<GS_TILE_H_1BUF><<<grid, nw * 32, smem, st>>>(img, psf, out, N, C, H, W, ks, c0, cn,
-                                                                                   P, nbuf, buf_bytes);
-            else
-                local_psf_stream_kernel<GS_TILE_H_2BUF><<<grid, nw * 32, smem, st>>>(img, psf, out, N, C, H, W, ks, c0, cn,
-                                                                                   P, nbuf, buf_bytes);
-            g_launches.fetch_add(1);
-            CUDA_TRY(cudaGetLastError());
-        }
-        return AADFF_OK;
-    }
+    // any other kernel size (1, or above 31): the generic kernel (gather_kernel.cuh)
     const int smem = GATHER_WARPS * 32 * (GATHER_TT + 1) * (int)sizeof(float);
     if (smem > 48 * 1024)
         CUDA_TRY(cudaFuncSetAttribute(local_psf_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -1117,25 +990,20 @@ int aadff_thinlens_render_f32(const float* img, const float* depth, const float*
     a.flip_dev = flip_sign_dev;
     if (ks > 31) return fail(AADFF_E_UNSUPPORTED, "thin-lens kernel sizes above 31 are not built");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const bool two_px = !(g_dbg_flags.load() & 2048);        // 2048: the one-pixel-per-thread kernel (A/B timing)
-    const int tl_r = (ks - 1) / 2, tl_sh = (4 - tl_r % 4) % 4;
-    const int tile_w = two_px ? TL2_TILE_W : TL_TILE_W;
-    const long long tiles = (long long)N * ((H + TL_TILE_H - 1) / TL_TILE_H) * ((W + tile_w - 1) / tile_w);
+    const long long tiles = (long long)N * ((H + TL_TILE_H - 1) / TL_TILE_H) * ((W + TL2_TILE_W - 1) / TL2_TILE_W);
     if (tiles >= (1ll << 31)) return fail(AADFF_E_INVALID, "image batch too large for one launch");
     const int grid = (int)std::min<long long>(tiles, (long long)sms * 4);
     for (int c0 = 0; c0 < C; c0 += TL_MAXC) {
         a.c0 = c0;
         a.cn = std::min(TL_MAXC, C - c0);
-        int HH = TL_TILE_H + ks - 1, BW = (TL_TILE_W + ks - 1 + tl_sh + 3) / 4 * 4;      // = ThinLensCfg<ks>::HH, BW
-        int smem = (ks <= 15 ? 2 : 1) * ((a.cn * HH * BW + 31) / 32 * 32) * 4 + 128;      // = ThinLensCfg<ks>::SMEM_BYTES(cn)
-        if (two_px && !thinlens2_geometry<1>(ks, a.cn, &BW, &HH, &smem)) return fail(AADFF_E_INVALID, "unsupported kernel size");
+        int HH = 0, BW = 0, smem = 0;
+        if (!thinlens2_geometry<1>(ks, a.cn, &BW, &HH, &smem)) return fail(AADFF_E_INVALID, "unsupported kernel size");
         if (smem > optin) return fail(AADFF_E_UNSUPPORTED, "kernel size too large for the shared-memory halo tile");
         // the image halo of interior tiles arrives as one TMA box [cn][HH][BW] of the [N*C, H, W] tensor
         CUtensorMap map;
         std::memset(&map, 0, sizeof(map));
         a.use_tma = make_image_map(&map, img, (long long)N * C, H, W, BW, HH, a.cn) && !(g_dbg_flags.load() & 16);
-        const bool launched = two_px ? launch_thinlens2<1>(ks, grid, smem, st, a, map) : launch_thinlens<1>(ks, grid, smem, st, a, map);
-        if (!launched) return fail(AADFF_E_INVALID, "unsupported kernel size");
+        if (!launch_thinlens2<1>(ks, grid, smem, st, a, map)) return fail(AADFF_E_INVALID, "unsupported kernel size");
         g_launches.fetch_add(1);
         CUDA_TRY(cudaGetLastError());
     }

@@ -97,7 +97,7 @@ struct TcParams {
     uint32_t off_bslab;     // bias-slab slot: [256 x 8] halves (K columns 0..7) + a shared [256 x 8] block of zeros (K 8..15)
     uint32_t off_stg;       // TA: raw head accumulator of the tile being gathered, [head columns / 4][128 rows] float4
     uint32_t halo_bytes;    // TA: one of the two halo slots (tile t is gathered while tile t+1's halo is fetched)
-    uint32_t dbg;           // what-if timing switches (results invalid): 1 = no weight copies, 2 = no A stores
+    uint32_t dbg;           // debug flags (include/aadff.h); the kernel reads bit 0: what-if, no weight copies
     // pred mode (kernel instantiated with PRED = true): probes [M,4] in, L1-normalised PSFs [M, ks*ks] out
     const float* probes;
     float* psf_out;
@@ -232,13 +232,6 @@ constexpr int TC_WARP_MMA = TC_EPI_WARPS + 1;        // warp 9
 // one after); 0 = per-group terms at run time (short rings, the traced build).  UNI >= 10 ("aligned"): the ring has four
 // stages and every group consumes a multiple of four, so the ring stage of a K-step is a compile-time constant too.
 //
-// CL2: the kernel runs as clusters of two CTAs (one TPC) that walk the weight ring in lock step: every ring stage is
-// filled by TWO multicast bulk copies, one half-slab from each CTA's producer, each landing in both CTAs' shared memory
-// (one L2 read feeds two SMs: the L2 -> SM weight stream, 2.3 MB per tile in parity mode, is halved).  A stage is
-// refilled only after BOTH CTAs' MMAs have released it (the release commits are multicast too, the "empty" barriers
-// count two arrivals).  Everything else -- activations, accumulators, MMAs, epilogue -- stays per CTA.  Both CTAs of a
-// pair run the same number of tile iterations; the one without a tile left computes a dummy tile and stores nothing.
-//
 // TA: the activations never touch shared memory.  Each layer's epilogue turns its accumulator into the next layer's A
 // operand in the same TMEM columns (epi_ta16), and the MMAs read A from tensor memory.  A group's A therefore lives in
 // the other accumulator buffer, so before a group's first MMA the MMA warp also waits for the previous group's
@@ -246,15 +239,11 @@ constexpr int TC_WARP_MMA = TC_EPI_WARPS + 1;        // warp 9
 // t's head MMAs, and tile t's head values are copied raw to shared memory (off_stg) so that its sigmoid / gather runs
 // after tile t+1's L1 epilogue, under L2's MMAs.  Render kernels with one head block of N <= 192, at least two hidden
 // layers and only 2-/3-term groups (host-checked).
-template <bool TRACE, bool PRED, int UNI, bool CL2 = false, bool TA = false>
+template <bool TRACE, bool PRED, int UNI, bool TA = false>
 __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __grid_constant__ TcParams P) {
-    static_assert(!(CL2 && (PRED || TRACE)), "the cluster variant exists for the render kernels only");
-    static_assert(!(TA && (CL2 || PRED)), "tensor-memory A operands exist for the one-CTA render kernels only");
+    static_assert(!(TA && PRED), "tensor-memory A operands exist for the render kernels only");
     constexpr int UM = UNI % 10;
-    const uint32_t cta_rank = CL2 ? cluster_ctarank() : 0u;
-    // tile iterations of this CTA: with CL2 both CTAs of a pair take the count of the even one
-    const long long first_tile = CL2 ? (long long)(blockIdx.x & ~1u) : (long long)blockIdx.x;
-    const long long my_iters = (P.n_tiles > first_tile) ? (P.n_tiles - first_tile + gridDim.x - 1) / gridDim.x : 0;
+    const long long my_iters = (P.n_tiles > blockIdx.x) ? (P.n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     constexpr bool ALIGNED = UNI >= 10;
     const int kslab_c = (UM == 3 || UM == 2 || UM == 4 || UM == 5) ? 1 : UM == 1 ? 2 : P.kslab;
     auto terms_of = [&](int gi) -> int {
@@ -290,7 +279,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
     static_assert(8 * (2 * TC_MAX_STAGES + 14) + 4 <= TC_BAR_BYTES, "barrier area too small");
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < TC_MAX_STAGES; ++s) { mbar_init(bar_full(s), 1); mbar_init(bar_empty(s), CL2 ? 2 : 1); }
+        for (int s = 0; s < TC_MAX_STAGES; ++s) { mbar_init(bar_full(s), 1); mbar_init(bar_empty(s), 1); }
         // one per 32-column A chunk.  3-term modes produce chunks 0 and 1 in 16-column steps by all 8 warps
         // (short first hand-off); every other chunk is written by the 4 warps of one column half.
         // Fast mode (kslab 2) hands over 64-column chunks written by all 8 warps.
@@ -322,22 +311,12 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
     __syncthreads();
     tc_fence_after_sync();
     const uint32_t tmem_base = *tmem_slot;
-    if (CL2) cluster_sync_all();          // the peer's barriers exist before any multicast copy / commit can reach them
 
     if (warp == TC_WARP_PRODUCER) {
         // =========================================================== weight producer (converged warp)
         int stage = 0;
         uint32_t phase = 0, bphase = 0;
         TcTrace<TRACE> tr; tr.init(lane == 0 ? P.trace : nullptr, 0);
-        // one slab -> one ring stage: the whole slab, or (CL2) this CTA's half of it into both CTAs of the pair
-        auto ring_copy = [&](uint32_t dst, const uint8_t* src, uint32_t bytes, uint32_t bar) {
-            if (CL2) {
-                const uint32_t half = bytes >> 1;
-                bulk_g2s_multicast(dst + cta_rank * half, src + cta_rank * half, half, bar, (uint16_t)3);
-            } else {
-                bulk_g2s(dst, src, bytes, bar);
-            }
-        };
         for (long long iter = 0; iter < my_iters; ++iter) {
             for (int gi = 0; gi < P.n_groups; ++gi) {
                 const uint32_t bytes = (uint32_t)P.g[gi].N * (TC_SLAB_K * 2);
@@ -376,12 +355,12 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                                 if (!(nparts == 2 && P.n_stages >= 4 && part == 1)) mbar_arrive(bar_full(stage));
                             } else if (nparts == 2 && P.n_stages >= 4) {
                                 if (part == 0) mbar_arrive_expect_tx(pair_bar, 2 * bytes);
-                                ring_copy(stage_addr(stage), src + (size_t)(it * 2 + part) * bytes, bytes, pair_bar);
+                                bulk_g2s(stage_addr(stage), src + (size_t)(it * 2 + part) * bytes, bytes, pair_bar);
                             } else {
                                 mbar_arrive_expect_tx(bar_full(stage), bytes * kslab);
                                 for (int hs = 0; hs < kslab; ++hs)
-                                    ring_copy(stage_addr(stage) + hs * TC_STAGE_BYTES,
-                                              src + (size_t)((it * kslab + hs) * 2 + part) * bytes, bytes, bar_full(stage));
+                                    bulk_g2s(stage_addr(stage) + hs * TC_STAGE_BYTES,
+                                             src + (size_t)((it * kslab + hs) * 2 + part) * bytes, bytes, bar_full(stage));
                             }
                         }
                         __syncwarp();
@@ -404,11 +383,6 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
         const uint64_t da_ones = umma_smem_desc(sbase + P.off_ones, TC_A_LBO, 128);
         constexpr uint32_t KSTEP_A = (2 * TC_A_LBO) >> 4;            // one K=16 step of A
         constexpr uint32_t STAGE_STEP = TC_STAGE_BYTES >> 4;
-        // ring stage released: locally, or (CL2) in both CTAs of the pair -- the peer's producer writes into this CTA too
-        auto release = [&](uint32_t bar) {
-            if (CL2) umma_commit_multicast(bar, (uint16_t)3);
-            else umma_commit(bar);
-        };
         for (long long iter = 0; iter < my_iters; ++iter) {
             for (int gi = 0; gi < P.n_groups; ++gi) {
                 const uint32_t gN = P.g[gi].N;
@@ -494,15 +468,15 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                             mma_a(true, 1, db + kstep_b, 1);
                             if (!three) {
                                 if (last) umma_commit(bar_accfull(buf));
-                                release(bar_empty(hi_stage));
+                                umma_commit(bar_empty(hi_stage));
                             } else {
-                                release(bar_empty(hi_stage));           // release the hi stage early (64 KB ring)
+                                umma_commit(bar_empty(hi_stage));       // release the hi stage early (64 KB ring)
                                 if (merged) {
                                     const uint64_t dl = (db0 & ~0x3FFFull) | ((stage_addr(stage) & 0x3FFFFu) >> 4);
                                     mma_a(false, 0, dl, 1);              // Ah*Wl
                                     mma_a(false, 1, dl + kstep_b, 1);
                                     if (last) umma_commit(bar_accfull(buf));
-                                    release(bar_empty(stage));
+                                    umma_commit(bar_empty(stage));
                                 }
                             }
                         }
@@ -518,7 +492,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                                     mma_a(false, 0, dl, 1);
                                     mma_a(false, 1, dl + kstep_b, 1);
                                     if (last) umma_commit(bar_accfull(buf));
-                                    release(bar_empty(stage));
+                                    umma_commit(bar_empty(stage));
                                 }
                                 __syncwarp();
                             }
@@ -553,7 +527,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     // ---- now the draining commit(s)
                     if (elect_one_sync()) {
                         if (last) umma_commit(bar_accfull(buf));
-                        release(bar_empty(hi_stage));
+                        umma_commit(bar_empty(hi_stage));
                     }
                     __syncwarp();
                 };
@@ -604,7 +578,6 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
         };
         float4 nx_in = make_float4(0.f, 0.f, 0.f, 0.f);   // pred mode: the probe (x, y, z, foc_z) of this row
         auto fetch_dz = [&](long long tile, float& d, float& f) {
-            if (CL2 && tile >= P.n_tiles) { d = 0.f; f = 0.f; }      // dummy tile of a pair: any finite input will do
             if (tile < P.n_tiles) {
                 if constexpr (PRED) {
                     const long long m = tile * TC_M + row;
@@ -769,12 +742,11 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
 
         long long tile = blockIdx.x;
         for (long long iter = 0; iter < my_iters; ++iter, tile += gridDim.x) {
-            const bool dummy = CL2 && tile >= P.n_tiles;    // this CTA only keeps its pair's ring in step
             int n = 0, s = 0, h0 = 0, w0 = 0;
-            if constexpr (!PRED) tile_coords(dummy ? 0 : tile, n, s, h0, w0);
+            if constexpr (!PRED) tile_coords(tile, n, s, h0, w0);
             const int h = h0 + ty, w = w0 + tx;
             const long long m_row = tile * TC_M + row;      // pred mode: probe index of this thread's row
-            const bool valid = PRED ? (m_row < P.n_probes) : ((h < ra.H) && (w < ra.W) && !dummy);
+            const bool valid = PRED ? (m_row < P.n_probes) : ((h < ra.H) && (w < ra.W));
             tr.ev(0x800);                                // tile start (its layer 0 is already done)
             fetch_dz(tile + gridDim.x, nx_depth, nx_foc);    // depth / focus of the next tile, used by layer0 below
 
@@ -788,7 +760,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
             const float* img_n = ra.img + ((long long)n * ra.Ctot + ra.c0) * ra.H * ra.W;
             const long long cstride = (long long)ra.H * ra.W;
             auto halo_fetch = [&](int idx, float4& v) -> int {       // returns the smem slot or -1
-                if (PRED || dummy || idx >= HH * HW) return -1;
+                if (PRED || idx >= HH * HW) return -1;
                 const int yy = idx / HW, xx = idx - yy * HW;
                 const int gy = min(max(h0 + yy - r, 0), ra.H - 1), gx = min(max(w0 + xx - r, 0), ra.W - 1);
                 const float* px = img_n + (long long)gy * ra.W + gx;
@@ -890,7 +862,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     }
                 }
             }
-            for (int idx = P.n_hidden * TC_EPI_THREADS + et; !PRED && !dummy && idx < HH * HW; idx += TC_EPI_THREADS) {   // remainder
+            for (int idx = P.n_hidden * TC_EPI_THREADS + et; !PRED && idx < HH * HW; idx += TC_EPI_THREADS) {   // remainder
                 float4 hv;
                 const int hslot = halo_fetch(idx, hv);
                 s_halo_t[hslot] = hv;
@@ -1074,7 +1046,6 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
 
     tc_fence_before_sync();
     __syncthreads();
-    if (CL2) cluster_sync_all();          // no CTA leaves while its peer's copies / commits may still target it
     if (warp == TC_WARP_PRODUCER) tmem_dealloc<512>(tmem_base);
 }
 

@@ -3,184 +3,14 @@
 // lives in HBM ([N,H,W,ks,ks] fp32).  HBM-bound on the PSF read: 4*ks^2 B per pixel
 // (484 B at ks = 11) against 12 B of image and 12 B of output.
 //
-// local_psf_stream_kernel (the fast path, needs W % 4 == 0 and 16-byte aligned psf):
-//   CTA tile = 8 rows x 32 columns; the replicate-clamped image halo of the tile sits in
-//   shared memory.  Each of the 8 warps owns one 32-pixel row strip and streams its PSFs
-//   through a private 16 KB buffer with cp.async.bulk + mbarrier (a pixel's taps are
-//   contiguous, so P pixels are ONE contiguous copy; P = 32 at ks <= 11, 4 at ks = 31).
-//   Eight independent warps keep ~124 KB of reads in flight per SM.  Inside a chunk
-//   32/P lanes share a pixel and split its taps; lanes of different pixels are ks^2
-//   floats apart (odd stride -> no bank conflicts).
-// local_psf_render_kernel (generic fallback: any W, any alignment): one warp per 32 pixels,
-//   taps staged through shared memory with plain coalesced loads, image through L1.
+// local_psf_render_kernel is the generic kernel (any ks, any W, any alignment): one warp per 32 pixels, taps staged
+// through shared memory with plain coalesced loads, image through L1.  Odd ks in 3..31 run the strip-walking or the
+// register-streaming kernel instead (gather_strip_kernel.cuh, gather_coalesced_kernel.cuh).
 #pragma once
 #include <cuda_runtime.h>
-#include "ptx_sm100.cuh"
 
 namespace aadff {
 
-constexpr int GS_TILE_H_1BUF = 8;               // warps per CTA (= tile rows), one 16 KB chunk buffer per warp
-constexpr int GS_TILE_H_2BUF = 6;               // warps per CTA with two chunk buffers per warp
-constexpr int GS_TILE_W = 32;
-constexpr int GS_BUF_BYTES = 16384;             // per-warp PSF chunk buffer
-constexpr int GS_MAXC = 4;
-
-template <int NW>      // warps per CTA = tile rows
-__global__ void __launch_bounds__(NW * 32, 1)
-local_psf_stream_kernel(const float* __restrict__ img, const float* __restrict__ psf, float* __restrict__ out,
-                        int N, int C, int H, int W, int ks, int c0, int cn, int P /*pixels per chunk*/,
-                        int nbuf /*1 or 2 chunk buffers per warp*/, int buf_bytes /*per chunk buffer*/) {
-    constexpr int GS_TILE_H = NW;
-    extern __shared__ __align__(128) uint8_t gsm[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int kk = ks * ks, r = (ks - 1) / 2;
-    const int HH = GS_TILE_H + ks - 1, HW = GS_TILE_W + ks - 1;
-    const int pitch = HW | 1;                                  // odd pitch: row-to-row bank skew
-    const int buf_floats = buf_bytes / 4;
-    float* s_psf = reinterpret_cast<float*>(gsm) + warp * nbuf * buf_floats;
-    float* s_img = reinterpret_cast<float*>(gsm + (size_t)GS_TILE_H * nbuf * buf_bytes);    // [cn][HH][pitch]
-    const uint32_t bar = smem_u32(gsm + (size_t)GS_TILE_H * nbuf * buf_bytes + (size_t)GS_MAXC * HH * pitch * 4) + 16u * warp;
-    if (lane == 0) { mbar_init(bar, 1); mbar_init(bar + 8, 1); }
-    fence_mbar_init();
-    __syncthreads();
-
-    const int LPP = 32 / P;                                     // lanes per pixel
-    const int pl = lane / LPP, sub = lane - pl * LPP;
-    const int tiles_x = (W + GS_TILE_W - 1) / GS_TILE_W, tiles_y = (H + GS_TILE_H - 1) / GS_TILE_H;
-    const long long n_tiles = (long long)N * tiles_x * tiles_y;
-
-    // this warp's strip of a tile: row h = tile row * 8 + warp, up to 32 pixels starting at w0
-    auto strip_of = [&](long long tile, const float*& strip, int& npx) -> bool {
-        if (tile >= n_tiles) return false;
-        const int tx = (int)(tile % tiles_x), ty = (int)((tile / tiles_x) % tiles_y);
-        const int n = (int)(tile / ((long long)tiles_x * tiles_y));
-        const int h = ty * GS_TILE_H + warp, w0 = tx * GS_TILE_W;
-        if (h >= H) return false;
-        npx = min(GS_TILE_W, W - w0);                           // multiple of 4 (W % 4 == 0)
-        strip = psf + ((long long)(n * H + h) * W + w0) * kk;
-        return true;
-    };
-    // chunk queue of this warp: (tile, p0) in processing order; `issue` sends the copy of the chunk that
-    // follows (q_tile, q_p0) -- possibly the first chunk of a later tile -- into buffer `b`
-    uint32_t phase_bits = 0;
-    int fill = 0;                                               // buffer the next issued chunk goes to
-    long long q_tile = blockIdx.x;
-    int q_p0 = 0;
-    bool q_valid = false;
-    auto advance_queue = [&]() {                                // position (q_tile, q_p0) on the next chunk to issue
-        const float* st;
-        int npx;
-        while (q_tile < n_tiles) {
-            if (strip_of(q_tile, st, npx) && q_p0 < npx) { q_valid = true; return; }
-            q_tile += gridDim.x;
-            q_p0 = 0;
-        }
-        q_valid = false;
-    };
-    auto issue_next = [&]() {
-        if (!q_valid) return;
-        const float* st;
-        int npx;
-        strip_of(q_tile, st, npx);
-        const uint32_t bytes = (uint32_t)min(P, npx - q_p0) * kk * 4;
-        if (lane == 0) {
-            mbar_arrive_expect_tx(bar + 8 * fill, bytes);
-            bulk_g2s(smem_u32(s_psf + fill * buf_floats), st + (long long)q_p0 * kk, bytes, bar + 8 * fill);
-        }
-        fill = (fill + 1) % nbuf;
-        q_p0 += P;
-        advance_queue();
-    };
-    advance_queue();
-    issue_next();                                               // first chunk goes out before any halo work
-    int use = 0;                                                // buffer the next processed chunk sits in
-
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int tx = (int)(tile % tiles_x), ty = (int)((tile / tiles_x) % tiles_y);
-        const int n = (int)(tile / ((long long)tiles_x * tiles_y));
-        const int h0 = ty * GS_TILE_H, w0 = tx * GS_TILE_W;
-        const int h = h0 + warp;
-        const int npx = min(GS_TILE_W, W - w0);
-        const bool row_ok = h < H;
-        __syncthreads();                                        // previous tile's halo no longer in use
-        {   // halo: loads are issued four at a time before their stores so that the L2 latencies overlap
-            const int total = cn * HH * HW;
-            for (int base = threadIdx.x; base < total; base += 4 * GS_TILE_H * 32) {
-                float v[4];
-                int slot[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int idx = base + u * GS_TILE_H * 32;
-                    slot[u] = -1;
-                    if (idx < total) {
-                        const int c = idx / (HH * HW), rem = idx - c * (HH * HW);
-                        const int yy = rem / HW, xx = rem - yy * HW;
-                        const int gy = min(max(h0 + yy - r, 0), H - 1), gx = min(max(w0 + xx - r, 0), W - 1);
-                        v[u] = __ldg(img + ((long long)(n * C + c0 + c) * H + gy) * W + gx);
-                        slot[u] = (c * HH + yy) * pitch + xx;
-                    }
-                }
-#pragma unroll
-                for (int u = 0; u < 4; ++u)
-                    if (slot[u] >= 0) s_img[slot[u]] = v[u];
-            }
-        }
-        __syncthreads();
-        if (!row_ok) continue;
-        for (int p0 = 0; p0 < npx; p0 += P) {
-            const int np = min(P, npx - p0);
-            if (nbuf == 2) issue_next();                        // the other buffer is free: prefetch the next chunk
-            mbar_wait(bar + 8 * use, (phase_bits >> use) & 1);
-            phase_bits ^= 1u << use;
-            const float* chunk = s_psf + use * buf_floats;
-            float acc[GS_MAXC] = {0.f, 0.f, 0.f, 0.f};
-            if (pl < np) {
-                const float* taps = chunk + pl * kk;
-                const float* ib = s_img + warp * pitch + (p0 + pl);
-                const int cstride = HH * pitch;
-                if (LPP == 1) {                                  // one lane per pixel: row / column loops
-                    for (int i = 0; i < ks; ++i) {
-                        const float* trow = taps + i * ks;
-                        const float* prow = ib + i * pitch;
-#pragma unroll 4
-                        for (int j = 0; j < ks; ++j) {
-                            const float tap = trow[j];
-                            acc[0] = fmaf(prow[j], tap, acc[0]);
-                            if (cn > 1) acc[1] = fmaf(prow[j + cstride], tap, acc[1]);
-                            if (cn > 2) acc[2] = fmaf(prow[j + 2 * cstride], tap, acc[2]);
-                            if (cn > 3) acc[3] = fmaf(prow[j + 3 * cstride], tap, acc[3]);
-                        }
-                    }
-                } else {                                         // LPP lanes share a pixel and split its taps
-                    int i = sub / ks, j = sub - i * ks;
-                    for (int t = sub; t < kk; t += LPP) {
-                        const float tap = taps[t];
-                        const float* px = ib + i * pitch + j;
-#pragma unroll
-                        for (int c = 0; c < GS_MAXC; ++c)
-                            if (c < cn) acc[c] = fmaf(px[c * cstride], tap, acc[c]);
-                        j += LPP;
-                        while (j >= ks) { j -= ks; ++i; }
-                    }
-                }
-            }
-            __syncwarp();                                       // everyone is done reading the buffer
-            use = (use + 1) % nbuf;
-            if (nbuf == 1) issue_next();                        // single buffer: refill only now
-            for (int o = LPP >> 1; o > 0; o >>= 1) {
-#pragma unroll
-                for (int c = 0; c < GS_MAXC; ++c) acc[c] += __shfl_xor_sync(0xffffffffu, acc[c], o);
-            }
-            if (sub == 0 && pl < np) {
-#pragma unroll
-                for (int c = 0; c < GS_MAXC; ++c)
-                    if (c < cn) out[((long long)(n * C + c0 + c) * H + h) * W + w0 + p0 + pl] = acc[c];
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------ fallback
 constexpr int GATHER_TT = 128;                  // taps staged per chunk
 constexpr int GATHER_WARPS = 4;                 // warps per CTA
 constexpr int GATHER_MAXC = 4;                  // channels per pass

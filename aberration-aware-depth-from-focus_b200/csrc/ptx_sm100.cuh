@@ -85,25 +85,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uin
         : "memory");
 }
 
-// Half of a 2-CTA cluster's copy: the bytes land at the same CTA-relative offset in BOTH CTAs of the pair and complete
-// the mbarrier at the same CTA-relative offset in both (UBLKCP.S.G.MULTICAST) -- one L2 read feeds two SMs.
-__device__ __forceinline__ void bulk_g2s_multicast(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar,
-                                                   uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-            dst_smem),
-        "l"(src), "r"(bytes), "r"(bar), "h"(cta_mask)
-        : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 // ----------------------------------------------------------------------------- TMEM
 template <int COLS>
 __device__ __forceinline__ void tmem_alloc(uint32_t slot_smem) {
@@ -207,13 +188,6 @@ __device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, ui
 // All previously issued MMAs of this thread complete -> one arrive on the mbarrier.
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-
-// The same, arriving on the mbarrier at this CTA-relative offset in every CTA of `cta_mask` (UTCBAR.MULTICAST).
-__device__ __forceinline__ void umma_commit_multicast(uint32_t bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(cta_mask)
-                 : "memory");
 }
 
 // ----------------------------------------------------------------------------- misc

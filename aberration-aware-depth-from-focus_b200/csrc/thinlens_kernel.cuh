@@ -4,18 +4,23 @@
 // -> normalise -> gather (deeplens/render_psf.py:76-107).  The reference materialises the
 // [N,H,W,k,k] PSF tensor through ~15 elementwise torch kernels; here taps live in registers.
 //
-// CTA tile = 8 rows x 32 columns, one thread per pixel, image halo tile in shared memory, planar per channel,
-// DOUBLE-BUFFERED: the halo of the next tile arrives under the current tile's arithmetic
+// CTA tile = 8 rows x 64 columns, two horizontally adjacent pixels per thread (warp = row, lane j = columns 2j, 2j+1),
+// image halo tile in shared memory, planar per channel, DOUBLE-BUFFERED: the halo of the next tile arrives under the
+// current tile's arithmetic
 //   * as ONE TMA tensor-tile copy (cp.async.bulk.tensor.3d: box = [channels][rows][columns] of the [N*C, H, W] image,
 //     issued by one thread, completion on an mbarrier; the box starts at a 16-byte-aligned column) when the tile's halo
 //     lies inside the image, and
 //   * by per-thread cp.async of the replicate-clamped pixels (render_psf.py:96 pads with mode='replicate', which a
 //     TMA box cannot do: it zero-fills out-of-bounds elements) for tiles that touch the image border, or when the
 //     image does not meet TMA's 16-byte row-pitch rule (W % 4 != 0).
-// The Gaussian is separable: exp(-(dx^2+dy^2)/2s^2) = g(dx) g(dy), so a pixel needs (k+1)/2 + k exponentials instead of
-// k^2 (the first version was bound by two MUFU-class operations per tap: ex2 and an int->float conversion); the disk
-// mask (dx^2+dy^2 < radius^2) is an integer compare against a per-row limit.  Per tap that leaves
-// FMUL + ISETP/FSEL + FADD + 3 FFMA + 3 LDS.
+// The Gaussian is separable: exp(-(dx^2+dy^2)/2s^2) = g(dx) g(dy), so a pixel needs (k+1)/2 exponentials per PSF row
+// pair instead of one per tap; the disk mask (dx^2+dy^2 < radius^2) is an integer compare against a per-row limit.
+//   * the weights of a PSF row depend on |dy| and |dx| only: for each |dy| the (k+1)/2 weights per pixel are formed
+//     once (FMUL + compare/select) and serve the rows -dy and +dy and both signs of dx; the normalising sum is taken
+//     from the same (k+1)/2 values -- nothing but LDS and FFMA is left per tap;
+//   * per PSF row and channel the thread loads ONE (k+1 [+1 for alignment])-wide window with LDS.64 and both pixels
+//     take their k taps from it: (k+3)/2 LDS.64 per 2k FFMA instead of 2k LDS.32.
+// ~5 instructions per tap and pixel, against ~9 for one pixel per thread (FMUL + ISETP/FSEL + FADD + 3 FFMA + 3 LDS).
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -24,7 +29,6 @@
 namespace aadff {
 
 constexpr int TL_TILE_H = 8;
-constexpr int TL_TILE_W = 32;
 constexpr int TL_MAXC = 3;                // channels per launch (RGB); more channels = more passes
 constexpr int TL_NT = TL_TILE_H * 32;
 
@@ -59,186 +63,9 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst_smem, const CUtensorMap
         : "memory");
 }
 
-template <int KS>
-struct ThinLensCfg {
-    static constexpr int R = (KS - 1) / 2;
-    static constexpr int HH = TL_TILE_H + KS - 1;
-    static constexpr int HW = TL_TILE_W + KS - 1;
-    // TMA rules (measured: a box whose first element is not 16-byte aligned in global memory raises "illegal
-    // instruction"): the box starts SH columns left of the halo, at a multiple of 4 floats, and its width is a multiple of 4
-    static constexpr int SH = (4 - R % 4) % 4;
-    static constexpr int BW = (HW + SH + 3) / 4 * 4;     // box / smem row width
-    static constexpr int CSTRIDE = HH * BW;
-    __host__ __device__ static constexpr int BUF_FLOATS(int cn) { return (cn * CSTRIDE + 31) / 32 * 32; }   // 128-byte multiple: TMA destination alignment
-    // Two halo buffers (the next tile's copy runs under this tile's arithmetic) while they are small; large kernels keep
-    // one buffer: at k = 31 two 29 KB buffers left 3 CTAs per SM and the kernel, which lives on resident warps hiding
-    // LDS latency, lost 11 % (measured)
-    static constexpr int NBUF = KS <= 15 ? 2 : 1;
-    __host__ __device__ static constexpr int SMEM_BYTES(int cn) { return NBUF * BUF_FLOATS(cn) * 4 + 128; }  // barriers in front
-};
-
-template <int KS>
-__global__ void __launch_bounds__(TL_NT)
-thinlens_render_kernel(const ThinLensArgs a, const __grid_constant__ CUtensorMap img_map) {
-    using Cfg = ThinLensCfg<KS>;
-    constexpr int R = Cfg::R, HH = Cfg::HH, HW = Cfg::HW, BW = Cfg::BW, SH = Cfg::SH, CSTRIDE = Cfg::CSTRIDE;
-    extern __shared__ __align__(128) unsigned char tl_smem[];
-    float* bufs = reinterpret_cast<float*>(tl_smem + 128);
-    const uint32_t bar0 = smem_u32(tl_smem);             // two mbarriers (one per buffer) in the first 16 bytes
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int tiles_x = (a.W + TL_TILE_W - 1) / TL_TILE_W, tiles_y = (a.H + TL_TILE_H - 1) / TL_TILE_H;
-    const long long n_tiles = (long long)a.N * tiles_x * tiles_y;
-    const bool flip = a.flip_dev ? (*a.flip_dev != 0) : (a.flip != 0);
-    const int buf_floats = Cfg::BUF_FLOATS(a.cn);
-
-    if (threadIdx.x == 0) {
-        mbar_init(bar0, 1);
-        mbar_init(bar0 + 8, 1);
-        fence_mbar_init();
-    }
-    __syncthreads();
-
-    auto coords = [&](long long tile, int& n, int& h0, int& w0) {
-        const int tx = (int)(tile % tiles_x), ty = (int)((tile / tiles_x) % tiles_y);
-        n = (int)(tile / ((long long)tiles_x * tiles_y));
-        h0 = ty * TL_TILE_H;
-        w0 = tx * TL_TILE_W;
-    };
-    auto interior = [&](int h0, int w0) {
-        return a.use_tma && h0 - R >= 0 && w0 - R >= 0 && h0 - R + HH <= a.H && w0 - R + HW <= a.W;
-    };
-    // start the halo copy of `tile` into buffer b
-    auto issue_halo = [&](long long tile, int b) {
-        int n, h0, w0;
-        coords(tile, n, h0, w0);
-        float* dst = bufs + b * buf_floats;
-        if (interior(h0, w0)) {
-            if (threadIdx.x == 0) {
-                mbar_arrive_expect_tx(bar0 + 8 * b, (uint32_t)(a.cn * CSTRIDE * 4));
-                tma_load_3d(smem_u32(dst), &img_map, w0 - R - SH, h0 - R, n * a.C + a.c0, bar0 + 8 * b);
-            }
-        } else {
-            const uint32_t d0 = smem_u32(dst);
-            for (int idx = threadIdx.x; idx < a.cn * HH * HW; idx += TL_NT) {
-                const int c = idx / (HH * HW), rem = idx - c * (HH * HW);
-                const int yy = rem / HW, xx = rem - yy * HW;
-                const int gy = min(max(h0 + yy - R, 0), a.H - 1), gx = min(max(w0 + xx - R, 0), a.W - 1);   // replicate
-                cp_async4(d0 + 4u * (uint32_t)(c * CSTRIDE + yy * BW + xx + SH),
-                          a.img + ((long long)(n * a.C + a.c0 + c) * a.H + gy) * a.W + gx);
-            }
-        }
-    };
-
-    constexpr bool DB = Cfg::NBUF == 2;
-    uint32_t phase = 0;                       // bit b: parity to wait for on buffer b's mbarrier
-    int cur = 0;
-    if (DB && (long long)blockIdx.x < n_tiles) issue_halo(blockIdx.x, 0);
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        int n, h0, w0;
-        coords(tile, n, h0, w0);
-        const int h = h0 + warp, w = w0 + lane;
-        const bool ok = (h < a.H) && (w < a.W);
-        // circle of confusion (ThinLens.coc, psfnet.py:503-511), operation order of the reference
-        float cexp = 0.f, r2 = 0.f;
-        if (ok) {
-            float d = __ldg(a.depth + ((long long)n * a.H + h) * a.W + w);
-            float f = __ldg(a.foc + n);
-            if (flip) { d = -d; f = -f; }
-            d = fminf(fmaxf(d, a.d_lo), a.d_hi);
-            float coc = a.k1 * fabsf(d - f);
-            coc = __fdiv_rn(coc, d);
-            coc = coc * a.foc_len;
-            coc = __fdiv_rn(coc, f - a.foc_len);
-            const float coc_px = fmaxf(__fdiv_rn(coc, a.ps), 0.1f);
-            const float rad = coc_px * 0.5f;
-            r2 = rad * rad;
-            cexp = __fdiv_rn(-0.5f * 1.4426950408889634f, r2);    // exp(-d2/2/r2) = 2^(d2 * cexp)
-        }
-        if (!DB) issue_halo(tile, 0);         // single buffer: released by the barrier that ended the previous tile
-        // this tile's halo has landed (TMA: mbarrier; cp.async: own copies + barrier below makes everyone's visible)
-        if (interior(h0, w0)) {
-            mbar_wait(bar0 + 8 * cur, (phase >> cur) & 1);
-            phase ^= 1u << cur;
-        } else {
-            cp_async_wait_all();
-        }
-        __syncthreads();
-        if (DB && tile + gridDim.x < n_tiles) issue_halo(tile + gridDim.x, cur ^ 1);   // buffer cur^1 was released by the barrier that ended the previous tile
-
-        if (ok) {
-            // separable Gaussian: g[j] = 2^((j-R)^2 * cexp); the disk mask d2 < r2 as an integer compare (d2 is an integer)
-            float g[R + 1];
-#pragma unroll
-            for (int j = 0; j <= R; ++j) g[j] = exp2f((float)((j - R) * (j - R)) * cexp);
-            const int r2c = (r2 >= 4096.f) ? 4096 : (int)ceilf(r2);      // d2 <= 2 R^2 <= 450
-            float acc[TL_MAXC] = {0.f, 0.f, 0.f}, wsum = 0.f;
-            const float* ib = bufs + cur * buf_floats + warp * BW + lane + SH;
-            // absent channels re-read channel 0 (results discarded at the store): unconditional loads keep the tap loop
-            // free of branches (`if (cn > 1) ... prow[j + CSTRIDE]` compiled to a branch per tap and channel)
-            const int cs1 = a.cn > 1 ? CSTRIDE : 0, cs2 = a.cn > 2 ? 2 * CSTRIDE : 0;
-#pragma unroll 1
-            for (int i = 0; i < KS; ++i) {
-                const int dy2 = (i - R) * (i - R);
-                const float gi = exp2f((float)dy2 * cexp);
-                const int lim = r2c - dy2;                     // tap (i, j) is inside the disk iff (j-R)^2 < lim
-                const float* prow = ib + i * BW;
-                const float* prow1 = prow + cs1;
-                const float* prow2 = prow + cs2;
-#pragma unroll
-                for (int j = 0; j < KS; ++j) {
-                    const int dx2 = (j - R) * (j - R);
-                    const float gj = g[j <= R ? j : KS - 1 - j];
-                    const float wt = (dx2 < lim) ? gi * gj : 0.f;   // psf_mask = (x^2 + y^2 < radius^2)
-                    wsum += wt;
-                    acc[0] = fmaf(prow[j], wt, acc[0]);
-                    acc[1] = fmaf(prow1[j], wt, acc[1]);
-                    acc[2] = fmaf(prow2[j], wt, acc[2]);
-                }
-            }
-            const float inv = __fdiv_rn(1.0f, wsum);            // the centre tap always passes the mask: wsum >= 1
-#pragma unroll
-            for (int c = 0; c < TL_MAXC; ++c)
-                if (c < a.cn) a.out[((long long)(n * a.C + a.c0 + c) * a.H + h) * a.W + w] = acc[c] * inv;
-        }
-        __syncthreads();                                        // everyone is done reading buffer `cur`
-        if (DB) cur ^= 1;
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// Two pixels per thread (round 2, second version).  The one-pixel kernel above is issue-bound: per tap and pixel it
-// spends 3 LDS + 3 FFMA + FMUL + ISETP/FSEL + FADD.  Here a thread owns two horizontally adjacent pixels:
-//   * the weights of a PSF row depend on |dy| and |dx| only: for each |dy| the (k+1)/2 weights per pixel are formed
-//     once (FMUL + compare/select) and serve the rows -dy and +dy and both signs of dx; the normalising sum is taken
-//     from the same (k+1)/2 values -- nothing but LDS and FFMA is left per tap;
-//   * per PSF row and channel the thread loads ONE (k+1 [+1 for alignment])-wide window with LDS.64 and both pixels
-//     take their k taps from it: (k+3)/2 LDS.64 per 2k FFMA instead of 2k LDS.32.
-// CTA tile = 8 rows x 64 columns (warp = row, lane j = columns 2j, 2j+1); halo staging (TMA box / clamped cp.async,
-// double-buffered) as above.  ~5 instead of ~9 instructions per tap and pixel.
 constexpr int TL2_TILE_W = 64;
-#ifndef AADFF_TL2_FFMA2
-#define AADFF_TL2_FFMA2 0         // 1: packed fma.rn.f32x2 (FFMA2, sm_100) over the aligned pairs of a window: built, same results, measured
-                                  // not to pay (k = 11: 21.96 against 22.27 Gpix/s; k = 31: 4.14 against 5.11 -- the pair-building MOVs and
-                                  // 148 registers cost more than the halved FFMA count saves), profiles/NOTES_r02.md
-#endif
-__device__ __forceinline__ unsigned long long tl_pack2(float x, float y) {
-    unsigned long long r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(x), "f"(y));
-    return r;
-}
-__device__ __forceinline__ void tl_unpack2(unsigned long long v, float& x, float& y) {
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(x), "=f"(y) : "l"(v));
-}
-__device__ __forceinline__ unsigned long long tl_ffma2(unsigned long long a, unsigned long long b, unsigned long long c) {
-    unsigned long long r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
 #ifndef AADFF_TL2_MINB
 #define AADFF_TL2_MINB 1          // resident CTAs per SM the register allocation aims at
-#endif
-#ifndef AADFF_TL2_UNROLL_SIDE
-#define AADFF_TL2_UNROLL_SIDE 1   // 1: rows -dy and +dy as straight-line code (windows of one under the FFMAs of the other)
 #endif
 
 template <int KS>
@@ -246,14 +73,19 @@ struct ThinLens2Cfg {
     static constexpr int R = (KS - 1) / 2;
     static constexpr int HH = TL_TILE_H + KS - 1;
     static constexpr int HW = TL2_TILE_W + KS - 1;
-    static constexpr int SH = (4 - R % 4) % 4;                  // box starts at a 16-byte aligned column (see above)
+    // TMA rules (measured: a box whose first element is not 16-byte aligned in global memory raises "illegal
+    // instruction"): the box starts SH columns left of the halo, at a multiple of 4 floats, and its width is a multiple of 4
+    static constexpr int SH = (4 - R % 4) % 4;
     static constexpr int WOFF = SH & 1;                         // LDS.64 windows start at an even float index
     static constexpr int NLD = (WOFF + KS + 1 + 1) / 2;         // float2 loads per window
     static constexpr int BW = (HW + SH + 1 + 3) / 4 * 4;        // one spare column: the last window may read one float past the halo
     static constexpr int CSTRIDE = HH * BW;
-    __host__ __device__ static constexpr int BUF_FLOATS(int cn) { return (cn * CSTRIDE + 31) / 32 * 32; }
+    __host__ __device__ static constexpr int BUF_FLOATS(int cn) { return (cn * CSTRIDE + 31) / 32 * 32; }   // 128-byte multiple: TMA destination alignment
+    // Two halo buffers (the next tile's copy runs under this tile's arithmetic) while they are small; large kernels keep
+    // one buffer: at k = 31 two 29 KB buffers left 3 CTAs per SM and the kernel, which lives on resident warps hiding
+    // LDS latency, lost 11 % (measured)
     static constexpr int NBUF = KS <= 15 ? 2 : 1;
-    __host__ __device__ static constexpr int SMEM_BYTES(int cn) { return NBUF * BUF_FLOATS(cn) * 4 + 128; }
+    __host__ __device__ static constexpr int SMEM_BYTES(int cn) { return NBUF * BUF_FLOATS(cn) * 4 + 128; }  // barriers in front
 };
 
 template <int KS>
@@ -367,18 +199,10 @@ thinlens_render2_kernel(const ThinLensArgs a, const __grid_constant__ CUtensorMa
 #pragma unroll
                 for (int d = 0; d <= R; ++d) g[p][d] = exp2f((float)(d * d) * cexp[p]);
             float acc[2][TL_MAXC], wsum[2] = {0.f, 0.f};
-#if AADFF_TL2_FFMA2
-            unsigned long long acc2[2][TL_MAXC];            // (even-element, odd-element) partial sums
-#endif
 #pragma unroll
             for (int p = 0; p < 2; ++p)
 #pragma unroll
-                for (int c = 0; c < TL_MAXC; ++c) {
-                    acc[p][c] = 0.f;
-#if AADFF_TL2_FFMA2
-                    acc2[p][c] = 0ull;
-#endif
-                }
+                for (int c = 0; c < TL_MAXC; ++c) acc[p][c] = 0.f;
             const float* ib = bufs + cur * buf_floats + warp * BW + (SH - WOFF) + 2 * lane;
             // absent channels re-read channel 0 (results discarded at the store): no branches in the tap loop
             const int cs[TL_MAXC] = {0, a.cn > 1 ? CSTRIDE : 0, a.cn > 2 ? 2 * CSTRIDE : 0};
@@ -399,53 +223,11 @@ thinlens_render2_kernel(const ThinLensArgs a, const __grid_constant__ CUtensorMa
                     rs = fmaf(2.f, rs, wt[p][0]);
                     wsum[p] += (da == 0) ? rs : 2.f * rs;
                 }
-#if AADFF_TL2_FFMA2
-                unsigned long long wp[2][NLD];                  // packed weights of the aligned window pairs
 #pragma unroll
-                for (int p = 0; p < 2; ++p)
-#pragma unroll
-                    for (int l = 0; l < NLD; ++l) {
-                        const int j0 = 2 * l - WOFF - p, j1 = j0 + 1;          // taps of window elements 2l, 2l+1
-                        const int d0 = j0 <= R ? R - j0 : j0 - R, d1 = j1 <= R ? R - j1 : j1 - R;
-                        wp[p][l] = (j0 >= 0 && j1 < KS) ? tl_pack2(wt[p][d0], wt[p][d1]) : 0ull;
-                    }
-#endif
-#if AADFF_TL2_UNROLL_SIDE
-#pragma unroll
-#else
-#pragma unroll 1
-#endif
-                for (int side = 0; side < 2; ++side) {
+                for (int side = 0; side < 2; ++side) {      // rows -dy and +dy, straight-line
                     if (side == 1 && da == 0) break;
                     const int i = side ? R + da : R - da;
                     const float* prow = ib + i * BW;
-#if AADFF_TL2_FFMA2
-                    // window element a = WOFF + p + j holds tap j of pixel p.  The aligned pairs (2l, 2l+1) that lie
-                    // inside a pixel's tap range take one FFMA2 against the packed weights (wt[|j-R|], wt[|j+1-R|]);
-                    // the odd element at either end takes a scalar FFMA.
-#pragma unroll
-                    for (int c = 0; c < TL_MAXC; ++c) {
-                        const float2* pw = reinterpret_cast<const float2*>(prow + cs[c]);
-                        float2 win2[NLD];
-#pragma unroll
-                        for (int l = 0; l < NLD; ++l) win2[l] = pw[l];
-#pragma unroll
-                        for (int p = 0; p < 2; ++p) {
-                            const int a_lo = WOFF + p, a_hi = a_lo + KS - 1;
-#pragma unroll
-                            for (int l = 0; l < NLD; ++l) {
-                                const int a0 = 2 * l, a1 = 2 * l + 1;
-                                if (a0 >= a_lo && a1 <= a_hi) {
-                                    acc2[p][c] = tl_ffma2(tl_pack2(win2[l].x, win2[l].y), wp[p][l], acc2[p][c]);
-                                } else if (a1 == a_lo) {                       // leading single: tap 0
-                                    acc[p][c] = fmaf(win2[l].y, wt[p][R], acc[p][c]);
-                                } else if (a0 == a_hi) {                       // trailing single: tap KS-1
-                                    acc[p][c] = fmaf(win2[l].x, wt[p][R], acc[p][c]);
-                                }
-                            }
-                        }
-                    }
-#else
 #pragma unroll
                     for (int c = 0; c < TL_MAXC; ++c) {
                         const float2* pw = reinterpret_cast<const float2*>(prow + cs[c]);
@@ -462,7 +244,6 @@ thinlens_render2_kernel(const ThinLensArgs a, const __grid_constant__ CUtensorMa
                             for (int j = 0; j < KS; ++j)
                                 acc[p][c] = fmaf(win[WOFF + p + j], wt[p][j <= R ? R - j : j - R], acc[p][c]);
                     }
-#endif
                 }
             }
 #pragma unroll
@@ -470,14 +251,8 @@ thinlens_render2_kernel(const ThinLensArgs a, const __grid_constant__ CUtensorMa
                 if (!ok[p]) continue;
                 const float inv = __fdiv_rn(1.0f, wsum[p]);     // the centre tap always passes the mask: wsum >= 1
 #pragma unroll
-                for (int c = 0; c < TL_MAXC; ++c) {
-#if AADFF_TL2_FFMA2
-                    float ex, ey;
-                    tl_unpack2(acc2[p][c], ex, ey);
-                    acc[p][c] += ex + ey;
-#endif
+                for (int c = 0; c < TL_MAXC; ++c)
                     if (c < a.cn) a.out[((long long)(n * a.C + a.c0 + c) * a.H + h) * a.W + w + p] = acc[p][c] * inv;
-                }
             }
         }
         __syncthreads();

@@ -188,18 +188,14 @@ int aadff_debug_set_desc_swap(int swap);
 int aadff_debug_set_trace(void* device_buffer);
 int aadff_debug_trace_entries(void);
 /* Debug switches, 0 restores normal operation.  What-if timing of the fused kernel (results become invalid):
- * bit 0 = skip the weight copies, bit 1 = skip the operand stores.  32 = AADFF_MODE_FAST through the two-tiles-in-flight kernel
- * (fused_fast2_kernel.cuh; same results, measured slower -- profiles/NOTES_r02.md).
- * 16 = aadff_thinlens_render_f32 fetches every halo tile with
- * clamped cp.async instead of TMA tensor tiles for interior tiles (results unchanged).  8 = run the fused kernel as 2-CTA clusters that share
- * the weight stream through multicast bulk copies (results unchanged; measured not to pay, see profiles/NOTES_r02.md).  Cross-check paths (results stay valid):
- * 128 = aadff_local_psf_render_f32 through the older cp.async.bulk streaming kernel instead of the register-
- * streaming one (128 + 64: with two chunk buffers per warp), 256 = AADFF_MODE_ECON with plainly rounded fp16
- * weights instead of the calibrated ones, 512 = aadff_local_psf_render_f32 through the register-streaming kernel
- * also where the strip-walking kernel would run (ks <= 15, W % 4 == 0); 8192 / 1024 / 4096 = the strip-walking
- * kernel with its shared-memory plan 0 / 1 / 2 forced (default: the widest strips that divide W well),
- * 2048 = aadff_thinlens_render_f32 through the one-pixel-per-thread kernel.  Bits 16..19 (value g > 4): AADFF_MODE_ECON
- * starts its two-term evaluation at layer group g instead of 4 (L5) -- accuracy / speed sweep, generic kernel.      */
+ * 1 = skip the weight copies.  16 = aadff_thinlens_render_f32 fetches every halo tile with clamped cp.async instead of
+ * TMA tensor tiles for interior tiles (results unchanged).  Cross-check paths (results stay valid): 256 =
+ * AADFF_MODE_ECON with plainly rounded fp16 weights instead of the calibrated ones, 512 = aadff_local_psf_render_f32
+ * through the register-streaming kernel also where the strip-walking kernel would run (ks <= 15, W % 4 == 0);
+ * 8192 / 1024 / 4096 = the strip-walking kernel with its shared-memory plan 0 / 1 / 2 forced (default: the widest
+ * strips that divide W well).  Bits 16..19 (value g > 4): AADFF_MODE_ECON starts its two-term evaluation at layer group
+ * g instead of 4 (L5) -- accuracy / speed sweep, generic kernel.  1 << 20 = the fused kernel keeps its A operands in
+ * shared memory also where it would keep them in tensor memory (results unchanged).                                 */
 int aadff_debug_set_flags(int flags);
 /* Host-only: the output-error-calibrated fp16 rounding used by AADFF_MODE_ECON (csrc/econ_calib.h) for one layer.
  * W [N][K], A [NC][K] = sample input activations of the layer, out [N][K] = fp16-representable values.  No GPU. */

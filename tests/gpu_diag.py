@@ -235,7 +235,7 @@ def stage_whatif():
     img, dep = img.cuda(), -dm.cuda() * 1e3
     for mode in ("parity", "fast"):
         lens = _lens(mode=mode)
-        for flags in (0, 1, 2, 3):
+        for flags in (0, 1):
             nat.lib.aadff_debug_set_flags(flags)
             for _ in range(2):
                 lens.render_stack(img, dep, foc)
@@ -289,7 +289,7 @@ def stage_rows():
     for (N, H, W, ks) in [(1, 480, 640, 11), (4, 512, 512, 11), (16, 512, 512, 11), (4, 512, 512, 7), (1, 540, 960, 31)]:
         img = torch.rand(N, 3, H, W, device="cuda")
         psf = torch.rand(N, H, W, ks, ks, device="cuda")
-        for flags in (0,):             # 64 = two chunk buffers per warp with 6 warps (measured slower)
+        for flags in (0,):
             aadff_b200.native.lib.aadff_debug_set_flags(flags)
             ms = timeit(lambda: aadff_b200.local_psf_render(img, psf, ks))
             px = N * H * W

@@ -62,11 +62,6 @@ bgr = torch.randint(0, 255, (2, 96, 130, 3), dtype=torch.uint8, device="cuda")
 d16 = torch.randint(0, 8000, (2, 96, 130), dtype=torch.int16, device="cuda").view(torch.uint16)
 a, d = aadff_b200.preprocess_rgbd(bgr, d16, (40, 56), jitter=torch.tensor([[0.5, 0.1], [-1.0, 0.0]]), flips=torch.tensor([3, 0], dtype=torch.uint8))
 print("preprocess", float(a.mean()), float(d.mean()))
-aadff_b200.native.lib.aadff_debug_set_flags(32)
-print("fast two tiles", float(lens.render_stack(img, dep, foc, mode="fast").mean()))
-aadff_b200.native.lib.aadff_debug_set_flags(8)
-print("cluster multicast", float(lens.render_stack(img, dep, foc, mode="parity").mean()))
-aadff_b200.native.lib.aadff_debug_set_flags(0)
 # ---- round 2, second half: strip-walking gather (every plan; W % 4 == 0, partial strips, runs crossing strips and
 # images), two-pixel thin-lens kernel on odd widths, AutoAgument's spline rotation
 for ks, (n_, h_, w_) in ((11, (2, 19, 68)), (7, (3, 9, 332)), (3, (1, 5, 4)), (13, (1, 33, 132)), (15, (1, 20, 64))):
