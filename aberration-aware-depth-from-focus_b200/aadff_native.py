@@ -105,6 +105,11 @@ def _load() -> ctypes.CDLL:
     lib.aadff_psfnet_pred_tc_f32.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
                                              ctypes.c_int, ctypes.c_void_p]
     lib.aadff_local_psf_render_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
+    lib.aadff_local_psf_render_backward_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
+    lib.aadff_render_psf_map_backward_work_bytes.argtypes = [ctypes.c_int] * 6 + [ctypes.POINTER(ctypes.c_int)] * 2
+    lib.aadff_render_psf_map_backward_work_bytes.restype = ctypes.c_int64
+    lib.aadff_render_psf_map_backward_f32.argtypes = [ctypes.c_void_p] * 6 + [ctypes.c_int64] + [ctypes.c_int] * 6 + \
+                                                     [ctypes.POINTER(ctypes.c_int)] * 2 + [ctypes.c_void_p]
     lib.aadff_debug_umma_gemm.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 3
     lib.aadff_thinlens_render_f32.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_int] * 5 + [ctypes.c_float] * 5 + \
                                              [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
@@ -118,7 +123,8 @@ def _load() -> ctypes.CDLL:
                "aadff_any_negative_f32", "aadff_render_psf_map_f32", "aadff_preprocess_rgbd_u8", "aadff_prepare_planes_u8",
                "aadff_spline_affine_f32", "aadff_resize_planes_f32", "aadff_trainer_create", "aadff_trainer_step",
                "aadff_trainer_read", "aadff_trainer_destroy",
-               "aadff_render_stack_host_f32", "aadff_psfnet_pred_f32", "aadff_psfnet_pred_tc_f32", "aadff_local_psf_render_f32", "aadff_thinlens_render_f32", "aadff_select_focus_f32",
+               "aadff_render_stack_host_f32", "aadff_psfnet_pred_f32", "aadff_psfnet_pred_tc_f32", "aadff_local_psf_render_f32",
+               "aadff_local_psf_render_backward_f32", "aadff_render_psf_map_backward_f32", "aadff_thinlens_render_f32", "aadff_select_focus_f32",
                "aadff_debug_umma_gemm", "aadff_debug_set_desc_swap"):
         getattr(lib, fn).restype = ctypes.c_int
     return lib

@@ -20,6 +20,8 @@
 #include "thinlens_kernel.cuh"
 #include "focus_kernel.cuh"
 #include "psf_conv_kernel.cuh"
+#include "psf_grad_kernel.cuh"
+#include "psf_conv_grad_kernel.cuh"
 #include "train_kernels.cuh"
 #include "preprocess_kernel.cuh"
 #include "spline_rotate_kernel.cuh"
@@ -139,6 +141,79 @@ bool launch_psf_conv(int ks, int grid, cudaStream_t st, const PsfConvArgs& a) {
             return true;
         }
         return launch_psf_conv<KS + 2>(ks, grid, st, a);
+    }
+}
+
+// dP of local_psf_render, strip kernel (psf_grad_kernel.cuh): 3 <= ks <= 15, C <= 4 channels in the halo
+template <int KS, int CN>
+void launch_gps(int sms, cudaStream_t st, const float* img, const float* gout, float* dpsf, int N, int H, int W) {
+    using Cfg = GradPsfStripCfg<KS, CN>;
+    static_assert(Cfg::SMEM_BYTES <= GPS_SMEM && Cfg::NW >= 1, "strip dP: shared memory plan does not fit");
+    if (Cfg::SMEM_BYTES > 48 * 1024)      // per-device attribute: set on every launch that needs the opt-in
+        cudaFuncSetAttribute(local_psf_grad_psf_strip_kernel<KS, CN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             Cfg::SMEM_BYTES);
+    const long long rows = (long long)N * ((W + GSW_PX - 1) / GSW_PX) * H;
+    const int grid = (int)std::min<long long>((rows + Cfg::NW - 1) / Cfg::NW, sms);
+    local_psf_grad_psf_strip_kernel<KS, CN><<<grid, Cfg::NW * 32, Cfg::SMEM_BYTES, st>>>(img, gout, dpsf, N, H, W);
+}
+template <int KS>
+bool launch_gps_ks(int ks, int C, int sms, cudaStream_t st, const float* img, const float* gout, float* dpsf, int N,
+                   int H, int W) {
+    if constexpr (KS > STRIP_MAX_KS) {
+        return false;
+    } else {
+        if (ks == KS) {
+            switch (C) {
+                case 1: launch_gps<KS, 1>(sms, st, img, gout, dpsf, N, H, W); return true;
+                case 2: launch_gps<KS, 2>(sms, st, img, gout, dpsf, N, H, W); return true;
+                case 3: launch_gps<KS, 3>(sms, st, img, gout, dpsf, N, H, W); return true;
+                case 4: launch_gps<KS, 4>(sms, st, img, gout, dpsf, N, H, W); return true;
+                default: return false;
+            }
+        }
+        return launch_gps_ks<KS + 2>(ks, C, sms, st, img, gout, dpsf, N, H, W);
+    }
+}
+
+// dimg of local_psf_render, strip kernel (psf_grad_kernel.cuh): 3 <= ks <= 15, channel passes of 3 or 1
+template <int KS, int CN>
+void launch_gis(int sms, cudaStream_t st, const float* psf, const float* gout, float* dimg, int N, int C, int H, int W,
+                int c0) {
+    using Cfg = GradImgStripCfg<KS, CN>;
+    static_assert(Cfg::SMEM_BYTES <= GPS_SMEM && Cfg::NW >= 1, "strip dimg: shared memory plan does not fit");
+    if (Cfg::SMEM_BYTES > 48 * 1024)
+        cudaFuncSetAttribute(local_psf_grad_img_strip_kernel<KS, CN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             Cfg::SMEM_BYTES);
+    const long long rows = (long long)N * ((W + GSW_PX - 1) / GSW_PX) * H;
+    const int grid = (int)std::min<long long>((rows + Cfg::NW - 1) / Cfg::NW, sms);
+    local_psf_grad_img_strip_kernel<KS, CN><<<grid, Cfg::NW * 32, Cfg::SMEM_BYTES, st>>>(psf, gout, dimg, N, C, H, W, c0);
+}
+template <int KS>
+bool launch_gis_ks(int ks, int cn, int sms, cudaStream_t st, const float* psf, const float* gout, float* dimg, int N,
+                   int C, int H, int W, int c0) {
+    if constexpr (KS > STRIP_MAX_KS) {
+        return false;
+    } else {
+        if (ks == KS) {
+            if (cn == 3) launch_gis<KS, 3>(sms, st, psf, gout, dimg, N, C, H, W, c0);
+            else launch_gis<KS, 1>(sms, st, psf, gout, dimg, N, C, H, W, c0);
+            return true;
+        }
+        return launch_gis_ks<KS + 2>(ks, cn, sms, st, psf, gout, dimg, N, C, H, W, c0);
+    }
+}
+
+// stage 1 of the PSF-map gradient (psf_conv_grad_kernel.cuh), odd ks in 1..31
+template <int KS>
+bool launch_psf_conv_grad_psf(int ks, int grid, cudaStream_t st, const PsfConvArgs& a, const float* gout, float* work) {
+    if constexpr (KS > 31) {
+        return false;
+    } else {
+        if (ks == KS) {
+            psf_conv_grad_psf_kernel<KS><<<grid, PC_NT, 0, st>>>(a, gout, work);
+            return true;
+        }
+        return launch_psf_conv_grad_psf<KS + 2>(ks, grid, st, a, gout, work);
     }
 }
 
@@ -958,6 +1033,54 @@ int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, i
     return AADFF_OK;
 }
 
+int aadff_local_psf_render_backward_f32(const float* img, const float* psf, const float* grad_out, float* grad_img,
+                                        float* grad_psf, int N, int C, int H, int W, int ks, void* stream) {
+    if (!img || !psf || !grad_out || (!grad_img && !grad_psf)) return fail(AADFF_E_INVALID, "null argument");
+    if (N < 0 || C < 1 || H < 1 || W < 1) return fail(AADFF_E_INVALID, "bad shape");
+    if (ks < 1 || (ks % 2) == 0) return fail(AADFF_E_INVALID, "kernel size must be odd and positive");
+    if (N == 0) return AADFF_OK;
+    int dev = 0, sms = 0;
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (grad_psf) {
+        // the forward strip kernel's conditions (aadff_local_psf_render_f32), and all channels in one halo
+        if (ks >= 3 && ks <= STRIP_MAX_KS && C <= GPS_MAXC && W % 4 == 0 &&
+            reinterpret_cast<uintptr_t>(grad_psf) % 16 == 0 && reinterpret_cast<uintptr_t>(grad_out) % 8 == 0 &&
+            (long long)N * H * ((W + 31) / 32) < (1ll << 40)) {
+            if (!launch_gps_ks<3>(ks, C, sms, st, img, grad_out, grad_psf, N, H, W))
+                return fail(AADFF_E_INVALID, "unsupported kernel size");
+        } else {
+            const long long total = (long long)N * H * W * ks * ks;
+            local_psf_grad_psf_kernel<<<(int)std::min<long long>((total + 255) / 256, (long long)sms * 16), 256, 0, st>>>(
+                img, grad_out, grad_psf, N, C, H, W, ks);
+        }
+        g_launches.fetch_add(1);
+        CUDA_TRY(cudaGetLastError());
+    }
+    if (grad_img) {
+        const bool strip = ks >= 3 && ks <= STRIP_MAX_KS && W % 4 == 0 && reinterpret_cast<uintptr_t>(psf) % 16 == 0 &&
+                           (long long)N * H * ((W + 31) / 32) < (1ll << 40);
+        // strip kernel: every pixel without the replicate folds, then rows 0, H-1 and columns 0, W-1 again with them
+        const long long px = (long long)N * (strip ? std::min<long long>((long long)H * W, 2ll * (H + W)) : (long long)H * W);
+        const int grid = (int)std::min<long long>((px + 255) / 256, (long long)sms * 8);
+        for (int c0 = 0; c0 < C;) {
+            const int cn = strip ? ((C - c0 >= 3) ? 3 : 1) : std::min(GPS_MAXC, C - c0);
+            if (strip) {
+                if (!launch_gis_ks<3>(ks, cn, sms, st, psf, grad_out, grad_img, N, C, H, W, c0))
+                    return fail(AADFF_E_INVALID, "unsupported kernel size");
+                g_launches.fetch_add(1);
+                CUDA_TRY(cudaGetLastError());
+            }
+            local_psf_grad_img_kernel<<<grid, 256, 0, st>>>(psf, grad_out, grad_img, N, C, H, W, ks, c0, cn, strip ? 1 : 0);
+            g_launches.fetch_add(1);
+            CUDA_TRY(cudaGetLastError());
+            c0 += cn;
+        }
+    }
+    return AADFF_OK;
+}
+
 int aadff_any_negative_f32(const float* x, int64_t n, unsigned char* flag_dev, void* stream) {
     if (!x || !flag_dev || n < 0) return fail(AADFF_E_INVALID, "bad argument");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1010,17 +1133,17 @@ int aadff_thinlens_render_f32(const float* img, const float* depth, const float*
     return AADFF_OK;
 }
 
-int aadff_render_psf_map_f32(const float* img, const float* psf_map, float* out, int B, int C, int H, int W, int ks,
-                             int grid, const int* row_bounds, const int* col_bounds, void* stream) {
-    if (!img || !psf_map || !out || !row_bounds || !col_bounds) return fail(AADFF_E_INVALID, "null argument");
+}  // extern "C"
+
+// Argument checks shared by aadff_render_psf_map_f32 and its backward (no device call); fills a.
+static int psf_map_args(PsfConvArgs& a, int B, int C, int H, int W, int ks, int grid, const int* row_bounds,
+                        const int* col_bounds) {
     if (B < 0 || C < 1 || H < 1 || W < 1) return fail(AADFF_E_INVALID, "bad shape");
     if (ks < 1 || ks > 31 || (ks % 2) == 0) return fail(AADFF_E_INVALID, "PSF kernel size should be odd (and <= 31)");
     if (grid < 1 || grid > PC_MAX_GRID) return fail(AADFF_E_INVALID, "grid must be in [1, 32]");
     if ((ks - 1) / 2 >= H || (ks - 1) / 2 >= W) return fail(AADFF_E_INVALID, "reflect padding needs (ks-1)/2 < H, W");
-    if (B == 0) return AADFF_OK;
-    PsfConvArgs a{};
-    a.img = img; a.psf_map = psf_map; a.out = out;
     a.B = B; a.C = C; a.H = H; a.W = W; a.grid = grid;
+    a.max_ch = a.max_cw = 0;
     for (int i = 0; i <= grid; ++i) { a.hb[i] = row_bounds[i]; a.wb[i] = col_bounds[i]; }
     if (a.hb[0] != 0 || a.wb[0] != 0 || a.hb[grid] > H || a.wb[grid] > W) return fail(AADFF_E_INVALID, "bad patch bounds");
     for (int i = 0; i < grid; ++i) {
@@ -1028,6 +1151,18 @@ int aadff_render_psf_map_f32(const float* img, const float* psf_map, float* out,
         a.max_ch = std::max(a.max_ch, a.hb[i + 1] - a.hb[i]);
         a.max_cw = std::max(a.max_cw, a.wb[i + 1] - a.wb[i]);
     }
+    return AADFF_OK;
+}
+
+extern "C" {
+
+int aadff_render_psf_map_f32(const float* img, const float* psf_map, float* out, int B, int C, int H, int W, int ks,
+                             int grid, const int* row_bounds, const int* col_bounds, void* stream) {
+    if (!img || !psf_map || !out || !row_bounds || !col_bounds) return fail(AADFF_E_INVALID, "null argument");
+    PsfConvArgs a{};
+    if (int rc = psf_map_args(a, B, C, H, W, ks, grid, row_bounds, col_bounds)) return rc;
+    if (B == 0) return AADFF_OK;
+    a.img = img; a.psf_map = psf_map; a.out = out;
     if (a.max_ch == 0 || a.max_cw == 0) return AADFF_OK;
     int dev = 0, sms = 0;
     CUDA_TRY(cudaGetDevice(&dev));
@@ -1038,6 +1173,63 @@ int aadff_render_psf_map_f32(const float* img, const float* psf_map, float* out,
     if (!launch_psf_conv<1>(ks, nblk, static_cast<cudaStream_t>(stream), a)) return fail(AADFF_E_INVALID, "unsupported kernel size");
     g_launches.fetch_add(1);
     CUDA_TRY(cudaGetLastError());
+    return AADFF_OK;
+}
+
+// Stage-1 partials of the PSF-map gradient: one ks^2 vector per (channel, cell, image, tile of the largest cell).
+static long long psf_map_grad_parts(const PsfConvArgs& a) {
+    return (long long)a.B * ((a.max_ch + PC_TILE_H - 1) / PC_TILE_H) * ((a.max_cw + PC_TILE_W - 1) / PC_TILE_W);
+}
+
+int64_t aadff_render_psf_map_backward_work_bytes(int B, int C, int H, int W, int ks, int grid, const int* row_bounds,
+                                                 const int* col_bounds) {
+    if (!row_bounds || !col_bounds) return fail(AADFF_E_INVALID, "null argument");
+    PsfConvArgs a{};
+    if (int rc = psf_map_args(a, B, C, H, W, ks, grid, row_bounds, col_bounds)) return rc;
+    return (int64_t)C * grid * grid * psf_map_grad_parts(a) * ks * ks * (int64_t)sizeof(float);
+}
+
+int aadff_render_psf_map_backward_f32(const float* img, const float* psf_map, const float* grad_out, float* grad_img,
+                                      float* grad_psf_map, void* work, int64_t work_bytes, int B, int C, int H, int W,
+                                      int ks, int grid, const int* row_bounds, const int* col_bounds, void* stream) {
+    if (!img || !psf_map || !grad_out || !row_bounds || !col_bounds || (!grad_img && !grad_psf_map) ||
+        (grad_psf_map && !work))
+        return fail(AADFF_E_INVALID, "null argument");
+    PsfConvArgs a{};
+    if (int rc = psf_map_args(a, B, C, H, W, ks, grid, row_bounds, col_bounds)) return rc;
+    const int64_t need = (int64_t)C * grid * grid * psf_map_grad_parts(a) * ks * ks * (int64_t)sizeof(float);
+    if (grad_psf_map && work_bytes < need) return fail(AADFF_E_INVALID, "workspace too small");
+    a.img = img; a.psf_map = psf_map; a.out = nullptr;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t psf_bytes = (size_t)C * grid * ks * grid * ks * sizeof(float);
+    if (B == 0 || a.max_ch == 0 || a.max_cw == 0) {                   // no pixel inside a cell: both gradients are 0
+        if (grad_img) CUDA_TRY(cudaMemsetAsync(grad_img, 0, (size_t)B * C * H * W * sizeof(float), st));
+        if (grad_psf_map) CUDA_TRY(cudaMemsetAsync(grad_psf_map, 0, psf_bytes, st));
+        return AADFF_OK;
+    }
+    int dev = 0, sms = 0;
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    if (grad_img) {
+        const long long tiles = (long long)B * C * ((H + PCG_TH - 1) / PCG_TH) * ((W + PCG_TW - 1) / PCG_TW);
+        psf_conv_grad_img_kernel<<<(int)std::min<long long>(tiles, (long long)sms * 8), PC_NT, 0, st>>>(a, grad_out,
+                                                                                                      grad_img, ks);
+        g_launches.fetch_add(1);
+        CUDA_TRY(cudaGetLastError());
+    }
+    if (grad_psf_map) {
+        const long long parts = psf_map_grad_parts(a), tiles = (long long)C * grid * grid * parts;
+        float* ws = static_cast<float*>(work);
+        if (!launch_psf_conv_grad_psf<1>(ks, (int)std::min<long long>(tiles, (long long)sms * 8), st, a, grad_out, ws))
+            return fail(AADFF_E_INVALID, "unsupported kernel size");
+        g_launches.fetch_add(1);
+        CUDA_TRY(cudaGetLastError());
+        const long long warps = (long long)C * grid * grid * ks * ks;
+        psf_conv_grad_reduce_kernel<<<(int)std::min<long long>((warps + 7) / 8, (long long)sms * 16), 256, 0, st>>>(
+            ws, grad_psf_map, C, grid, ks, parts);
+        g_launches.fetch_add(1);
+        CUDA_TRY(cudaGetLastError());
+    }
     return AADFF_OK;
 }
 

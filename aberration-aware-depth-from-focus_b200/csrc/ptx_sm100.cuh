@@ -85,6 +85,21 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uin
         : "memory");
 }
 
+// ----------------------------------------------------------------------------- bulk copy shared -> global
+// Issued by one thread; the writing threads put fence_proxy_async_smem() before the warp/CTA sync that precedes it.
+__device__ __forceinline__ void bulk_s2g(void* dst, uint32_t src_smem, uint32_t bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src_smem), "r"(bytes)
+                 : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most N of this thread's bulk groups still READ their shared-memory source (older slots may be rewritten)
+template <int N>
+__device__ __forceinline__ void bulk_wait_read() {
+    asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
+}
+// every bulk group of this thread has completed (writes included)
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+
 // ----------------------------------------------------------------------------- TMEM
 template <int COLS>
 __device__ __forceinline__ void tmem_alloc(uint32_t slot_smem) {

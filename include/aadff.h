@@ -99,6 +99,11 @@ int aadff_psfnet_pred_tc_f32(aadff_psfnet_t net, const float* inp, float* psf, i
  *   img [N,C,H,W], psf [N,H,W,ks,ks] -> out [N,C,H,W]; device pointers.                        */
 int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, int N, int C, int H, int W, int ks,
                                void* stream);
+/* Backward of aadff_local_psf_render_f32: grad_out [N,C,H,W] -> grad_img [N,C,H,W] and/or grad_psf [N,H,W,ks,ks]
+ * (either may be NULL, not both; img, psf, grad_out must not be).  Outputs are overwritten, not accumulated; no
+ * atomics, so two calls give bit-identical results; stream-ordered, no allocation, CUDA-graph capturable.          */
+int aadff_local_psf_render_backward_f32(const float* img, const float* psf, const float* grad_out, float* grad_img,
+                                        float* grad_psf, int N, int C, int H, int W, int ks, void* stream);
 
 /* Replaces ThinLens.render + ThinLens.coc (deeplens/psfnet.py:503-570), the thin-lens baseline of the paper:
  * circle of confusion -> clipped Gaussian PSF (sigma = coc/2) -> normalise -> per-pixel gather, fused (no PSF
@@ -120,6 +125,16 @@ int aadff_any_negative_f32(const float* x, int64_t n, unsigned char* flag_dev, v
  * left untouched, as in the reference.  ks odd, <= 31; grid <= 32; img, psf_map, out are device pointers.        */
 int aadff_render_psf_map_f32(const float* img, const float* psf_map, float* out, int B, int C, int H, int W, int ks,
                              int grid, const int* row_bounds, const int* col_bounds, void* stream);
+/* Backward of aadff_render_psf_map_f32 (same arguments): grad_out [B,C,H,W] -> grad_img [B,C,H,W] and/or
+ * grad_psf_map [C, grid*ks, grid*ks] (either may be NULL, not both).  `work` is device memory of at least
+ * aadff_render_psf_map_backward_work_bytes(...) bytes (needed only when grad_psf_map != NULL; the library allocates
+ * nothing).  Outputs are overwritten; deterministic; stream-ordered, CUDA-graph capturable.  The size query returns
+ * a negative AADFF_E_* code for arguments the backward would reject.                                             */
+int64_t aadff_render_psf_map_backward_work_bytes(int B, int C, int H, int W, int ks, int grid, const int* row_bounds,
+                                                 const int* col_bounds);
+int aadff_render_psf_map_backward_f32(const float* img, const float* psf_map, const float* grad_out, float* grad_img,
+                                      float* grad_psf_map, void* work, int64_t work_bytes, int B, int C, int H, int W,
+                                      int ks, int grid, const int* row_bounds, const int* col_bounds, void* stream);
 
 /* Replaces the per-sample CPU work of the reference's Dataset classes after file decoding (dff/dataset.py:43-52
  * Matterport3D, :190-205 Middlebury; AutoAgument's colour jitter and flips :259-272): BGR uint8 -> RGB float / 255
