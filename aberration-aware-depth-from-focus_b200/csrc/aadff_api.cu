@@ -1244,11 +1244,12 @@ int aadff_preprocess_rgbd_u8(const uint8_t* bgr, const uint16_t* depth, float* a
     PreprocessArgs a{};
     a.bgr = bgr; a.depth = depth; a.aif_out = bgr ? aif_out : nullptr; a.depth_out = depth ? depth_out : nullptr;
     a.jitter = jitter; a.flips = flips;
-    a.B = B; a.H = H; a.W = W; a.h = h; a.w = w; a.depth_div = depth_div; a.depth_mode = depth_mode;
+    a.B = B; a.H = H; a.W = W; a.h = h; a.w = w; a.depth_div = depth_div;
     const long long per_image = (long long)h * w;
     const dim3 grid((unsigned)std::min<long long>((per_image + 255) / 256, 148 * 16), (unsigned)B);
     if (B > 65535) return fail(AADFF_E_INVALID, "batch too large for one launch");
-    preprocess_rgbd_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    if (depth_mode == 1) preprocess_rgbd_kernel<false, true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    else preprocess_rgbd_kernel<false, false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
     g_launches.fetch_add(1);
     CUDA_TRY(cudaGetLastError());
     return AADFF_OK;
@@ -1304,10 +1305,11 @@ int aadff_resize_planes_f32(const float* planes, float* aif_out, float* depth_ou
     if (B == 0) return AADFF_OK;
     PreprocessArgs a{};
     a.aif_out = aif_out; a.depth_out = depth_out; a.fsrc = planes; a.fsrc_planes = P; a.fsrc_depth_plane = P - 1;
-    a.B = B; a.H = H; a.W = W; a.h = h; a.w = w; a.depth_div = 1.f; a.depth_mode = depth_mode;
+    a.B = B; a.H = H; a.W = W; a.h = h; a.w = w; a.depth_div = 1.f;
     const long long per_image = (long long)h * w;
     const dim3 grid((unsigned)std::min<long long>((per_image + 255) / 256, 148 * 16), (unsigned)B);
-    preprocess_rgbd_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    if (depth_mode == 1) preprocess_rgbd_kernel<true, true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    else preprocess_rgbd_kernel<true, false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
     g_launches.fetch_add(1);
     CUDA_TRY(cudaGetLastError());
     return AADFF_OK;

@@ -28,7 +28,6 @@ struct PreprocessArgs {
     const uint8_t* flips;     // [B] bit 0: horizontal (np.flip axis 1), bit 1: vertical (axis 0); or null
     int B, H, W, h, w;
     float depth_div;
-    int depth_mode;           // 0: antialiased bilinear (torchvision Resize), 1: cv2 INTER_LINEAR
     // alternative source: fp32 planes [B,P,H,W] at full resolution (RGB planes first, then depth) that already carry
     // jitter / flips / rotation (spline_rotate_kernel.cuh); aif_out / depth_out say which outputs are wanted
     const float* fsrc;
@@ -53,7 +52,10 @@ constexpr int PP_MAXW = 12;      // filter taps per axis kept in registers (down
 // grid = (chunks of output pixels, image): a block works on ONE image, so the whole per-value arithmetic of the image --
 // /255 and the colour jitter, both evaluated in double like the reference's numpy code and then rounded to fp32 as its
 // astype('float32') does -- is a 256-entry table in shared memory: per tap and channel one byte load, one LDS, one FFMA.
-template <bool FSRC>      // FSRC: read the fp32 planes `fsrc` instead of the decoded uint8 / uint16 arrays
+// FSRC: read the fp32 planes `fsrc` instead of the decoded uint8 / uint16 arrays.  CV2: resize the depth like
+// cv2.resize INTER_LINEAR instead of the antialiased filter (a template parameter so that its double-precision
+// coordinate arithmetic costs the antialias instantiation no registers)
+template <bool FSRC, bool CV2>
 __global__ void __launch_bounds__(256) preprocess_rgbd_kernel(const PreprocessArgs a) {
     __shared__ float lut[256];
     const int b = blockIdx.y;
@@ -126,7 +128,7 @@ __global__ void __launch_bounds__(256) preprocess_rgbd_kernel(const PreprocessAr
                 return (float)dp[(long long)sy * a.W + sx] / a.depth_div;
             };
             float v = 0.f;
-            if (a.depth_mode == 0) {
+            if (!CV2) {
                 for (int jy = 0; jy < yn; ++jy) {
                     const float wy = aa_weight(jy, ylo, yc, yinv) / wysum;
                     float r = 0.f;
@@ -134,10 +136,15 @@ __global__ void __launch_bounds__(256) preprocess_rgbd_kernel(const PreprocessAr
                     v = fmaf(wy, r, v);
                 }
             } else {
-                // cv2.resize INTER_LINEAR: source coordinate (dst + 0.5) * scale - 0.5, clamped at the borders
-                float fy = ((float)oy + 0.5f) * ((float)a.H / (float)a.h) - 0.5f, fx = ((float)ox + 0.5f) * ((float)a.W / (float)a.w) - 0.5f;
-                int sy = (int)floorf(fy), sx = (int)floorf(fx);
-                fy -= (float)sy; fx -= (float)sx;
+                // cv2.resize INTER_LINEAR on float64 depth (Middlebury): source coordinate (dst + 0.5) * scale - 0.5, its
+                // floor and its fraction in double as OpenCV computes them, clamped at the borders; only the fraction
+                // is rounded to fp32.  An fp32 coordinate has steps of 2.4e-4 px at 2964 columns: millimetres of depth
+                // across a hard depth edge.
+                const double cy = ((double)oy + 0.5) * ((double)a.H / (double)a.h) - 0.5;
+                const double cx = ((double)ox + 0.5) * ((double)a.W / (double)a.w) - 0.5;
+                const double y0 = floor(cy), x0 = floor(cx);
+                int sy = (int)y0, sx = (int)x0;
+                float fy = (float)(cy - y0), fx = (float)(cx - x0);
                 if (sy < 0) { sy = 0; fy = 0.f; }
                 if (sy >= a.H - 1) { sy = a.H - 1; fy = 0.f; }
                 if (sx < 0) { sx = 0; fx = 0.f; }
