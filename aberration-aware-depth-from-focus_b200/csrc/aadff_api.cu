@@ -9,6 +9,8 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/aadff.h"
@@ -42,32 +44,53 @@ int fail(int code, const std::string& msg) {
     return code;
 }
 
-// Template switch of the register-streaming gather: odd ks in 3..31, cn in {1, 3}.
-template <int KS, int CN>
-void launch_gc(int grid, cudaStream_t st, const float* img, const float* psf, float* out, int N, int C, int H, int W,
-               int c0) {
-    constexpr int smem = GatherCfg<KS>::SMEM_FLOATS(CN) * (int)sizeof(float);      // <= 69.6 KB (ks = 31, 3 channels)
-    if (smem > 48 * 1024)      // the attribute is per device: set it on every launch (a host-side table write)
-        cudaFuncSetAttribute(local_psf_coalesced_kernel<KS, CN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    local_psf_coalesced_kernel<KS, CN><<<grid, GC_WARPS * 32, smem, st>>>(img, psf, out, N, C, H, W, c0);
+#define CUDA_TRY(expr)                                                                          \
+    do {                                                                                        \
+        cudaError_t _e = (expr);                                                                \
+        if (_e != cudaSuccess)                                                                  \
+            return fail(AADFF_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));      \
+    } while (0)
+
+// Bits of aadff_debug_set_flags (include/aadff.h documents them).  Bit 1, the fused kernel's what-if without weight
+// copies, is read on the device (TcParams::dbg).
+constexpr int DBG_THINLENS_NO_TMA = 16;
+constexpr int DBG_ECON_PLAIN_ROUNDING = 256;
+constexpr int DBG_NO_STRIP_GATHER = 512;
+constexpr int DBG_STRIP_PLAN1 = 1024, DBG_STRIP_PLAN2 = 4096, DBG_STRIP_PLAN0 = 8192;
+constexpr int DBG_ECON_FIRST_SHIFT = 16;           // bits 16..19: first two-term group of AADFF_MODE_ECON
+constexpr int DBG_SMEM_A_OPERANDS = 1 << 20;
+
+template <int V> constexpr std::integral_constant<int, V> ic{};
+
+// f(ic<KS>) for the odd KS in [LO, HI] equal to ks; returns f's status code
+template <int LO, int HI, class F>
+int with_odd_ks(int ks, F&& f) {
+    if constexpr (LO > HI) return fail(AADFF_E_INVALID, "unsupported kernel size");
+    else return ks == LO ? f(ic<LO>) : with_odd_ks<LO + 2, HI>(ks, std::forward<F>(f));
 }
-template <int KS>
-bool launch_gc_ks(int ks, int cn, int grid, cudaStream_t st, const float* img, const float* psf, float* out, int N, int C,
-                  int H, int W, int c0) {
-    if constexpr (KS > 31) {
-        return false;
-    } else {
-        if (ks == KS) {
-            if (cn == 3) launch_gc<KS, 3>(grid, st, img, psf, out, N, C, H, W, c0);
-            else launch_gc<KS, 1>(grid, st, img, psf, out, N, C, H, W, c0);
-            return true;
-        }
-        return launch_gc_ks<KS + 2>(ks, cn, grid, st, img, psf, out, N, C, H, W, c0);
-    }
+
+int counted_launch() {
+    g_launches.fetch_add(1);
+    CUDA_TRY(cudaGetLastError());
+    return AADFF_OK;
 }
-bool launch_gather_coalesced(int ks, int cn, int grid, cudaStream_t st, const float* img, const float* psf, float* out,
-                             int N, int C, int H, int W, int c0) {
-    return launch_gc_ks<3>(ks, cn, grid, st, img, psf, out, N, C, H, W, c0);
+
+// One counted launch.  The dynamic-shared-memory opt-in is a per-device attribute, so it is set on every launch that
+// needs it (a host-side table write).
+template <class... P, class... A>
+int launch(void (*kernel)(P...), dim3 grid, int block, int smem, cudaStream_t st, A... args) {
+    if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    kernel<<<grid, block, smem, st>>>(args...);
+    return counted_launch();
+}
+
+// SM count (and opt-in shared memory per block) of the current device
+int device_sms(int& sms, int* optin = nullptr) {
+    int dev = 0;
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    if (optin) CUDA_TRY(cudaDeviceGetAttribute(optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    return AADFF_OK;
 }
 
 // Strip-walking gather (gather_strip_kernel.cuh), ks <= 15: slots per warp (SL) / warps per CTA (NW) / strip width
@@ -90,161 +113,16 @@ template <> struct StripPlan<15> { static constexpr StripShape P[3] = {{1, 3, 64
 // or four warps) are bound by the warps' own arithmetic: 0.58 / 0.48 / 0.49 / 0.35 at ks = 17 / 19 / 21 / 23.
 constexpr int STRIP_MAX_KS = 15;
 
-template <int KS, int CN, int SL, int NW, int SPX>
-void launch_gs(int sms, cudaStream_t st, const float* img, const float* psf, float* out, int N, int C, int H, int W,
-               int c0) {
-    constexpr int smem = StripCfg<KS, CN, SPX>::SMEM_BYTES(SL, NW);
-    static_assert(smem <= 232448, "strip gather: shared memory plan does not fit");
-    if (smem > 48 * 1024)      // per-device attribute: set on every launch that needs the opt-in
-        cudaFuncSetAttribute(local_psf_strip_kernel<KS, CN, SL, NW, SPX>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    const long long rows = (long long)N * ((W + SPX - 1) / SPX) * H;
-    const int grid = (int)std::min<long long>((rows + NW - 1) / NW, sms);
-    local_psf_strip_kernel<KS, CN, SL, NW, SPX><<<grid, NW * 32, smem, st>>>(img, psf, out, N, C, H, W, c0);
-}
-template <int KS, int I>
-void launch_gs_plan(int cn, int sms, cudaStream_t st, const float* img, const float* psf, float* out, int N, int C, int H,
-                    int W, int c0) {
-    constexpr StripShape S = StripPlan<KS>::P[I];
-    if (cn == 3) launch_gs<KS, 3, S.SL, S.NW, S.SPX>(sms, st, img, psf, out, N, C, H, W, c0);
-    else launch_gs<KS, 1, S.SL, S.NW, S.SPX>(sms, st, img, psf, out, N, C, H, W, c0);
-}
-template <int KS>
-bool launch_gs_ks(int ks, int cn, int plan, int sms, cudaStream_t st, const float* img, const float* psf, float* out,
-                  int N, int C, int H, int W, int c0) {
-    if constexpr (KS > STRIP_MAX_KS) {
-        return false;
-    } else {
-        if (ks == KS) {
-            if (plan < 0) {                                    // automatic: widest strips that cover W with <= 10 % padding
-                plan = 2;
-                for (int i = 0; i < 3; ++i) {
-                    const int spx = StripPlan<KS>::P[i].SPX;
-                    if ((long long)((W + spx - 1) / spx) * spx * 10 <= (long long)W * 11 || spx <= GSW_PX) { plan = i; break; }
-                }
-            }
-            if (plan == 1) launch_gs_plan<KS, 1>(cn, sms, st, img, psf, out, N, C, H, W, c0);
-            else if (plan == 2) launch_gs_plan<KS, 2>(cn, sms, st, img, psf, out, N, C, H, W, c0);
-            else launch_gs_plan<KS, 0>(cn, sms, st, img, psf, out, N, C, H, W, c0);
-            return true;
-        }
-        return launch_gs_ks<KS + 2>(ks, cn, plan, sms, st, img, psf, out, N, C, H, W, c0);
+// index into StripPlan<KS>::P: forced by a debug flag, else the widest strips that cover W with <= 10 % padding
+int strip_plan(const StripShape (&plans)[3], int W, int dbg) {
+    if (dbg & DBG_STRIP_PLAN1) return 1;
+    if (dbg & DBG_STRIP_PLAN2) return 2;
+    if (dbg & DBG_STRIP_PLAN0) return 0;
+    for (int i = 0; i < 3; ++i) {
+        const int spx = plans[i].SPX;
+        if ((long long)((W + spx - 1) / spx) * spx * 10 <= (long long)W * 11 || spx <= GSW_PX) return i;
     }
-}
-
-template <int KS>
-bool launch_psf_conv(int ks, int grid, cudaStream_t st, const PsfConvArgs& a) {
-    if constexpr (KS > 31) {
-        return false;
-    } else {
-        if (ks == KS) {
-            psf_conv_kernel<KS><<<grid, PC_NT, 0, st>>>(a);
-            return true;
-        }
-        return launch_psf_conv<KS + 2>(ks, grid, st, a);
-    }
-}
-
-// dP of local_psf_render, strip kernel (psf_grad_kernel.cuh): 3 <= ks <= 15, C <= 4 channels in the halo
-template <int KS, int CN>
-void launch_gps(int sms, cudaStream_t st, const float* img, const float* gout, float* dpsf, int N, int H, int W) {
-    using Cfg = GradPsfStripCfg<KS, CN>;
-    static_assert(Cfg::SMEM_BYTES <= GPS_SMEM && Cfg::NW >= 1, "strip dP: shared memory plan does not fit");
-    if (Cfg::SMEM_BYTES > 48 * 1024)      // per-device attribute: set on every launch that needs the opt-in
-        cudaFuncSetAttribute(local_psf_grad_psf_strip_kernel<KS, CN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             Cfg::SMEM_BYTES);
-    const long long rows = (long long)N * ((W + GSW_PX - 1) / GSW_PX) * H;
-    const int grid = (int)std::min<long long>((rows + Cfg::NW - 1) / Cfg::NW, sms);
-    local_psf_grad_psf_strip_kernel<KS, CN><<<grid, Cfg::NW * 32, Cfg::SMEM_BYTES, st>>>(img, gout, dpsf, N, H, W);
-}
-template <int KS>
-bool launch_gps_ks(int ks, int C, int sms, cudaStream_t st, const float* img, const float* gout, float* dpsf, int N,
-                   int H, int W) {
-    if constexpr (KS > STRIP_MAX_KS) {
-        return false;
-    } else {
-        if (ks == KS) {
-            switch (C) {
-                case 1: launch_gps<KS, 1>(sms, st, img, gout, dpsf, N, H, W); return true;
-                case 2: launch_gps<KS, 2>(sms, st, img, gout, dpsf, N, H, W); return true;
-                case 3: launch_gps<KS, 3>(sms, st, img, gout, dpsf, N, H, W); return true;
-                case 4: launch_gps<KS, 4>(sms, st, img, gout, dpsf, N, H, W); return true;
-                default: return false;
-            }
-        }
-        return launch_gps_ks<KS + 2>(ks, C, sms, st, img, gout, dpsf, N, H, W);
-    }
-}
-
-// dimg of local_psf_render, strip kernel (psf_grad_kernel.cuh): 3 <= ks <= 15, channel passes of 3 or 1
-template <int KS, int CN>
-void launch_gis(int sms, cudaStream_t st, const float* psf, const float* gout, float* dimg, int N, int C, int H, int W,
-                int c0) {
-    using Cfg = GradImgStripCfg<KS, CN>;
-    static_assert(Cfg::SMEM_BYTES <= GPS_SMEM && Cfg::NW >= 1, "strip dimg: shared memory plan does not fit");
-    if (Cfg::SMEM_BYTES > 48 * 1024)
-        cudaFuncSetAttribute(local_psf_grad_img_strip_kernel<KS, CN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             Cfg::SMEM_BYTES);
-    const long long rows = (long long)N * ((W + GSW_PX - 1) / GSW_PX) * H;
-    const int grid = (int)std::min<long long>((rows + Cfg::NW - 1) / Cfg::NW, sms);
-    local_psf_grad_img_strip_kernel<KS, CN><<<grid, Cfg::NW * 32, Cfg::SMEM_BYTES, st>>>(psf, gout, dimg, N, C, H, W, c0);
-}
-template <int KS>
-bool launch_gis_ks(int ks, int cn, int sms, cudaStream_t st, const float* psf, const float* gout, float* dimg, int N,
-                   int C, int H, int W, int c0) {
-    if constexpr (KS > STRIP_MAX_KS) {
-        return false;
-    } else {
-        if (ks == KS) {
-            if (cn == 3) launch_gis<KS, 3>(sms, st, psf, gout, dimg, N, C, H, W, c0);
-            else launch_gis<KS, 1>(sms, st, psf, gout, dimg, N, C, H, W, c0);
-            return true;
-        }
-        return launch_gis_ks<KS + 2>(ks, cn, sms, st, psf, gout, dimg, N, C, H, W, c0);
-    }
-}
-
-// stage 1 of the PSF-map gradient (psf_conv_grad_kernel.cuh), odd ks in 1..31
-template <int KS>
-bool launch_psf_conv_grad_psf(int ks, int grid, cudaStream_t st, const PsfConvArgs& a, const float* gout, float* work) {
-    if constexpr (KS > 31) {
-        return false;
-    } else {
-        if (ks == KS) {
-            psf_conv_grad_psf_kernel<KS><<<grid, PC_NT, 0, st>>>(a, gout, work);
-            return true;
-        }
-        return launch_psf_conv_grad_psf<KS + 2>(ks, grid, st, a, gout, work);
-    }
-}
-
-// thinlens_render2_kernel: tile geometry by kernel size
-template <int KS>
-bool thinlens2_geometry(int ks, int cn, int* box_w, int* box_h, int* smem) {
-    if constexpr (KS > 31) {
-        return false;
-    } else {
-        if (ks == KS) {
-            *box_w = ThinLens2Cfg<KS>::BW;
-            *box_h = ThinLens2Cfg<KS>::HH;
-            *smem = ThinLens2Cfg<KS>::SMEM_BYTES(cn);
-            return true;
-        }
-        return thinlens2_geometry<KS + 2>(ks, cn, box_w, box_h, smem);
-    }
-}
-template <int KS>
-bool launch_thinlens2(int ks, int grid, int smem, cudaStream_t st, const ThinLensArgs& a, const CUtensorMap& map) {
-    if constexpr (KS > 31) {
-        return false;
-    } else {
-        if (ks == KS) {
-            if (smem > 48 * 1024)      // per-device attribute
-                cudaFuncSetAttribute(thinlens_render2_kernel<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            thinlens_render2_kernel<KS><<<grid, TL_NT, smem, st>>>(a, map);
-            return true;
-        }
-        return launch_thinlens2<KS + 2>(ks, grid, smem, st, a, map);
-    }
+    return 2;
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda)
@@ -276,13 +154,6 @@ bool make_image_map(CUtensorMap* map, const float* img, long long planes, int H,
                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-
-#define CUDA_TRY(expr)                                                                          \
-    do {                                                                                        \
-        cudaError_t _e = (expr);                                                                \
-        if (_e != cudaSuccess)                                                                  \
-            return fail(AADFF_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));      \
-    } while (0)
 
 struct DeviceGuard {
     int prev = -1;
@@ -334,6 +205,52 @@ void pack_bias_slab(const float* bias, int N, std::vector<__half>& dst) {
         dst[base + (size_t)n * 8 + 0] = hi;
         dst[base + (size_t)n * 8 + 1] = __float2half_rn(bias[n] - __half2float(hi));
     }
+}
+
+// Every specialisation of the fused kernel that launch_tc runs.  aadff_psfnet_create sets their shared-memory opt-in,
+// launch_tc picks one by <TRACE, PRED, UNI, TA> (fused_tc_kernel.cuh).
+using FusedKernel = void (*)(TcParams);
+struct FusedVariant { bool trace, pred; int uni; bool ta; FusedKernel fn; };
+#define FUSED(TR, PR, U, TA) {TR, PR, U, TA, fused_psfnet_render_kernel<TR, PR, U, TA>}
+const FusedVariant FUSED_VARIANTS[] = {
+    FUSED(true, false, 0, false), FUSED(true, false, 0, true),                       // traced render
+    FUSED(false, false, 0, false), FUSED(false, true, 0, false),                      // render / pred, by UNI
+    FUSED(false, false, 1, false), FUSED(false, true, 1, false),
+    FUSED(false, false, 3, false), FUSED(false, true, 3, false),
+    FUSED(false, false, 12, false), FUSED(false, true, 12, false),
+    FUSED(false, false, 13, false), FUSED(false, true, 13, false),
+    FUSED(false, false, 14, false), FUSED(false, true, 14, false),
+    FUSED(false, false, 15, false), FUSED(false, true, 15, false),
+    FUSED(false, false, 12, true), FUSED(false, false, 13, true), FUSED(false, false, 14, true),   // render, TA
+};
+#undef FUSED
+
+// Arithmetic of each mode: the layer groups from `first` on take `terms` MMA terms, the groups before three.  um is
+// the kernel specialisation of that pattern (UNI % 10 in fused_tc_kernel.cuh).
+struct TermPattern { int mode, first, terms, um; };
+constexpr TermPattern TERM_PATTERNS[] = {
+    {AADFF_MODE_PARITY, TC_MAX_GROUPS, 3, 3},           // no group reduced
+    {AADFF_MODE_FAST, 0, 1, 1},
+    {AADFF_MODE_ECON, TC_ECON_FIRST_GROUP, 2, 2},       // L5.. and the head: fp16 weights
+    {AADFF_MODE_ECON8, TC_ECON8_FIRST_GROUP, 2, 4},     // L8, L9 and the head
+    {AADFF_MODE_MIXED, TC_MIXED_FIRST_GROUP, 1, 5},
+};
+static_assert(TC_ECON_FIRST_GROUP == TC_ECON_FIRST_LAYER - 1, "group g holds layer g + 1");
+
+// Shared-memory carve-up of the fused kernel into P's offsets; returns its size.  A operands in shared memory: both
+// A parts (hi, lo), `stages` ring stages, one halo slot.  In tensor memory (ta): the ring, the raw head values of the
+// tile being gathered (stg_bytes), two halo slots.
+uint32_t carve_smem(TcParams& P, bool ta, int stages, uint32_t stg_bytes, uint32_t bias_bytes, uint32_t halo_bytes) {
+    P.off_stage = ta ? 0 : 2 * TC_A_PART_BYTES;
+    P.off_stg = P.off_stage + stages * TC_STAGE_BYTES;
+    P.off_bias = P.off_stg + stg_bytes;
+    P.off_w0 = P.off_bias + bias_bytes;
+    P.off_halo = (P.off_w0 + 320 * 4 + 15u) & ~15u;
+    P.off_red = P.off_halo + (ta ? 2 : 1) * halo_bytes;
+    P.off_bar = P.off_red + TC_M * 5 * 4;
+    P.off_ones = (P.off_bar + TC_BAR_BYTES + 15u) & ~15u;      // constant A operand of the bias slabs
+    P.off_bslab = P.off_ones + 2 * TC_A_LBO;
+    return P.off_bslab + 2 * TC_BSLAB_BYTES;                     // bias-slab slot + its block of zeros
 }
 
 }  // namespace
@@ -601,19 +518,8 @@ int aadff_psfnet_create(const float* const* weights, const float* const* biases,
         if (rc) { aadff_psfnet_destroy(h); return rc; }
         rc = upload(w0b0, &h->d_w0b0);
         if (rc) { aadff_psfnet_destroy(h); return rc; }
-        const int so = h->smem_optin;
-        const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<true, false, 0>, attr, so));
-#define AADFF_SET_ATTR(U)                                                                        \
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, U>, attr, so));   \
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, true, U>, attr, so));
-        AADFF_SET_ATTR(0) AADFF_SET_ATTR(1) AADFF_SET_ATTR(3) AADFF_SET_ATTR(13) AADFF_SET_ATTR(12) AADFF_SET_ATTR(14)
-        AADFF_SET_ATTR(15)
-#undef AADFF_SET_ATTR
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<true, false, 0, true>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 12, true>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 13, true>, attr, so));
-        CREATE_TRY(cudaFuncSetAttribute(fused_psfnet_render_kernel<false, false, 14, true>, attr, so));
+        for (const FusedVariant& v : FUSED_VARIANTS)
+            CREATE_TRY(cudaFuncSetAttribute(v.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
     }
 #undef CREATE_TRY
     *out = h;
@@ -682,6 +588,7 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
         const int rc = ensure_econ(h);
         if (rc) return rc;
     }
+    const int dbg = g_dbg_flags.load();
     TcParams P{};
     P.ra = ra;
     P.wpack = econ_like ? h->d_wpack_econ : h->d_wpack;
@@ -692,21 +599,23 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     P.n_bias = h->n_bias;
     P.bias_skip = h->head_bias0;                               // hidden biases live in the bias slabs
     P.kk = h->kk;
+    TermPattern tp = TERM_PATTERNS[0];
+    for (const TermPattern& p : TERM_PATTERNS)
+        if (p.mode == mode) tp = p;
     // debug flags bits 16..19: first two-term group of AADFF_MODE_ECON for this launch (0 = the shipped pattern, L5 =
-    // group 4; later groups trade speed for accuracy -- tests/gpu_econ_certificate.py sweeps it; runs the generic kernel)
-    const int econ_first_dbg = (g_dbg_flags.load() >> 16) & 15;
-    const int econ_first = (econ_first_dbg > TC_ECON_FIRST_GROUP) ? econ_first_dbg : TC_ECON_FIRST_GROUP;
+    // group 4; later groups trade speed for accuracy -- tests/gpu_econ_certificate.py sweeps it)
+    if (mode == AADFF_MODE_ECON) tp.first = std::max(tp.first, (dbg >> DBG_ECON_FIRST_SHIFT) & 15);
+    if (tp.first >= h->n_groups) tp = TERM_PATTERNS[0];       // no group reduced: the network runs as in parity mode
+    bool any_lo = false, all2 = true, aligned = true;
     for (int i = 0; i < h->n_groups; ++i) {
         P.g[i] = h->groups[i];
-        const bool hidden = i < h->n_hidden;
-        P.g[i].terms = (mode == AADFF_MODE_FAST) ? 1
-                       : (mode == AADFF_MODE_MIXED && i >= TC_MIXED_FIRST_GROUP) ? 1
-                       : (mode == AADFF_MODE_ECON && i >= econ_first) ? 2              // L5.. and the head: fp16 weights
-                       : (mode == AADFF_MODE_ECON8 && i >= TC_ECON8_FIRST_GROUP) ? 2   // L8, L9 and the head
-                       : 3;
-        if (econ_like && P.g[i].terms == 2 && !(g_dbg_flags.load() & 256))
-            P.g[i].w_off = h->w_off_econ[i];                   // calibrated rounding (debug flag 256: plain rounding)
-        (void)hidden;
+        const int t = i >= tp.first ? tp.terms : 3;
+        P.g[i].terms = t;
+        if (econ_like && t == 2 && !(dbg & DBG_ECON_PLAIN_ROUNDING))
+            P.g[i].w_off = h->w_off_econ[i];                   // calibrated rounding
+        any_lo |= t >= 2;
+        all2 &= t >= 2;
+        aligned &= ((P.g[i].K / TC_SLAB_K) * (t == 3 ? 2 : 1)) % 4 == 0;
     }
     P.tiles_x = (ra.W + TC_TILE_W - 1) / TC_TILE_W;
     P.tiles_y = (ra.H + TC_TILE_H - 1) / TC_TILE_H;
@@ -723,137 +632,59 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
         P.n_tiles = (n_probes + TC_M - 1) / TC_M;
     }
     P.trace = g_trace.load();
-    P.dbg = (uint32_t)g_dbg_flags.load();
-    // shared-memory carve-up
+    P.dbg = (uint32_t)dbg;
     uint32_t halo_bytes = (uint32_t)(TC_TILE_H + ra.ks - 1) * TC_HALO_PITCH * 16;          // float4 per pixel
     if (probes != nullptr) halo_bytes = std::max<uint32_t>(halo_bytes, 8 * 32 * 9 * 4);        // pred mode: the store staging lives there
     const uint32_t bias_bytes = (uint32_t)(h->n_bias - h->head_bias0) * 4;                 // head bias only
-    const uint32_t ones_bytes = 2 * TC_A_LBO;                                              // constant A operand of the bias slabs
-    const uint32_t bslab_bytes = 2 * TC_BSLAB_BYTES;                                        // bias-slab slot + its block of zeros
-    const uint32_t fixed = 2 * TC_A_PART_BYTES + bias_bytes + 320 * 4 + halo_bytes + TC_M * 5 * 4 + TC_BAR_BYTES + ones_bytes +
-                           bslab_bytes + 16;
+    // the deepest weight ring (4..2 stages of 16 KB) that fits, 16 bytes held back for the alignment of the carve-up
     int stages = 4;
-    while (stages >= 2 && fixed + (uint32_t)stages * TC_STAGE_BYTES > (uint32_t)h->smem_optin) --stages;
+    uint32_t smem = 0;
+    while (stages >= 2 && (smem = carve_smem(P, false, stages, 0, bias_bytes, halo_bytes)) + 16 > (uint32_t)h->smem_optin)
+        --stages;
     if (stages < 2) return fail(AADFF_E_UNSUPPORTED, "shared memory budget exceeded for this kernel size / channel count");
-    bool any_lo = false;
-    for (int i = 0; i < h->n_groups; ++i) any_lo |= (P.g[i].terms >= 2);
-    P.off_stage = 2 * TC_A_PART_BYTES;
-    P.off_bias = P.off_stage + stages * TC_STAGE_BYTES;
-    P.off_w0 = P.off_bias + bias_bytes;
-    P.off_halo = P.off_w0 + 320 * 4;
-    P.off_red = P.off_halo + halo_bytes;
-    P.off_bar = P.off_red + TC_M * 5 * 4;
-    P.off_ones = (P.off_bar + TC_BAR_BYTES + 15u) & ~15u;
-    P.off_bslab = P.off_ones + ones_bytes;
-    const uint32_t smem = P.off_bslab + bslab_bytes;
     // no layer needs lo operands (fast mode): the A_lo region doubles the ring to 128 KB, organised as four
     // 32 KB stages (two packed K=32 slabs each) so that every issue iteration queues four MMAs
     P.kslab = (!any_lo && stages == 4) ? 2 : 1;
     P.n_stages = (P.kslab == 2) ? 4 : stages;
-    const int grid = (int)std::min<long long>(P.n_tiles, h->num_sms);
-    // kernel specialisation (fused_tc_kernel.cuh, template UNI): pattern 3 = all groups three-term (parity), 1 = all
-    // single-term with the long ring (fast), 2 = econ, 5 = mixed, 0 = per-group terms at run time; +10 when the ring has
-    // four stages and every group consumes a multiple of four of them (ring position of a K-step = compile-time)
-    bool all3 = true, all1 = true, econ_pat = true, econ8_pat = true, mixed_pat = true, aligned = (P.n_stages == 4 && P.kslab == 1);
-    for (int i = 0; i < h->n_groups; ++i) {
-        const int t = P.g[i].terms;
-        all3 &= (t == 3);
-        all1 &= (t == 1);
-        econ_pat &= (t == (i < TC_ECON_FIRST_GROUP ? 3 : 2));
-        econ8_pat &= (t == (i < TC_ECON8_FIRST_GROUP ? 3 : 2));
-        mixed_pat &= (t == (i < TC_MIXED_FIRST_GROUP ? 3 : 1));
-        aligned &= (((P.g[i].K / TC_SLAB_K) * (t == 3 ? 2 : 1)) % 4 == 0);
-    }
-    static_assert(TC_ECON_FIRST_GROUP == TC_ECON_FIRST_LAYER - 1, "group g holds layer g + 1");
-    int uni = 0;
-    if (all3 && P.kslab == 1) uni = aligned ? 13 : 3;
-    else if (all1 && P.kslab == 2) uni = 1;
-    else if (econ_pat && aligned) uni = 12;
-    else if (econ8_pat && aligned && h->n_groups > TC_ECON8_FIRST_GROUP) uni = 14;
-    else if (mixed_pat && aligned) uni = 15;
+    // UNI (fused_tc_kernel.cuh): the specialisation of this launch's term pattern, 0 = per-group terms at run time.
+    // +10 when the ring has four stages and every group consumes a multiple of four of them (ring position of a K-step
+    // = compile-time); the fast pattern needs the long ring, the reduced ones the aligned ring.
+    aligned &= P.n_stages == 4 && P.kslab == 1;
+    int um = 0;
+    for (const TermPattern& p : TERM_PATTERNS)
+        if (p.first == tp.first && p.terms == tp.terms) um = p.um;
+    const int uni = um == 3 ? (aligned ? 13 : 3) : um == 1 ? (P.kslab == 2 ? 1 : 0) : aligned ? 10 + um : 0;
     // A operands in tensor memory (fused_tc_kernel.cuh, TA): render launches of the 2-/3-term specialisations with one
     // head block of N <= 192 (ks <= 13) and at least two hidden layers, 4-stage ring.  Its shared memory holds no
     // activations: ring, raw head values of the tile being gathered, two halo slots.  Debug flag 1 << 20 keeps such
     // launches on the shared-memory path (equality tests, A/B timing).
-    bool all2 = true;
-    for (int i = 0; i < h->n_groups; ++i) all2 &= (P.g[i].terms >= 2);
     const uint32_t head_n = h->groups[h->n_hidden].N;
-    uint32_t smem_launch = smem;
-    const bool ta = P.probes == nullptr && !(P.dbg & (1u << 20)) && h->n_groups == h->n_hidden + 1 &&
+    const bool trace = P.trace != nullptr && P.probes == nullptr;
+    const bool ta = P.probes == nullptr && !(dbg & DBG_SMEM_A_OPERANDS) && h->n_groups == h->n_hidden + 1 &&
                     h->n_hidden >= 2 && head_n <= (uint32_t)TC_TA_L1_COL && P.kslab == 1 && P.n_stages == 4 && all2 &&
                     (uni == 12 || uni == 13 || uni == 14 || P.trace != nullptr);
     if (ta) {
         const uint32_t stg_bytes = ((head_n + 31u) & ~31u) * TC_M * 4;      // the gather reads 32-column blocks
         P.halo_bytes = halo_bytes;
-        P.off_stage = 0;
-        P.off_stg = 4 * TC_STAGE_BYTES;
-        P.off_bias = P.off_stg + stg_bytes;
-        P.off_w0 = P.off_bias + bias_bytes;
-        P.off_halo = (P.off_w0 + 320 * 4 + 15u) & ~15u;
-        P.off_red = P.off_halo + 2 * halo_bytes;
-        P.off_bar = P.off_red + TC_M * 5 * 4;
-        P.off_ones = (P.off_bar + TC_BAR_BYTES + 15u) & ~15u;
-        P.off_bslab = P.off_ones + ones_bytes;
-        smem_launch = P.off_bslab + bslab_bytes;
-        if (smem_launch > (uint32_t)h->smem_optin) return fail(AADFF_E_UNSUPPORTED, "shared memory budget exceeded (TA)");
+        smem = carve_smem(P, true, 4, stg_bytes, bias_bytes, halo_bytes);
+        if (smem > (uint32_t)h->smem_optin) return fail(AADFF_E_UNSUPPORTED, "shared memory budget exceeded (TA)");
     }
-    if (P.trace != nullptr && P.probes == nullptr) {
-        if (ta) fused_psfnet_render_kernel<true, false, 0, true><<<grid, TC_NT, smem_launch, st>>>(P);
-        else fused_psfnet_render_kernel<true, false, 0><<<grid, TC_NT, smem, st>>>(P);
-    } else if (ta) {
-        switch (uni) {
-            case 12: fused_psfnet_render_kernel<false, false, 12, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
-            case 13: fused_psfnet_render_kernel<false, false, 13, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
-            default: fused_psfnet_render_kernel<false, false, 14, true><<<grid, TC_NT, smem_launch, st>>>(P); break;
-        }
-    } else {
-#define AADFF_LAUNCH(U)                                                                                   \
-        case U:                                                                                           \
-            if (P.probes != nullptr) fused_psfnet_render_kernel<false, true, U><<<grid, TC_NT, smem, st>>>(P);   \
-            else fused_psfnet_render_kernel<false, false, U><<<grid, TC_NT, smem, st>>>(P);               \
-            break;
-        switch (uni) {
-            AADFF_LAUNCH(1) AADFF_LAUNCH(3) AADFF_LAUNCH(13) AADFF_LAUNCH(12) AADFF_LAUNCH(14) AADFF_LAUNCH(15)
-            default:
-                if (P.probes != nullptr) fused_psfnet_render_kernel<false, true, 0><<<grid, TC_NT, smem, st>>>(P);
-                else fused_psfnet_render_kernel<false, false, 0><<<grid, TC_NT, smem, st>>>(P);
-        }
-#undef AADFF_LAUNCH
-    }
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    FusedKernel kernel = nullptr;
+    for (const FusedVariant& v : FUSED_VARIANTS)
+        if (v.trace == trace && v.pred == (probes != nullptr) && v.uni == (trace ? 0 : uni) && v.ta == ta) kernel = v.fn;
+    if (!kernel) return fail(AADFF_E_UNSUPPORTED, "fused kernel specialisation not built");
+    const int grid = (int)std::min<long long>(P.n_tiles, h->num_sms);
+    kernel<<<grid, TC_NT, smem, st>>>(P);
+    return counted_launch();
 }
 
 static int render_stack_impl(aadff_psfnet_t h, const float* img, const float* depth, const float* foc, int foc_stride,
                              float* out, const int64_t out_strides[5], int N, int C, int S, int H, int W, float d_min,
-                             float d_max, int mode, void* stream, long long tile_row0 = 0, long long tile_row1 = -1);
-
-int aadff_tile_row_height(void) { return TC_TILE_H; }
-int aadff_econ_first_group(void) { return TC_ECON_FIRST_GROUP; }
-
-int aadff_render_stack_rows_f32(aadff_psfnet_t h, const float* img, const float* depth, const float* foc, float* out,
-                                const int64_t out_strides[5], int N, int C, int S, int H, int W, float d_min,
-                                float d_max, int mode, int64_t tile_row_begin, int64_t tile_row_end, void* stream) {
-    const long long total = (long long)N * S * ((H + TC_TILE_H - 1) / TC_TILE_H);
-    if (tile_row_begin < 0 || tile_row_end < tile_row_begin || tile_row_end > total)
-        return fail(AADFF_E_INVALID, "tile-row range outside [0, N*S*ceil(H/8)]");
-    return render_stack_impl(h, img, depth, foc, S, out, out_strides, N, C, S, H, W, d_min, d_max, mode, stream,
-                             tile_row_begin, tile_row_end);
-}
-
-int aadff_render_stack_f32(aadff_psfnet_t h, const float* img, const float* depth, const float* foc, float* out,
-                           const int64_t out_strides[5], int N, int C, int S, int H, int W, float d_min,
-                           float d_max, int mode, void* stream) {
-    return render_stack_impl(h, img, depth, foc, S, out, out_strides, N, C, S, H, W, d_min, d_max, mode, stream);
-}
-
-static int render_stack_impl(aadff_psfnet_t h, const float* img, const float* depth, const float* foc, int foc_stride,
-                             float* out, const int64_t out_strides[5], int N, int C, int S, int H, int W, float d_min,
-                             float d_max, int mode, void* stream, long long tile_row0, long long tile_row1) {
+                             float d_max, int mode, void* stream, long long tile_row0 = 0,
+                             long long tile_row1 = -1) {
     if (!h || !img || !depth || !foc || !out || !out_strides) return fail(AADFF_E_INVALID, "null argument");
     if (N < 0 || C < 1 || S < 1 || H < 1 || W < 1) return fail(AADFF_E_INVALID, "bad shape");
-    if (mode < 0 || mode > 5) return fail(AADFF_E_INVALID, "unknown mode");
+    if (mode < 0 || mode > AADFF_MODE_ECON8) return fail(AADFF_E_INVALID, "unknown mode");
     if (d_max == d_min) return fail(AADFF_E_INVALID, "d_max == d_min");
     if (N == 0) return AADFF_OK;
     DeviceGuard guard(h->device);
@@ -883,8 +714,7 @@ static int render_stack_impl(aadff_psfnet_t h, const float* img, const float* de
             if (M > M0) {
                 const int grid = (int)std::min<long long>((M - M0 + F32_TP - 1) / F32_TP, (long long)h->num_sms * 8);
                 mlp_fp32_kernel<true><<<grid, F32_NT, F32_SMEM, st>>>(h->f32, ra, nullptr, nullptr, M0, M);
-                g_launches.fetch_add(1);
-                CUDA_TRY(cudaGetLastError());
+                if (int rc = counted_launch()) return rc;
             }
         } else {
             int rc = launch_tc(h, ra, mode, st, tile_row0, tile_row1);
@@ -892,6 +722,25 @@ static int render_stack_impl(aadff_psfnet_t h, const float* img, const float* de
         }
     }
     return AADFF_OK;
+}
+
+int aadff_tile_row_height(void) { return TC_TILE_H; }
+int aadff_econ_first_group(void) { return TC_ECON_FIRST_GROUP; }
+
+int aadff_render_stack_rows_f32(aadff_psfnet_t h, const float* img, const float* depth, const float* foc, float* out,
+                                const int64_t out_strides[5], int N, int C, int S, int H, int W, float d_min,
+                                float d_max, int mode, int64_t tile_row_begin, int64_t tile_row_end, void* stream) {
+    const long long total = (long long)N * S * ((H + TC_TILE_H - 1) / TC_TILE_H);
+    if (tile_row_begin < 0 || tile_row_end < tile_row_begin || tile_row_end > total)
+        return fail(AADFF_E_INVALID, "tile-row range outside [0, N*S*ceil(H/8)]");
+    return render_stack_impl(h, img, depth, foc, S, out, out_strides, N, C, S, H, W, d_min, d_max, mode, stream,
+                             tile_row_begin, tile_row_end);
+}
+
+int aadff_render_stack_f32(aadff_psfnet_t h, const float* img, const float* depth, const float* foc, float* out,
+                           const int64_t out_strides[5], int N, int C, int S, int H, int W, float d_min,
+                           float d_max, int mode, void* stream) {
+    return render_stack_impl(h, img, depth, foc, S, out, out_strides, N, C, S, H, W, d_min, d_max, mode, stream);
 }
 
 int aadff_render_stack_host_f32(aadff_psfnet_t h, const float* img, const float* depth, const float* foc,
@@ -958,16 +807,14 @@ int aadff_psfnet_pred_f32(aadff_psfnet_t h, const float* inp, float* psf, int64_
     ra.ks = h->ks;
     const int grid = (int)std::min<long long>((M + F32_TP - 1) / F32_TP, (long long)h->num_sms * 8);
     mlp_fp32_kernel<false><<<grid, F32_NT, F32_SMEM, static_cast<cudaStream_t>(stream)>>>(h->f32, ra, inp, psf, 0, M);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return counted_launch();
 }
 
 int aadff_psfnet_pred_tc_f32(aadff_psfnet_t h, const float* inp, float* psf, int64_t M, int mode, void* stream) {
     if (!h || !inp || !psf) return fail(AADFF_E_INVALID, "null argument");
     if (M < 0) return fail(AADFF_E_INVALID, "negative M");
     if (mode == AADFF_MODE_FP32) return aadff_psfnet_pred_f32(h, inp, psf, M, stream);
-    if (mode < 0 || mode > 5) return fail(AADFF_E_INVALID, "unknown mode");
+    if (mode < 0 || mode > AADFF_MODE_ECON8) return fail(AADFF_E_INVALID, "unknown mode");
     if (reinterpret_cast<uintptr_t>(inp) % 16) return fail(AADFF_E_INVALID, "inp must be 16-byte aligned");
     if (M == 0) return AADFF_OK;
     DeviceGuard guard(h->device);
@@ -983,21 +830,32 @@ int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, i
     if (N < 0 || C < 1 || H < 1 || W < 1) return fail(AADFF_E_INVALID, "bad shape");
     if (ks < 1 || (ks % 2) == 0) return fail(AADFF_E_INVALID, "kernel size must be odd and positive");
     if (N == 0) return AADFF_OK;
-    int dev = 0, sms = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    if (int rc = device_sms(sms)) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int dbg = g_dbg_flags.load();
-    if (ks >= 3 && ks <= STRIP_MAX_KS && !(dbg & 512) && W % 4 == 0 && reinterpret_cast<uintptr_t>(psf) % 16 == 0 &&
+    if (ks >= 3 && ks <= STRIP_MAX_KS && !(dbg & DBG_NO_STRIP_GATHER) && W % 4 == 0 && reinterpret_cast<uintptr_t>(psf) % 16 == 0 &&
         reinterpret_cast<uintptr_t>(out) % 8 == 0 && (long long)N * H * ((W + 31) / 32) < (1ll << 40)) {
         // strip-walking kernel (gather_strip_kernel.cuh): bulk-copied PSF rows, per-warp pipelines
-        int c0 = 0;
-        while (c0 < C) {
+        for (int c0 = 0; c0 < C;) {
             const int cn = (C - c0 >= 3) ? 3 : 1;
-            if (!launch_gs_ks<3>(ks, cn, (dbg & 1024) ? 1 : (dbg & 4096) ? 2 : (dbg & 8192) ? 0 : -1, sms, st, img, psf, out, N, C, H, W, c0))
-                return fail(AADFF_E_INVALID, "unsupported kernel size");
-            g_launches.fetch_add(1);
-            CUDA_TRY(cudaGetLastError());
+            const int rc = with_odd_ks<3, STRIP_MAX_KS>(ks, [&](auto ks_c) {
+                constexpr int KS = decltype(ks_c)::value;
+                auto run = [&](auto plan_c, auto cn_c) {
+                    constexpr StripShape S = StripPlan<KS>::P[decltype(plan_c)::value];
+                    constexpr int CN = decltype(cn_c)::value;
+                    constexpr int smem = StripCfg<KS, CN, S.SPX>::SMEM_BYTES(S.SL, S.NW);
+                    static_assert(smem <= 232448, "strip gather: shared memory plan does not fit");
+                    const long long rows = (long long)N * ((W + S.SPX - 1) / S.SPX) * H;
+                    return launch(local_psf_strip_kernel<KS, CN, S.SL, S.NW, S.SPX>,
+                                  (int)std::min<long long>((rows + S.NW - 1) / S.NW, sms), S.NW * 32, smem, st, img, psf,
+                                  out, N, C, H, W, c0);
+                };
+                auto run_plan = [&](auto plan_c) { return cn == 3 ? run(plan_c, ic<3>) : run(plan_c, ic<1>); };
+                const int plan = strip_plan(StripPlan<KS>::P, W, dbg);
+                return plan == 1 ? run_plan(ic<1>) : plan == 2 ? run_plan(ic<2>) : run_plan(ic<0>);
+            });
+            if (rc) return rc;
             c0 += cn;
         }
         return AADFF_OK;
@@ -1007,29 +865,31 @@ int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, i
         const long long tiles = (long long)N * ((H + GC_WARPS - 1) / GC_WARPS) * ((W + GC_TW - 1) / GC_TW);
         if (tiles >= (1ll << 31)) return fail(AADFF_E_INVALID, "image batch too large for one launch");
         const int grid = (int)std::min<long long>(tiles, sms);
-        int c0 = 0;
-        while (c0 < C) {
+        for (int c0 = 0; c0 < C;) {
             const int cn = (C - c0 >= 3) ? 3 : 1;
-            if (!launch_gather_coalesced(ks, cn, grid, st, img, psf, out, N, C, H, W, c0))
-                return fail(AADFF_E_INVALID, "unsupported kernel size");
-            g_launches.fetch_add(1);
-            CUDA_TRY(cudaGetLastError());
+            const int rc = with_odd_ks<3, 31>(ks, [&](auto ks_c) {
+                constexpr int KS = decltype(ks_c)::value;
+                auto run = [&](auto cn_c) {
+                    constexpr int CN = decltype(cn_c)::value;
+                    constexpr int smem = GatherCfg<KS>::SMEM_FLOATS(CN) * (int)sizeof(float);   // <= 69.6 KB (ks = 31, 3 channels)
+                    return launch(local_psf_coalesced_kernel<KS, CN>, grid, GC_WARPS * 32, smem, st, img, psf, out, N, C, H,
+                                  W, c0);
+                };
+                return cn == 3 ? run(ic<3>) : run(ic<1>);
+            });
+            if (rc) return rc;
             c0 += cn;
         }
         return AADFF_OK;
     }
     // any other kernel size (1, or above 31): the generic kernel (gather_kernel.cuh)
     const int smem = GATHER_WARPS * 32 * (GATHER_TT + 1) * (int)sizeof(float);
-    if (smem > 48 * 1024)
-        CUDA_TRY(cudaFuncSetAttribute(local_psf_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const long long items = (long long)N * H * ((W + 31) / 32);
     const int grid = (int)std::min<long long>((items + GATHER_WARPS - 1) / GATHER_WARPS, (long long)sms * 3);
-    for (int c0 = 0; c0 < C; c0 += GATHER_MAXC) {
-        local_psf_render_kernel<<<grid, GATHER_WARPS * 32, smem, st>>>(img, psf, out, N, C, H, W, ks, c0,
-                                                                       std::min(GATHER_MAXC, C - c0));
-        g_launches.fetch_add(1);
-        CUDA_TRY(cudaGetLastError());
-    }
+    for (int c0 = 0; c0 < C; c0 += GATHER_MAXC)
+        if (int rc = launch(local_psf_render_kernel, grid, GATHER_WARPS * 32, smem, st, img, psf, out, N, C, H, W, ks, c0,
+                            std::min(GATHER_MAXC, C - c0)))
+            return rc;
     return AADFF_OK;
 }
 
@@ -1039,24 +899,40 @@ int aadff_local_psf_render_backward_f32(const float* img, const float* psf, cons
     if (N < 0 || C < 1 || H < 1 || W < 1) return fail(AADFF_E_INVALID, "bad shape");
     if (ks < 1 || (ks % 2) == 0) return fail(AADFF_E_INVALID, "kernel size must be odd and positive");
     if (N == 0) return AADFF_OK;
-    int dev = 0, sms = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    if (int rc = device_sms(sms)) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (grad_psf) {
         // the forward strip kernel's conditions (aadff_local_psf_render_f32), and all channels in one halo
+        int rc;
         if (ks >= 3 && ks <= STRIP_MAX_KS && C <= GPS_MAXC && W % 4 == 0 &&
             reinterpret_cast<uintptr_t>(grad_psf) % 16 == 0 && reinterpret_cast<uintptr_t>(grad_out) % 8 == 0 &&
             (long long)N * H * ((W + 31) / 32) < (1ll << 40)) {
-            if (!launch_gps_ks<3>(ks, C, sms, st, img, grad_out, grad_psf, N, H, W))
-                return fail(AADFF_E_INVALID, "unsupported kernel size");
+            rc = with_odd_ks<3, STRIP_MAX_KS>(ks, [&](auto ks_c) {
+                constexpr int KS = decltype(ks_c)::value;
+                auto run = [&](auto cn_c) {
+                    constexpr int CN = decltype(cn_c)::value;
+                    using Cfg = GradPsfStripCfg<KS, CN>;
+                    static_assert(Cfg::SMEM_BYTES <= GPS_SMEM && Cfg::NW >= 1, "strip dP: shared memory plan does not fit");
+                    const long long rows = (long long)N * ((W + GSW_PX - 1) / GSW_PX) * H;
+                    return launch(local_psf_grad_psf_strip_kernel<KS, CN>,
+                                  (int)std::min<long long>((rows + Cfg::NW - 1) / Cfg::NW, sms), Cfg::NW * 32,
+                                  Cfg::SMEM_BYTES, st, img, grad_out, grad_psf, N, H, W);
+                };
+                switch (C) {
+                    case 1: return run(ic<1>);
+                    case 2: return run(ic<2>);
+                    case 3: return run(ic<3>);
+                    case 4: return run(ic<4>);
+                    default: return fail(AADFF_E_INVALID, "unsupported kernel size");
+                }
+            });
         } else {
             const long long total = (long long)N * H * W * ks * ks;
-            local_psf_grad_psf_kernel<<<(int)std::min<long long>((total + 255) / 256, (long long)sms * 16), 256, 0, st>>>(
-                img, grad_out, grad_psf, N, C, H, W, ks);
+            rc = launch(local_psf_grad_psf_kernel, (int)std::min<long long>((total + 255) / 256, (long long)sms * 16), 256, 0,
+                        st, img, grad_out, grad_psf, N, C, H, W, ks);
         }
-        g_launches.fetch_add(1);
-        CUDA_TRY(cudaGetLastError());
+        if (rc) return rc;
     }
     if (grad_img) {
         const bool strip = ks >= 3 && ks <= STRIP_MAX_KS && W % 4 == 0 && reinterpret_cast<uintptr_t>(psf) % 16 == 0 &&
@@ -1067,14 +943,23 @@ int aadff_local_psf_render_backward_f32(const float* img, const float* psf, cons
         for (int c0 = 0; c0 < C;) {
             const int cn = strip ? ((C - c0 >= 3) ? 3 : 1) : std::min(GPS_MAXC, C - c0);
             if (strip) {
-                if (!launch_gis_ks<3>(ks, cn, sms, st, psf, grad_out, grad_img, N, C, H, W, c0))
-                    return fail(AADFF_E_INVALID, "unsupported kernel size");
-                g_launches.fetch_add(1);
-                CUDA_TRY(cudaGetLastError());
+                const int rc = with_odd_ks<3, STRIP_MAX_KS>(ks, [&](auto ks_c) {
+                    constexpr int KS = decltype(ks_c)::value;
+                    auto run = [&](auto cn_c) {
+                        using Cfg = GradImgStripCfg<KS, decltype(cn_c)::value>;
+                        static_assert(Cfg::SMEM_BYTES <= GPS_SMEM && Cfg::NW >= 1, "strip dimg: shared memory plan does not fit");
+                        const long long rows = (long long)N * ((W + GSW_PX - 1) / GSW_PX) * H;
+                        return launch(local_psf_grad_img_strip_kernel<KS, decltype(cn_c)::value>,
+                                      (int)std::min<long long>((rows + Cfg::NW - 1) / Cfg::NW, sms), Cfg::NW * 32,
+                                      Cfg::SMEM_BYTES, st, psf, grad_out, grad_img, N, C, H, W, c0);
+                    };
+                    return cn == 3 ? run(ic<3>) : run(ic<1>);
+                });
+                if (rc) return rc;
             }
-            local_psf_grad_img_kernel<<<grid, 256, 0, st>>>(psf, grad_out, grad_img, N, C, H, W, ks, c0, cn, strip ? 1 : 0);
-            g_launches.fetch_add(1);
-            CUDA_TRY(cudaGetLastError());
+            if (int rc = launch(local_psf_grad_img_kernel, grid, 256, 0, st, psf, grad_out, grad_img, N, C, H, W, ks, c0, cn,
+                                strip ? 1 : 0))
+                return rc;
             c0 += cn;
         }
     }
@@ -1086,11 +971,7 @@ int aadff_any_negative_f32(const float* x, int64_t n, unsigned char* flag_dev, v
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     CUDA_TRY(cudaMemsetAsync(flag_dev, 0, 1, st));
     if (n == 0) return AADFF_OK;
-    const int grid = (int)std::min<long long>((n + 255) / 256, 592);
-    any_negative_kernel<<<grid, 256, 0, st>>>(x, (long long)n, flag_dev);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return launch(any_negative_kernel, (int)std::min<long long>((n + 255) / 256, 592), 256, 0, st, x, (long long)n, flag_dev);
 }
 
 int aadff_thinlens_render_f32(const float* img, const float* depth, const float* foc, float* out, int N, int C, int H,
@@ -1101,10 +982,8 @@ int aadff_thinlens_render_f32(const float* img, const float* depth, const float*
     if (ks < 1 || (ks % 2) == 0) return fail(AADFF_E_INVALID, "kernel size must be odd and positive");
     if (!(fnum > 0.f) || !(pixel_size > 0.f) || !(d_hi > d_lo)) return fail(AADFF_E_INVALID, "bad lens parameters");
     if (N == 0) return AADFF_OK;
-    int dev = 0, sms = 0, optin = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    int sms = 0, optin = 0;
+    if (int rc = device_sms(sms, &optin)) return rc;
     ThinLensArgs a{};
     a.img = img; a.depth = depth; a.foc = foc; a.out = out;
     a.N = N; a.C = C; a.H = H; a.W = W;
@@ -1119,16 +998,18 @@ int aadff_thinlens_render_f32(const float* img, const float* depth, const float*
     for (int c0 = 0; c0 < C; c0 += TL_MAXC) {
         a.c0 = c0;
         a.cn = std::min(TL_MAXC, C - c0);
-        int HH = 0, BW = 0, smem = 0;
-        if (!thinlens2_geometry<1>(ks, a.cn, &BW, &HH, &smem)) return fail(AADFF_E_INVALID, "unsupported kernel size");
-        if (smem > optin) return fail(AADFF_E_UNSUPPORTED, "kernel size too large for the shared-memory halo tile");
-        // the image halo of interior tiles arrives as one TMA box [cn][HH][BW] of the [N*C, H, W] tensor
-        CUtensorMap map;
-        std::memset(&map, 0, sizeof(map));
-        a.use_tma = make_image_map(&map, img, (long long)N * C, H, W, BW, HH, a.cn) && !(g_dbg_flags.load() & 16);
-        if (!launch_thinlens2<1>(ks, grid, smem, st, a, map)) return fail(AADFF_E_INVALID, "unsupported kernel size");
-        g_launches.fetch_add(1);
-        CUDA_TRY(cudaGetLastError());
+        const int rc = with_odd_ks<1, 31>(ks, [&](auto ks_c) {
+            using Cfg = ThinLens2Cfg<decltype(ks_c)::value>;
+            const int smem = Cfg::SMEM_BYTES(a.cn);
+            if (smem > optin) return fail(AADFF_E_UNSUPPORTED, "kernel size too large for the shared-memory halo tile");
+            // the image halo of interior tiles arrives as one TMA box [cn][HH][BW] of the [N*C, H, W] tensor
+            CUtensorMap map;
+            std::memset(&map, 0, sizeof(map));
+            a.use_tma = make_image_map(&map, img, (long long)N * C, H, W, Cfg::BW, Cfg::HH, a.cn) &&
+                        !(g_dbg_flags.load() & DBG_THINLENS_NO_TMA);
+            return launch(thinlens_render2_kernel<decltype(ks_c)::value>, grid, TL_NT, smem, st, a, map);
+        });
+        if (rc) return rc;
     }
     return AADFF_OK;
 }
@@ -1164,16 +1045,14 @@ int aadff_render_psf_map_f32(const float* img, const float* psf_map, float* out,
     if (B == 0) return AADFF_OK;
     a.img = img; a.psf_map = psf_map; a.out = out;
     if (a.max_ch == 0 || a.max_cw == 0) return AADFF_OK;
-    int dev = 0, sms = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    if (int rc = device_sms(sms)) return rc;
     const long long tiles = (long long)B * C * grid * grid * ((a.max_ch + PC_TILE_H - 1) / PC_TILE_H) *
                             ((a.max_cw + PC_TILE_W - 1) / PC_TILE_W);
     const int nblk = (int)std::min<long long>(tiles, (long long)sms * 8);
-    if (!launch_psf_conv<1>(ks, nblk, static_cast<cudaStream_t>(stream), a)) return fail(AADFF_E_INVALID, "unsupported kernel size");
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return with_odd_ks<1, 31>(ks, [&](auto ks_c) {
+        return launch(psf_conv_kernel<decltype(ks_c)::value>, nblk, PC_NT, 0, static_cast<cudaStream_t>(stream), a);
+    });
 }
 
 // Stage-1 partials of the PSF-map gradient: one ks^2 vector per (channel, cell, image, tile of the largest cell).
@@ -1207,28 +1086,25 @@ int aadff_render_psf_map_backward_f32(const float* img, const float* psf_map, co
         if (grad_psf_map) CUDA_TRY(cudaMemsetAsync(grad_psf_map, 0, psf_bytes, st));
         return AADFF_OK;
     }
-    int dev = 0, sms = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    if (int rc = device_sms(sms)) return rc;
     if (grad_img) {
         const long long tiles = (long long)B * C * ((H + PCG_TH - 1) / PCG_TH) * ((W + PCG_TW - 1) / PCG_TW);
-        psf_conv_grad_img_kernel<<<(int)std::min<long long>(tiles, (long long)sms * 8), PC_NT, 0, st>>>(a, grad_out,
-                                                                                                      grad_img, ks);
-        g_launches.fetch_add(1);
-        CUDA_TRY(cudaGetLastError());
+        if (int rc = launch(psf_conv_grad_img_kernel, (int)std::min<long long>(tiles, (long long)sms * 8), PC_NT, 0, st, a,
+                            grad_out, grad_img, ks))
+            return rc;
     }
     if (grad_psf_map) {
         const long long parts = psf_map_grad_parts(a), tiles = (long long)C * grid * grid * parts;
         float* ws = static_cast<float*>(work);
-        if (!launch_psf_conv_grad_psf<1>(ks, (int)std::min<long long>(tiles, (long long)sms * 8), st, a, grad_out, ws))
-            return fail(AADFF_E_INVALID, "unsupported kernel size");
-        g_launches.fetch_add(1);
-        CUDA_TRY(cudaGetLastError());
+        if (int rc = with_odd_ks<1, 31>(ks, [&](auto ks_c) {
+                return launch(psf_conv_grad_psf_kernel<decltype(ks_c)::value>,
+                              (int)std::min<long long>(tiles, (long long)sms * 8), PC_NT, 0, st, a, grad_out, ws);
+            }))
+            return rc;
         const long long warps = (long long)C * grid * grid * ks * ks;
-        psf_conv_grad_reduce_kernel<<<(int)std::min<long long>((warps + 7) / 8, (long long)sms * 16), 256, 0, st>>>(
-            ws, grad_psf_map, C, grid, ks, parts);
-        g_launches.fetch_add(1);
-        CUDA_TRY(cudaGetLastError());
+        return launch(psf_conv_grad_reduce_kernel, (int)std::min<long long>((warps + 7) / 8, (long long)sms * 16), 256, 0,
+                      st, ws, grad_psf_map, C, grid, ks, parts);
     }
     return AADFF_OK;
 }
@@ -1248,11 +1124,8 @@ int aadff_preprocess_rgbd_u8(const uint8_t* bgr, const uint16_t* depth, float* a
     const long long per_image = (long long)h * w;
     const dim3 grid((unsigned)std::min<long long>((per_image + 255) / 256, 148 * 16), (unsigned)B);
     if (B > 65535) return fail(AADFF_E_INVALID, "batch too large for one launch");
-    if (depth_mode == 1) preprocess_rgbd_kernel<false, true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    else preprocess_rgbd_kernel<false, false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return launch(depth_mode == 1 ? preprocess_rgbd_kernel<false, true> : preprocess_rgbd_kernel<false, false>, grid, 256, 0,
+                  static_cast<cudaStream_t>(stream), a);
 }
 
 int aadff_prepare_planes_u8(const uint8_t* bgr, const uint16_t* depth, float* planes, int B, int H, int W, float depth_div,
@@ -1266,10 +1139,7 @@ int aadff_prepare_planes_u8(const uint8_t* bgr, const uint16_t* depth, float* pl
     a.bgr = bgr; a.depth = depth; a.planes = planes; a.jitter = jitter; a.flips = flips;
     a.B = B; a.H = H; a.W = W; a.P = (bgr ? 3 : 0) + (depth ? 1 : 0); a.depth_div = depth_div;
     const dim3 grid((unsigned)std::min<long long>(((long long)H * W + 255) / 256, 148 * 8), (unsigned)B);
-    prepare_planes_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return launch(prepare_planes_kernel, grid, 256, 0, static_cast<cudaStream_t>(stream), a);
 }
 
 int aadff_spline_affine_f32(const float* planes, float* work, float* out, int B, int P, int H, int W, const double* xform,
@@ -1284,15 +1154,12 @@ int aadff_spline_affine_f32(const float* planes, float* work, float* out, int B,
     float* tmp = work;                 // prefiltered along W
     float* coef = work + n;            // ... and along H
     const unsigned blocks = (unsigned)std::min<long long>((n + 255) / 256, 148 * 16);
-    spline_prefilter_kernel<1><<<blocks, 256, 0, st>>>(planes, tmp, (long long)B * P, H, W);
-    spline_prefilter_kernel<0><<<blocks, 256, 0, st>>>(tmp, coef, (long long)B * P, H, W);
+    if (int rc = launch(spline_prefilter_kernel<1>, blocks, 256, 0, st, planes, tmp, (long long)B * P, H, W)) return rc;
+    if (int rc = launch(spline_prefilter_kernel<0>, blocks, 256, 0, st, tmp, coef, (long long)B * P, H, W)) return rc;
     AffineArgs a{};
     a.coef = coef; a.raw = planes; a.out = out; a.xform = xform; a.B = B; a.P = P; a.H = H; a.W = W; a.clamp_plane = clamp_plane;
     const dim3 grid((unsigned)std::min<long long>(((long long)H * W + 255) / 256, 148 * 8), (unsigned)B);
-    spline_affine_kernel<<<grid, 256, 0, st>>>(a);
-    g_launches.fetch_add(3);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return launch(spline_affine_kernel, grid, 256, 0, st, a);
 }
 
 int aadff_resize_planes_f32(const float* planes, float* aif_out, float* depth_out, int B, int P, int H, int W, int h, int w,
@@ -1308,11 +1175,8 @@ int aadff_resize_planes_f32(const float* planes, float* aif_out, float* depth_ou
     a.B = B; a.H = H; a.W = W; a.h = h; a.w = w; a.depth_div = 1.f;
     const long long per_image = (long long)h * w;
     const dim3 grid((unsigned)std::min<long long>((per_image + 255) / 256, 148 * 16), (unsigned)B);
-    if (depth_mode == 1) preprocess_rgbd_kernel<true, true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    else preprocess_rgbd_kernel<true, false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return launch(depth_mode == 1 ? preprocess_rgbd_kernel<true, true> : preprocess_rgbd_kernel<true, false>, grid, 256, 0,
+                  static_cast<cudaStream_t>(stream), a);
 }
 
 int aadff_select_focus_f32(const float* depth_m, int B, int64_t HW, int num, float* out, void* stream) {
@@ -1320,10 +1184,7 @@ int aadff_select_focus_f32(const float* depth_m, int B, int64_t HW, int num, flo
     if (B < 0 || HW < 1) return fail(AADFF_E_INVALID, "bad shape");
     if (num <= 3) return fail(AADFF_E_INVALID, "Focal stack size is too small");   // the reference asserts num > 3
     if (B == 0) return AADFF_OK;
-    select_focus_kernel<<<B, FOCUS_NT, 0, static_cast<cudaStream_t>(stream)>>>(depth_m, (long long)HW, num, out);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return AADFF_OK;
+    return launch(select_focus_kernel, B, FOCUS_NT, 0, static_cast<cudaStream_t>(stream), depth_m, (long long)HW, num, out);
 }
 
 
@@ -1339,11 +1200,9 @@ int aadff_trainer_create(const float* const* weights, const float* const* biases
     t->dims.assign(dims, dims + n_layers + 1);
     t->host_hyper.beta1 = beta1; t->host_hyper.beta2 = beta2; t->host_hyper.eps = eps; t->host_hyper.weight_decay = weight_decay;
     size_t off = 0;
-    int wmax = 0;
     for (int l = 0; l < n_layers; ++l) {
         t->w_off.push_back(off); off += (size_t)dims[l] * dims[l + 1];
         t->b_off.push_back(off); off += (size_t)dims[l + 1];
-        wmax = std::max(wmax, std::max(dims[l], dims[l + 1]));
     }
     t->n_params = off;
 #define TR_TRY(expr)                                                                             \
@@ -1372,7 +1231,6 @@ int aadff_trainer_create(const float* const* weights, const float* const* biases
         TR_TRY(dalloc(&d, (size_t)batch * dims[l + 1]));
         t->dz.push_back(d);
     }
-    (void)wmax;
     TR_TRY(dalloc(&t->loss, 1));
     TR_TRY(cudaMalloc(reinterpret_cast<void**>(&t->hyper), sizeof(AdamHyper)));
     TR_TRY(cudaStreamCreateWithFlags(&t->cap_stream, cudaStreamNonBlocking));
@@ -1456,12 +1314,9 @@ int aadff_debug_umma_gemm(const float* A, const float* B, float* D, int K, int N
     CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&dB), pack_hi.size() * 2));
     CUDA_TRY(cudaMemcpy(dA, A, (size_t)128 * K * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(cudaMemcpy(dB, pack_hi.data(), pack_hi.size() * 2, cudaMemcpyHostToDevice));
-    const int smem = TC_A_PART_BYTES + 131072 + 64;
-    CUDA_TRY(cudaFuncSetAttribute(debug_umma_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    debug_umma_gemm_kernel<<<1, 128, smem>>>(dA, reinterpret_cast<const uint8_t*>(dB), dD, K, N,
-                                             (uint32_t)g_desc_swap.load());
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
+    if (int rc = launch(debug_umma_gemm_kernel, 1, 128, TC_A_PART_BYTES + 131072 + 64, nullptr, dA,
+                        reinterpret_cast<const uint8_t*>(dB), dD, K, N, (uint32_t)g_desc_swap.load()))
+        return rc;
     CUDA_TRY(cudaDeviceSynchronize());
     CUDA_TRY(cudaMemcpy(D, dD, (size_t)128 * N * 4, cudaMemcpyDeviceToHost));
     cudaFree(dA); cudaFree(dB); cudaFree(dD);

@@ -386,7 +386,6 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
         for (long long iter = 0; iter < my_iters; ++iter) {
             for (int gi = 0; gi < P.n_groups; ++gi) {
                 const uint32_t gN = P.g[gi].N;
-                const int nkc = P.g[gi].K / TC_SLAB_K;
                 const bool three = terms_of(gi) == 3;        // Ah*Wh + Al*Wh + Ah*Wl
                 const bool use_al = terms_of(gi) >= 2;       // 2 terms: Ah*Wh + Al*Wh (weights rounded to fp16)
                 const bool new_a = P.g[gi].new_a != 0;
