@@ -60,8 +60,9 @@ SHAPES = [(1, 3, 1, 8, 16), (1, 3, 3, 37, 50), (2, 1, 2, 24, 40), (1, 4, 3, 29, 
 @pytest.mark.parametrize("ks,hidden_layers", [(11, 8), (13, 8), (15, 8), (11, 2), (11, 5), (11, 0)])
 @pytest.mark.parametrize("mode", ["parity", "econ8", "econ"])
 def test_tmem_operand_path_bit_identical(pkg, ks, hidden_layers, mode):
-    """ks <= 13 with at least two hidden groups takes the tensor-memory path; ks = 15 (two head blocks) and the
-    single-hidden-group net fall back to the shared-memory path, so the comparison is trivially equal there."""
+    """ks <= 13 with at least two hidden groups takes the tensor-memory path; ks = 15 (one head block of N = 240, more
+    than the 192 columns the path leaves for the head) and the single-hidden-group net fall back to the shared-memory
+    path, so the comparison is trivially equal there.  tests/test_gpu_fused_vs_f64.py compares both paths with float64."""
     lens = make_lens(pkg, ks, hidden_layers)
     for i, (N, C, S, H, W) in enumerate(SHAPES):
         img, dep, foc = inputs(N, C, S, H, W, seed=20 + i)
