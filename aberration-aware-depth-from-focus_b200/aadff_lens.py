@@ -264,6 +264,9 @@ class PSFNet(nn.Module):
                     inp, psf = data(bs=bs, spp=spp)
                     inp = inp.detach().to(dev, torch.float32).reshape(bs, 4).contiguous()
                     psf = psf.detach().to(dev, torch.float32).reshape(bs, -1).contiguous()
+                    if psf.shape[-1] != self.kernel_size ** 2:      # the step reads bs * ks^2 target values
+                        raise ValueError(f"train_psfnet: data returned PSFs of {psf.shape[-1]} taps per probe; "
+                                         f"kernel_size {self.kernel_size} needs {self.kernel_size ** 2}")
                     lr_i = 0.5 * lr * (1.0 + math.cos(math.pi * i / iters)) if iters > 0 else lr   # CosineAnnealingLR, eta_min 0
                     _nat.check(_nat.lib.aadff_trainer_step(trainer.handle, inp.data_ptr(), psf.data_ptr(), lr_i,
                                                            loss_dev.data_ptr(), torch.cuda.current_stream().cuda_stream))

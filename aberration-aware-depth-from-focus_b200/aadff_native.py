@@ -192,7 +192,14 @@ class NativeTrainer:
         self._np = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
         self._nb = [np.ascontiguousarray(b, dtype=np.float32) for b in biases]
         n = len(self._np)
-        self.dims = [self._np[0].shape[1]] + [w.shape[0] for w in self._np]
+        if n < 1 or len(self._nb) != n:
+            raise ValueError(f"NativeTrainer: need as many biases as weights (>= 1), got {n} and {len(self._nb)}")
+        self.dims = [self._np[0].shape[-1]] + [w.shape[0] for w in self._np]
+        for l, (w, b) in enumerate(zip(self._np, self._nb)):
+            # the library copies dims[l+1] * dims[l] weights and dims[l+1] biases of each layer from these buffers
+            if w.shape != (self.dims[l + 1], self.dims[l]) or b.shape != (self.dims[l + 1],):
+                raise ValueError(f"NativeTrainer: layer {l} has weight {tuple(w.shape)} and bias {tuple(b.shape)}; "
+                                 f"expected ({self.dims[l + 1]}, {self.dims[l]}) and ({self.dims[l + 1]},)")
         self.batch, self.device_index = int(batch), device_index
         c_f32p = ctypes.POINTER(ctypes.c_float)
         wp = (c_f32p * n)(*[w.ctypes.data_as(c_f32p) for w in self._np])

@@ -1193,6 +1193,21 @@ int aadff_trainer_create(const float* const* weights, const float* const* biases
                          aadff_trainer_t* out) {
     if (!weights || !biases || !dims || !out) return fail(AADFF_E_INVALID, "null argument");
     if (n_layers < 1 || n_layers > MAX_LAYERS || batch < 1) return fail(AADFF_E_INVALID, "bad n_layers / batch");
+    // aadff_psfnet_create's dims rules, except that any kk >= 1 goes (the trainer takes no kernel size): every step
+    // copies batch * dims[0] floats from an input documented as [batch, 4]
+    if (dims[0] != 4) return fail(AADFF_E_INVALID, "dims must start with 4");
+    for (int l = 0; l < n_layers; ++l) {
+        if (!weights[l] || !biases[l]) return fail(AADFF_E_INVALID, "null layer pointer");
+        if (l + 1 < n_layers && (dims[l + 1] < 8 || dims[l + 1] > 256 || dims[l + 1] % 8))
+            return fail(AADFF_E_INVALID, "hidden widths must be multiples of 8 and <= 256");
+    }
+    if (dims[n_layers] < 1) return fail(AADFF_E_INVALID, "dims must end with kk >= 1");
+    // the ranges torch.optim.AdamW accepts
+    if (!(beta1 >= 0.f && beta1 < 1.f)) return fail(AADFF_E_INVALID, "beta1 must be in [0, 1)");
+    if (!(beta2 >= 0.f && beta2 < 1.f)) return fail(AADFF_E_INVALID, "beta2 must be in [0, 1)");
+    if (!(eps >= 0.f && std::isfinite(eps))) return fail(AADFF_E_INVALID, "eps must be finite and >= 0");
+    if (!(weight_decay >= 0.f && std::isfinite(weight_decay)))
+        return fail(AADFF_E_INVALID, "weight_decay must be finite and >= 0");
     DeviceGuard guard(device);
     if (!guard.ok) return fail(AADFF_E_CUDA, "cannot select CUDA device " + std::to_string(device));
     aadff_trainer* t = new aadff_trainer();
@@ -1217,7 +1232,6 @@ int aadff_trainer_create(const float* const* weights, const float* const* biases
     TR_TRY(dalloc(&t->params, off)); TR_TRY(dalloc(&t->grads, off)); TR_TRY(dalloc(&t->m, off)); TR_TRY(dalloc(&t->v, off));
     TR_TRY(cudaMemset(t->m, 0, off * sizeof(float))); TR_TRY(cudaMemset(t->v, 0, off * sizeof(float)));
     for (int l = 0; l < n_layers; ++l) {
-        if (!weights[l] || !biases[l]) { trainer_free(t); return fail(AADFF_E_INVALID, "null layer pointer"); }
         TR_TRY(cudaMemcpy(t->params + t->w_off[l], weights[l], (size_t)dims[l] * dims[l + 1] * sizeof(float), cudaMemcpyHostToDevice));
         TR_TRY(cudaMemcpy(t->params + t->b_off[l], biases[l], (size_t)dims[l + 1] * sizeof(float), cudaMemcpyHostToDevice));
         float* a = nullptr;
@@ -1256,6 +1270,8 @@ int aadff_trainer_destroy(aadff_trainer_t t) {
 }
 
 int aadff_trainer_step(aadff_trainer_t t, const float* inp, const float* target, float lr, float* loss_out, void* stream) {
+    // the scalar first: its check needs no handle, so it is testable without a device or a trainer
+    if (!(lr >= 0.f && std::isfinite(lr))) return fail(AADFF_E_INVALID, "lr must be finite and >= 0");
     if (!t || !inp || !target) return fail(AADFF_E_INVALID, "null argument");
     DeviceGuard guard(t->device);
     if (!guard.ok) return fail(AADFF_E_CUDA, "cannot select device");

@@ -175,10 +175,12 @@ int aadff_select_focus_f32(const float* depth_m, int B, int64_t HW, int num, flo
 /* Replaces the optimisation half of PSFNet.train_psfnet (deeplens/psfnet.py:79-132): `psfnet(inp)` ->
  * nn.MSELoss()(pred, psf) -> loss.backward() -> torch.optim.AdamW.step(), fp32, for MLP(4, ks*ks, 256, n) -- the
  * training targets (ray-traced PSFs, psfnet.py:135-170) stay with the caller.  The trainer owns a device copy of the
- * parameters (weights/biases/dims as for aadff_psfnet_create, HOST pointers), their AdamW state and the activations of
+ * parameters (weights/biases as for aadff_psfnet_create, HOST pointers), their AdamW state and the activations of
  * one batch of `batch` probes; one step is a CUDA graph replay (3 kernels per layer and direction + head + AdamW).
- *   aadff_trainer_step: inp [batch,4], target [batch,ks*ks] device pointers; lr = this step's learning rate (the
- *     reference drives it with CosineAnnealingLR); loss_out = optional DEVICE scalar receiving the MSE loss of the
+ * dims = [4, hidden widths (multiples of 8, <= 256), kk >= 1], 1 to 16 layers; 0 <= beta1, beta2 < 1; eps and
+ * weight_decay finite and >= 0 (as torch.optim.AdamW): anything else is AADFF_E_INVALID, checked before any device work.
+ *   aadff_trainer_step: inp [batch,4], target [batch,ks*ks] device pointers; lr = this step's learning rate, finite
+ *     and >= 0 (the reference drives it with CosineAnnealingLR); loss_out = optional DEVICE scalar receiving the MSE loss of the
  *     forward pass that preceded the update.  Stream-ordered, no synchronisation.
  *   aadff_trainer_read: which = 0 parameters / 1 gradients of the last step into HOST arrays shaped like the
  *     create call's; which = 2: the last step's predicted PSFs [batch, ks*ks] into weights[0].  Synchronises.   */

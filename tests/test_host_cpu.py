@@ -47,6 +47,65 @@ def test_argument_validation_needs_no_device(pkg):
     assert lib.aadff_psfnet_destroy(None) == 0
 
 
+def test_trainer_argument_validation_needs_no_device(pkg):
+    """aadff_trainer_create / _step refuse what would make a step read outside its buffers (dims that are not
+    [4, hidden widths, kk]) and the AdamW settings torch.optim.AdamW refuses, before touching a device."""
+    lib = pkg.native.lib
+    c_f32p = ctypes.POINTER(ctypes.c_float)
+
+    def create(dims, batch=8, beta1=0.9, beta2=0.999, eps=1e-8, wd=1e-2, null_layer=None):
+        # every layer gets buffers as large as its dims ask for, so that a call the library accepts (on a box with a
+        # GPU it goes on to copy dims[l+1] * dims[l] weights and dims[l+1] biases per layer) reads only what it owns
+        n = len(dims) - 1
+        ws = [np.zeros(max(dims[l + 1], 1) * max(dims[l], 1), np.float32) for l in range(n)]
+        bs = [np.zeros(max(dims[l + 1], 1), np.float32) for l in range(n)]
+        wp = (c_f32p * n)(*[c_f32p() if l == null_layer else w.ctypes.data_as(c_f32p) for l, w in enumerate(ws)])
+        bp = (c_f32p * n)(*[b.ctypes.data_as(c_f32p) for b in bs])
+        handle = ctypes.c_void_p()
+        rc = lib.aadff_trainer_create(wp, bp, (ctypes.c_int * (n + 1))(*dims), n, batch, beta1, beta2, eps, wd, 0,
+                                      ctypes.byref(handle))
+        return rc, lib.aadff_last_error().decode(), handle
+
+    nan, inf = float("nan"), float("inf")
+    bad = [
+        (dict(dims=[5, 64, 9]), "start with 4"), (dict(dims=[3, 64, 9]), "start with 4"),
+        (dict(dims=[4, 60, 9]), "hidden widths"), (dict(dims=[4, 0, 9]), "hidden widths"),
+        (dict(dims=[4, -8, 9]), "hidden widths"), (dict(dims=[4, 264, 9]), "hidden widths"),
+        (dict(dims=[4, 64, 256, 0]), "kk"), (dict(dims=[4, -1]), "kk"),
+        (dict(dims=[4] + [64] * 16 + [9]), "n_layers"), (dict(dims=[4, 64, 9], batch=0), "batch"),
+        (dict(dims=[4, 64, 9], null_layer=1), "null layer"),
+        (dict(dims=[4, 64, 9], beta1=1.0), "beta1"), (dict(dims=[4, 64, 9], beta1=-0.1), "beta1"),
+        (dict(dims=[4, 64, 9], beta1=nan), "beta1"), (dict(dims=[4, 64, 9], beta2=1.0), "beta2"),
+        (dict(dims=[4, 64, 9], beta2=nan), "beta2"), (dict(dims=[4, 64, 9], eps=-1e-8), "eps"),
+        (dict(dims=[4, 64, 9], eps=inf), "eps"), (dict(dims=[4, 64, 9], eps=nan), "eps"),
+        (dict(dims=[4, 64, 9], wd=-1e-2), "weight_decay"), (dict(dims=[4, 64, 9], wd=inf), "weight_decay"),
+        (dict(dims=[4, 64, 9], wd=nan), "weight_decay"),
+    ]
+    for kwargs, name in bad:
+        rc, msg, _ = create(**kwargs)
+        assert rc == -1 and name in msg, (kwargs, rc, msg)
+    # the edges that are valid get past validation (on a box without a GPU, to the device selection)
+    for kwargs in (dict(dims=[4, 1]), dict(dims=[4, 8, 256, 961], beta1=0.0, beta2=0.0, eps=0.0, wd=0.0)):
+        rc, msg, handle = create(**kwargs)
+        if rc == 0:
+            lib.aadff_trainer_destroy(handle)
+        else:
+            assert rc == -2 and "CUDA device" in msg, (kwargs, rc, msg)
+    for lr in (nan, inf, -inf, -1e-4):            # checked first, so no handle is needed (every pointer is null)
+        assert lib.aadff_trainer_step(None, None, None, lr, None, None) == -1
+        assert b"lr" in lib.aadff_last_error()
+    # NativeTrainer checks layer shapes before the library copies dims[l+1] * dims[l] floats from each buffer
+    Ws = [np.zeros((64, 4), np.float32), np.zeros((256, 64), np.float32), np.zeros((9, 256), np.float32)]
+    bs = [np.zeros(64, np.float32), np.zeros(256, np.float32), np.zeros(9, np.float32)]
+    for l, W in ((1, np.zeros((256, 63), np.float32)), (2, np.zeros((9, 255), np.float32))):
+        with pytest.raises(ValueError, match=f"layer {l}"):
+            pkg.native.NativeTrainer(Ws[:l] + [W] + Ws[l + 1:], bs, 8, 0)
+    with pytest.raises(ValueError, match="layer 1"):
+        pkg.native.NativeTrainer(Ws, bs[:1] + [np.zeros(255, np.float32)] + bs[2:], 8, 0)
+    with pytest.raises(ValueError, match="biases"):
+        pkg.native.NativeTrainer(Ws, bs[:2], 8, 0)
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks behaviour on a box without a GPU")
 def test_no_cpu_fallback(pkg):
     """Without a device every compute entry fails loudly; nothing silently computes on the host."""
