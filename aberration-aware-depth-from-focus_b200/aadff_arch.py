@@ -2,7 +2,9 @@
 
 ``MLP`` only *holds* the parameters, under the same ``net.{0,2,4,...}`` state_dict keys as the
 reference so checkpoints round-trip; evaluating it goes to the CUDA library.  There is no
-PyTorch forward path here on purpose.
+PyTorch forward path here on purpose.  Under autograd (grad mode on, and the input or a parameter
+requiring grad) the evaluation is differentiable in the input and the parameters, with backward
+kernels of the same library.
 """
 import torch
 import torch.nn as nn
@@ -38,4 +40,6 @@ class MLP(nn.Module):
         if self._evaluator is None:
             raise RuntimeError("MLP has no CUDA evaluator attached; use PSFNet.pred / PSFNet.render "
                                "(this build has no PyTorch-eager forward path)")
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+            return self._evaluator(x, layers=self.linear_layers())
         return self._evaluator(x)

@@ -25,6 +25,7 @@ import os
 import numpy as np
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 import aadff_native as _nat
 from aadff_arch import MLP, initialize_weights
@@ -44,6 +45,53 @@ def _device_index(device) -> int:
 def _linear_layers(net):
     """The nn.Linear modules of an MLP container (ours or the reference's: both keep them in ``.net``)."""
     return [m for m in net.net if isinstance(m, nn.Linear)]
+
+
+class _PSFNetMLP(torch.autograd.Function):
+    """psf [M, kk] = MLP(flat [M, 4]) with the parameters (w0, b0, w1, b1, ...): fp32, contiguous, on the device of the
+    handle `nat`.  The forward is aadff_psfnet_pred_f32, the very call of the no-grad path; the backward
+    (aadff_psfnet_backward_f32) recomputes the activations and reads the weights of the same handle, which the graph
+    keeps alive.  The saved probes and parameters make autograd refuse a backward after an in-place change to them."""
+
+    @staticmethod
+    def forward(ctx, nat, flat, *params):
+        out = torch.empty(flat.shape[0], nat.ks ** 2, device=flat.device, dtype=torch.float32)
+        if flat.shape[0]:
+            with torch.cuda.device(flat.device):
+                _nat.check(_nat.lib.aadff_psfnet_pred_f32(nat.handle, flat.data_ptr(), out.data_ptr(), flat.shape[0],
+                                                          torch.cuda.current_stream().cuda_stream))
+        ctx.nat = nat
+        ctx.save_for_backward(flat, *params)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_psf):
+        flat, *params = ctx.saved_tensors
+        need_inp, need_p = ctx.needs_input_grad[1], ctx.needs_input_grad[2:]
+        grads = [torch.empty_like(p) if n else None for p, n in zip(params, need_p)]
+        grad_inp = torch.empty_like(flat) if need_inp else None
+        M = flat.shape[0]
+        if not (need_inp or any(need_p)):
+            return (None, None) + tuple(grads)
+        if M == 0:          # no probe: the parameter gradients are 0 (data_ptr() of an empty tensor is NULL)
+            return (None, grad_inp) + tuple(g.zero_() if g is not None else None for g in grads)
+        nat = ctx.nat
+        g = grad_psf.to(torch.float32).contiguous()
+        c_f32p = _nat.ctypes.POINTER(_nat.ctypes.c_float)
+        ptr = lambda t: _nat.ctypes.cast(_nat.ctypes.c_void_p(t.data_ptr()), c_f32p) if t is not None else None
+        n = nat.n_layers
+        wp = (c_f32p * n)(*[ptr(t) for t in grads[0::2]])
+        bp = (c_f32p * n)(*[ptr(t) for t in grads[1::2]])
+        with torch.cuda.device(flat.device):
+            work_bytes = _nat.lib.aadff_psfnet_backward_work_bytes(nat.handle, M)
+            if work_bytes < 0:
+                _nat.check(int(work_bytes))
+            work = torch.empty(work_bytes, dtype=torch.uint8, device=flat.device)
+            _nat.check(_nat.lib.aadff_psfnet_backward_f32(
+                nat.handle, flat.data_ptr(), g.data_ptr(), grad_inp.data_ptr() if need_inp else None, wp, bp,
+                work.data_ptr(), work_bytes, M, torch.cuda.current_stream().cuda_stream))
+        return (None, grad_inp) + tuple(grads)
 
 
 class PSFNet(nn.Module):
@@ -97,8 +145,8 @@ class PSFNet(nn.Module):
             idx = _device_index(layers[0].weight.device)
             ws = [l.weight.detach().float().cpu().numpy() for l in layers]
             bs = [l.bias.detach().float().cpu().numpy() for l in layers]
-            if getattr(self, "_native", None) is not None:
-                self._native.close()
+            # the old handle is dropped, not closed: an autograd graph whose forward ran on it still holds it for its
+            # backward, and NativePSFNet.__del__ frees it once the last reference is gone
             self._native = _nat.NativePSFNet(ws, bs, self.kernel_size, idx)
             self._native_sig = sig
         return self._native
@@ -111,9 +159,18 @@ class PSFNet(nn.Module):
         logging.info("PSFNet.analysis(): lens plots/ray tracing are outside the synthesis path; skipped.")
 
     # ------------------------------------------------------------------ inference
-    def _mlp_eval(self, inp, mode="fp32"):
+    def _mlp_eval(self, inp, mode="fp32", layers=None):
+        """psf [..., ks*ks] of the probes inp [..., 4].  With `layers` (the network's nn.Linear modules, passed by
+        MLP.forward when autograd needs it) the result is differentiable in inp and in their parameters."""
         nat = PSFNet.native(self)
         kk = self.kernel_size ** 2
+        if layers is not None:
+            dev = torch.device(f"cuda:{nat.device_index}")
+            flat = inp.reshape(-1, 4).to(dev, torch.float32).contiguous()
+            params = []
+            for l in layers:
+                params += [l.weight.to(dev, torch.float32).contiguous(), l.bias.to(dev, torch.float32).contiguous()]
+            return _PSFNetMLP.apply(nat, flat, *params).reshape(*inp.shape[:-1], kk)
         flat = inp.detach().reshape(-1, 4).to(f"cuda:{nat.device_index}", torch.float32).contiguous()
         out = torch.empty(flat.shape[0], kk, device=flat.device, dtype=torch.float32)
         if flat.shape[0] == 0:

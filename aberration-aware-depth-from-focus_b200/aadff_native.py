@@ -104,6 +104,11 @@ def _load() -> ctypes.CDLL:
                                           ctypes.c_void_p]
     lib.aadff_psfnet_pred_tc_f32.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
                                              ctypes.c_int, ctypes.c_void_p]
+    lib.aadff_psfnet_backward_work_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int64]
+    lib.aadff_psfnet_backward_work_bytes.restype = ctypes.c_int64
+    lib.aadff_psfnet_backward_f32.argtypes = [ctypes.c_void_p] * 4 + [ctypes.POINTER(c_f32p)] * 2 + \
+                                             [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p]
+    lib.aadff_psfnet_backward_f32.restype = ctypes.c_int
     lib.aadff_local_psf_render_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
     lib.aadff_local_psf_render_backward_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
     lib.aadff_render_psf_map_backward_work_bytes.argtypes = [ctypes.c_int] * 6 + [ctypes.POINTER(ctypes.c_int)] * 2
@@ -167,6 +172,7 @@ class NativePSFNet:
         dm = (ctypes.c_int * (n + 1))(*dims)
         self.handle = ctypes.c_void_p()
         self.ks = ks
+        self.n_layers = n
         self.device_index = device_index
         check(lib.aadff_psfnet_create(wp, bp, dm, n, ks, device_index, ctypes.byref(self.handle)))
         self._np = self._nb = None

@@ -25,6 +25,7 @@
 #include "psf_grad_kernel.cuh"
 #include "psf_conv_grad_kernel.cuh"
 #include "train_kernels.cuh"
+#include "mlp_grad_kernel.cuh"
 #include "preprocess_kernel.cuh"
 #include "spline_rotate_kernel.cuh"
 #include "econ_calib.h"
@@ -260,6 +261,8 @@ struct aadff_psfnet {
     int num_sms = 0, smem_optin = 0;
     // fp32 (CUDA-core) path
     Fp32Net f32{};
+    const float* w_row[MAX_LAYERS]{};       // W [N][K] row-major fp32: the right operand of dZ W in the backward
+    std::vector<int> dims;
     std::vector<float*> owned;
     // tcgen05 path
     bool tc_ok = false;
@@ -441,7 +444,14 @@ int aadff_psfnet_create(const float* const* weights, const float* const* biases,
         h->f32.bias[l] = db;
         h->f32.k[l] = K;
         h->f32.npad[l] = npad;
+        std::vector<float> wr(weights[l], weights[l] + (size_t)Nf * K);
+        float* dr = nullptr;
+        rc = upload(wr, &dr);
+        if (rc) { aadff_psfnet_destroy(h); return rc; }
+        h->owned.push_back(dr);
+        h->w_row[l] = dr;
     }
+    h->dims.assign(dims, dims + n_layers + 1);
 #define CREATE_TRY(expr)                                                                         \
     do {                                                                                         \
         cudaError_t _e = (expr);                                                                 \
@@ -822,6 +832,147 @@ int aadff_psfnet_pred_tc_f32(aadff_psfnet_t h, const float* inp, float* psf, int
     RenderArgs ra{};
     ra.ks = h->ks; ra.N = 1; ra.S = 1; ra.H = 1; ra.W = 1; ra.C = 1; ra.Ctot = 1;
     return launch_tc(h, ra, mode, static_cast<cudaStream_t>(stream), 0, -1, inp, psf, (long long)M);
+}
+
+}  // extern "C"
+
+// Workspace of aadff_psfnet_backward_f32 for chunks of cp probes: float offsets of each buffer (256-byte aligned).
+struct MlpGradLayout {
+    int cp = 0, lds = 0, ldz = 0, slices = 0;
+    size_t act[MAX_LAYERS]{}, s = 0, ssum = 0, dz[2]{}, part_w = 0, part_b = 0, floats = 0;
+};
+
+static MlpGradLayout mlp_grad_layout(const aadff_psfnet* h, long long M) {
+    MlpGradLayout g;
+    g.cp = (int)std::min<long long>((M + F32_TP - 1) / F32_TP * F32_TP, MG_CHUNK);
+    g.slices = (g.cp + MG_SLICE - 1) / MG_SLICE;
+    g.lds = (h->kk + 3) / 4 * 4;
+    g.ldz = g.lds;
+    size_t max_w = 0, max_n = 0;
+    for (int l = 0; l < h->n_layers; ++l) {
+        g.ldz = std::max(g.ldz, (h->dims[l + 1] + 3) / 4 * 4);
+        max_w = std::max(max_w, (size_t)h->dims[l] * h->dims[l + 1]);
+        max_n = std::max(max_n, (size_t)h->dims[l + 1]);
+    }
+    size_t off = 0;
+    auto take = [&](size_t n) { const size_t o = off; off += (n + 63) / 64 * 64; return o; };
+    for (int l = 1; l < h->n_layers; ++l) g.act[l] = take((size_t)g.cp * h->dims[l]);
+    g.s = take((size_t)g.cp * g.lds);
+    g.ssum = take((size_t)g.cp);
+    g.dz[0] = take((size_t)g.cp * g.ldz);
+    g.dz[1] = take((size_t)g.cp * g.ldz);
+    g.part_w = take((size_t)g.slices * max_w);
+    g.part_b = take((size_t)g.slices * max_n);
+    g.floats = off;
+    return g;
+}
+
+extern "C" {
+
+int64_t aadff_psfnet_backward_work_bytes(aadff_psfnet_t h, int64_t M) {
+    if (M < 0) return fail(AADFF_E_INVALID, "M must be >= 0");
+    if (!h) return fail(AADFF_E_INVALID, "net is NULL");
+    if (M == 0) return 0;
+    return (int64_t)(mlp_grad_layout(h, M).floats * sizeof(float));
+}
+
+int aadff_psfnet_backward_f32(aadff_psfnet_t h, const float* inp, const float* grad_psf, float* grad_inp,
+                              float* const* grad_weights, float* const* grad_biases, void* work, int64_t work_bytes,
+                              int64_t M, void* stream) {
+    // the checks that need no handle first: they are testable without a device
+    if (M < 0) return fail(AADFF_E_INVALID, "M must be >= 0");
+    if (!inp) return fail(AADFF_E_INVALID, "inp is NULL");
+    if (!grad_psf) return fail(AADFF_E_INVALID, "grad_psf is NULL");
+    if (reinterpret_cast<uintptr_t>(inp) % 16) return fail(AADFF_E_INVALID, "inp must be 16-byte aligned");
+    if (!grad_inp && !grad_weights && !grad_biases)
+        return fail(AADFF_E_INVALID, "no output requested: grad_inp, grad_weights and grad_biases are all NULL");
+    if (!h) return fail(AADFF_E_INVALID, "net is NULL");
+    const int L = h->n_layers;
+    int lowest = grad_inp ? 0 : L;                   // the lowest layer whose dZ is needed
+    for (int l = 0; l < L; ++l)
+        if ((grad_weights && grad_weights[l]) || (grad_biases && grad_biases[l])) lowest = std::min(lowest, l);
+    if (lowest == L)
+        return fail(AADFF_E_INVALID, "no output requested: grad_inp and every grad_weights / grad_biases entry are NULL");
+    const MlpGradLayout g = mlp_grad_layout(h, M);
+    if (M > 0 && !work) return fail(AADFF_E_INVALID, "work is NULL");
+    if (M > 0 && work_bytes < (int64_t)(g.floats * sizeof(float)))
+        return fail(AADFF_E_INVALID, "work_bytes is smaller than aadff_psfnet_backward_work_bytes(net, M)");
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return fail(AADFF_E_CUDA, "cannot select device");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    auto dW = [&](int l) { return grad_weights ? grad_weights[l] : nullptr; };
+    auto dB = [&](int l) { return grad_biases ? grad_biases[l] : nullptr; };
+    if (M == 0) {                                    // no probe: the parameter gradients are 0
+        for (int l = 0; l < L; ++l) {
+            if (dW(l)) CUDA_TRY(cudaMemsetAsync(dW(l), 0, (size_t)h->dims[l] * h->dims[l + 1] * sizeof(float), st));
+            if (dB(l)) CUDA_TRY(cudaMemsetAsync(dB(l), 0, (size_t)h->dims[l + 1] * sizeof(float), st));
+        }
+        return AADFF_OK;
+    }
+    float* ws = static_cast<float*>(work);
+    MlpActs acts{};
+    for (int l = 1; l < L; ++l) acts.act[l] = ws + g.act[l];
+    acts.s = ws + g.s;
+    acts.ssum = ws + g.ssum;
+    acts.lds = g.lds;
+    float* part_w = ws + g.part_w;
+    float* part_b = ws + g.part_b;
+    auto blocks = [](long long n, long long per, long long cap) { return (int)std::min<long long>((n + per - 1) / per, cap); };
+    for (long long m0 = 0; m0 < M; m0 += MG_CHUNK) {
+        const int valid = (int)std::min<long long>(MG_CHUNK, M - m0);
+        const int cp = (valid + F32_TP - 1) / F32_TP * F32_TP;
+        const int slices = (valid + MG_SLICE - 1) / MG_SLICE;
+        const int first = m0 == 0;
+        acts.cp = cp;
+        if (int rc = launch(mlp_fp32_store_kernel, blocks(cp, F32_TP, (long long)h->num_sms * 8), F32_NT, F32_SMEM, st,
+                            h->f32, inp, m0, (long long)M, acts))
+            return rc;
+        int cur = 0;                                 // dz[cur] holds dZ of the layer being processed
+        float* dz = ws + g.dz[cur];
+        if (int rc = launch(mlp_head_backward_kernel, blocks(cp, 8, 1ll << 30), 256, 0, st, (const float*)acts.s, g.lds,
+                            (const float*)acts.ssum, grad_psf, m0, valid, cp, h->kk, dz, (h->kk + 3) / 4 * 4))
+            return rc;
+        for (int l = L - 1; l >= lowest; --l) {
+            const int K = h->dims[l], N = h->dims[l + 1], ldz = (N + 3) / 4 * 4;
+            const float* act = l ? acts.act[l] : inp + m0 * 4;
+            if (dW(l)) {                             // dW_l = dZ_l^T A_l, one partial per probe slice
+                const long long n = (long long)N * K;
+                if (int rc = launch(mlp_grad_gemm_kernel<false, MG_PLAIN>,
+                                    dim3((K + MG_BN - 1) / MG_BN, (N + MG_BM - 1) / MG_BM, slices), MG_NT, 0, st,
+                                    (const float*)dz, (long long)ldz, act, (long long)K, part_w, (long long)K, N, K, valid,
+                                    MG_SLICE, n, (const float*)nullptr))
+                    return rc;
+                if (int rc = launch(mlp_grad_reduce_kernel, blocks(n, 256, (long long)h->num_sms * 8), 256, 0, st,
+                                    (const float*)part_w, n, slices, dW(l), first))
+                    return rc;
+            }
+            if (dB(l)) {                             // db_l = column sums of dZ_l, one partial per probe slice
+                if (int rc = launch(mlp_colsum_kernel, dim3((N + 255) / 256, slices), 256, 0, st, (const float*)dz, ldz, N,
+                                    valid, part_b))
+                    return rc;
+                if (int rc = launch(mlp_grad_reduce_kernel, blocks(N, 256, (long long)h->num_sms * 8), 256, 0, st,
+                                    (const float*)part_b, (long long)N, slices, dB(l), first))
+                    return rc;
+            }
+            if (l > lowest) {                        // dZ_{l-1} = (dZ_l W_l) masked by A_l > 0
+                float* dz_next = ws + g.dz[cur ^ 1];
+                if (int rc = launch(mlp_grad_gemm_kernel<true, MG_RELU_MASK>,
+                                    dim3((K + MG_BN - 1) / MG_BN, (cp + MG_BM - 1) / MG_BM, 1), MG_NT, 0, st,
+                                    (const float*)dz, (long long)ldz, h->w_row[l], (long long)K, dz_next, (long long)K,
+                                    cp, K, N, 0, 0ll, (const float*)acts.act[l]))
+                    return rc;
+                cur ^= 1;
+                dz = dz_next;
+            } else if (l == 0 && grad_inp) {         // dX = dZ_0 W_0, rows of this chunk
+                if (int rc = launch(mlp_grad_gemm_kernel<true, MG_PLAIN>,
+                                    dim3((K + MG_BN - 1) / MG_BN, (valid + MG_BM - 1) / MG_BM, 1), MG_NT, 0, st,
+                                    (const float*)dz, (long long)ldz, h->w_row[0], (long long)K, grad_inp + m0 * K,
+                                    (long long)K, valid, K, N, 0, 0ll, (const float*)nullptr))
+                    return rc;
+            }
+        }
+    }
+    return AADFF_OK;
 }
 
 int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, int N, int C, int H, int W, int ks,

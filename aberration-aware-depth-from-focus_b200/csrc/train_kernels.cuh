@@ -93,9 +93,16 @@ __global__ void __launch_bounds__(256) train_colsum_kernel(const float* __restri
     db[j] = s;
 }
 
+// dL/dz_j of the head s = sigmoid(z), p = s / max(S, 1e-12), S = sum s, from g = dL/dp_j and gp = sum_i g_i p_i:
+//   dL/ds_j = (g_j - gp) / S,   dL/dz_j = dL/ds_j * s_j (1 - s_j);
+// for S below the clamp the denominator is constant: no normalisation gradient (F.normalize's clamp_min).
+__device__ __forceinline__ float head_dz(float s, float g, float gp, float S, float denom) {
+    const float ds = (S > 1e-12f) ? (g - gp) / denom : g / denom;
+    return ds * s * (1.0f - s);
+}
+
 // Head: z -> s = sigmoid(z) -> p = s / max(sum|s|, 1e-12) (psfnet_arch.py:39-46) -> loss += sum (p - t)^2 / (M*kk)
-// -> dZ = dL/dz.  One warp per probe.  With g = dL/dp = 2 (p - t) / (M*kk):
-//   dL/ds_j = (g_j - sum_i g_i p_i) / S,   dL/dz_j = dL/ds_j * s_j (1 - s_j).
+// -> dZ = dL/dz (head_dz).  One warp per probe, g = dL/dp = 2 (p - t) / (M*kk).
 __global__ void __launch_bounds__(256)
 train_head_kernel(const float* __restrict__ z, const float* __restrict__ target, float* __restrict__ p_out,
                   float* __restrict__ dZ, float* __restrict__ loss, int M, int kk) {
@@ -125,9 +132,7 @@ train_head_kernel(const float* __restrict__ z, const float* __restrict__ target,
     for (int j = lane; j < kk; j += 32) {
         const float s = 1.0f / (1.0f + expf(-zr[j]));
         const float g = scale * (s / denom - tr[j]);
-        // for S below the clamp the denominator is constant: no normalisation gradient (F.normalize's clamp_min)
-        const float ds = (S > 1e-12f) ? (g - gp) / denom : g / denom;
-        dZ[(long long)warp * kk + j] = ds * s * (1.0f - s);
+        dZ[(long long)warp * kk + j] = head_dz(s, g, gp, S, denom);
     }
     if (lane == 0) atomicAdd(loss, l / ((float)M * (float)kk));
 }

@@ -95,6 +95,26 @@ int aadff_psfnet_pred_f32(aadff_psfnet_t net, const float* inp, float* psf, int6
  * aadff_render_stack_f32 (AADFF_MODE_FP32 forwards to the call above).  inp must be 16-byte aligned.          */
 int aadff_psfnet_pred_tc_f32(aadff_psfnet_t net, const float* inp, float* psf, int64_t M, int mode, void* stream);
 
+/* Backward of aadff_psfnet_pred_f32 (what autograd does through the reference's MLP, deeplens/psfnet_arch.py:44-47):
+ * grad_psf = dL/dpsf [M, ks*ks] -> grad_inp = dL/dinp [M,4], grad_weights[l] = dL/d net.{2l}.weight ([dims[l+1],
+ * dims[l]] row-major), grad_biases[l] = dL/d net.{2l}.bias [dims[l+1]].  inp (16-byte aligned), grad_psf and the outputs
+ * are device pointers; grad_weights / grad_biases are HOST arrays of n_layers device pointers.  Either array, any entry
+ * of them and grad_inp may be NULL (that gradient is not computed: a layer without a weight gradient costs no dW
+ * GEMM), but at least one output must be requested.  Outputs are overwritten, not accumulated.  Hidden ReLUs pass the
+ * gradient where relu(z) > 0; the head is sigmoid + L1 normalisation with F.normalize's 1e-12 clamp.
+ * The activations are recomputed, not stored: probes are processed in chunks of 16384, each chunk recomputes its
+ * activations with the forward's exact arithmetic, then runs the backward from the head down.  `work` is device memory
+ * of at least aadff_psfnet_backward_work_bytes(net, M) bytes, which stays bounded whatever M is: per chunk probe the
+ * input of every layer, the head's sigmoid outputs and two dZ buffers, plus dW partial sums over slices of 256
+ * probes -- 213 778 432 bytes (204 MiB) for the rf50mm network (11 layers, ks = 11) from M >= 16384 on.  The size query returns a negative
+ * AADFF_E_* code for arguments the backward would refuse.  dW and db are per-slice partial sums added in slice order,
+ * chunk after chunk: no atomics, two calls give bit-identical results.  Stream-ordered, no allocation, no
+ * synchronisation, CUDA-graph capturable.                                                                             */
+int64_t aadff_psfnet_backward_work_bytes(aadff_psfnet_t net, int64_t M);
+int aadff_psfnet_backward_f32(aadff_psfnet_t net, const float* inp, const float* grad_psf, float* grad_inp,
+                              float* const* grad_weights, float* const* grad_biases, void* work, int64_t work_bytes,
+                              int64_t M, void* stream);
+
 /* Replaces local_psf_render (deeplens/render_psf.py:76-107) for a PSF tensor in memory:
  *   img [N,C,H,W], psf [N,H,W,ks,ks] -> out [N,C,H,W]; device pointers.                        */
 int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, int N, int C, int H, int W, int ks,
