@@ -94,6 +94,93 @@ class _PSFNetMLP(torch.autograd.Function):
         return (None, grad_inp) + tuple(grads)
 
 
+def _launch_stack(nat, img, depth, foc, out_ptr, strides, m, d_min, d_max, rows=None):
+    """aadff_render_stack_f32 (or its tile-row variant) for fp32 contiguous img [N,C,H,W], depth [N,H,W], foc [N,S]."""
+    N, C, H, W = img.shape
+    S = foc.shape[1]
+    if N * C * S * H * W == 0:      # empty batch: nothing to launch (data_ptr() of an empty tensor is NULL)
+        return
+    arr = (_nat.ctypes.c_int64 * 5)(*strides)
+    with torch.cuda.device(img.device):
+        st = torch.cuda.current_stream().cuda_stream
+        if rows is None:
+            _nat.check(_nat.lib.aadff_render_stack_f32(
+                nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, arr,
+                N, C, S, H, W, d_min, d_max, m, st))
+        else:
+            _nat.check(_nat.lib.aadff_render_stack_rows_f32(
+                nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, arr,
+                N, C, S, H, W, d_min, d_max, m, int(rows[0]), int(rows[1]), st))
+
+
+# element strides (n, c, s, h, w) of each output layout of render / render_stack
+def _layout_strides(layout, N, C, S, H, W):
+    if layout == "NCHW":
+        return (N, C, H, W), (C * H * W, H * W, 0, W, 1)
+    if layout == "BCSHW":
+        return (N, C, S, H, W), (C * S * H * W, S * H * W, H * W, W, 1)
+    if layout == "BSCHW":
+        return (N, S, C, H, W), (S * C * H * W, H * W, C * H * W, W, 1)
+    raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
+
+
+class _RenderStack(torch.autograd.Function):
+    """out = render_stack(img, depth, foc) with the network (w0, b0, w1, b1, ...) of the handle `nat`: fp32 contiguous
+    img [N,C,H,W], depth [N,H,W], foc [N,S] on the handle's device, `layout` one of _layout_strides'.  The forward is
+    the launch of the no-grad path, so the output is bit-identical to it; the backward
+    (aadff_render_stack_backward_f32) recomputes the PSFs and activations band by band and reads the weights of the
+    same handle, which the graph keeps alive.  The saved inputs make autograd refuse a backward after an in-place change
+    to them."""
+
+    @staticmethod
+    def forward(ctx, nat, m, layout, d_min, d_max, img, depth, foc, *params):
+        N, C, H, W = img.shape
+        shape, strides = _layout_strides(layout, N, C, foc.shape[1], H, W)
+        out = torch.empty(shape, device=img.device, dtype=torch.float32)
+        _launch_stack(nat, img, depth, foc, out.data_ptr(), strides, m, d_min, d_max)
+        ctx.nat, ctx.m, ctx.layout, ctx.d_min, ctx.d_max = nat, m, layout, d_min, d_max
+        ctx.save_for_backward(img, depth, foc, *params)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        img, depth, foc, *params = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        need_img, need_depth, need_foc, need_p = need[5], need[6], need[7], need[8:]
+        grad_img = torch.empty_like(img) if need_img else None
+        grad_depth = torch.empty_like(depth) if need_depth else None
+        grad_foc = torch.empty_like(foc) if need_foc else None
+        grads = [torch.empty_like(p) if n else None for p, n in zip(params, need_p)]
+        head = (None,) * 5
+        N, C, H, W = img.shape
+        S = foc.shape[1]
+        if not (need_img or need_depth or need_foc or any(need_p)):
+            return head + (None, None, None) + tuple(grads)
+        if N * C * S * H * W == 0:      # no pixel: the parameter gradients are 0, the other gradients are empty
+            return head + (grad_img, grad_depth, grad_foc) + tuple(g.zero_() if g is not None else None for g in grads)
+        nat = ctx.nat
+        g = grad_out.to(torch.float32).contiguous()
+        _, strides = _layout_strides(ctx.layout, N, C, S, H, W)
+        arr = (_nat.ctypes.c_int64 * 5)(*strides)
+        c_f32p = _nat.ctypes.POINTER(_nat.ctypes.c_float)
+        ptr = lambda t: _nat.ctypes.cast(_nat.ctypes.c_void_p(t.data_ptr()), c_f32p) if t is not None else None
+        n = nat.n_layers
+        wp = (c_f32p * n)(*[ptr(t) for t in grads[0::2]])
+        bp = (c_f32p * n)(*[ptr(t) for t in grads[1::2]])
+        dp = lambda t: t.data_ptr() if t is not None else None
+        with torch.cuda.device(img.device):
+            work_bytes = _nat.lib.aadff_render_stack_backward_work_bytes(nat.handle, H, W)
+            if work_bytes < 0:
+                _nat.check(int(work_bytes))
+            work = torch.empty(work_bytes, dtype=torch.uint8, device=img.device)
+            _nat.check(_nat.lib.aadff_render_stack_backward_f32(
+                nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), g.data_ptr(), arr, dp(grad_img),
+                dp(grad_depth), dp(grad_foc), wp, bp, N, C, S, H, W, ctx.d_min, ctx.d_max, ctx.m, work.data_ptr(),
+                work_bytes, torch.cuda.current_stream().cuda_stream))
+        return head + (grad_img, grad_depth, grad_foc) + tuple(grads)
+
+
 class PSFNet(nn.Module):
     def __init__(self, filename=None, model_name='mlp', kernel_size=11, sensor_res=(512, 512), device='cuda',
                  mode=None):
@@ -188,23 +275,11 @@ class PSFNet(nn.Module):
         return psf.reshape(*psf.shape[:-1], self.kernel_size, self.kernel_size)
 
     def _launch(self, img, depth, foc, out_ptr, strides, mode, rows=None):
-        nat = PSFNet.native(self)
-        N, C, H, W = img.shape
-        S = foc.shape[1]
-        if N * C * S * H * W == 0:      # empty batch: nothing to launch (data_ptr() of an empty tensor is NULL)
-            return
-        arr = (_nat.ctypes.c_int64 * 5)(*strides)
-        m = _nat.MODES[mode or getattr(self, "mode", None) or os.environ.get("AADFF_MODE", "parity")]
-        with torch.cuda.device(img.device):
-            st = torch.cuda.current_stream().cuda_stream
-            if rows is None:
-                _nat.check(_nat.lib.aadff_render_stack_f32(
-                    nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, arr,
-                    N, C, S, H, W, float(self.d_min), float(self.d_max), m, st))
-            else:
-                _nat.check(_nat.lib.aadff_render_stack_rows_f32(
-                    nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, arr,
-                    N, C, S, H, W, float(self.d_min), float(self.d_max), m, int(rows[0]), int(rows[1]), st))
+        _launch_stack(PSFNet.native(self), img, depth, foc, out_ptr, strides, PSFNet._mode(self, mode),
+                      float(self.d_min), float(self.d_max), rows)
+
+    def _mode(self, mode):
+        return _nat.MODES[mode or getattr(self, "mode", None) or os.environ.get("AADFF_MODE", "parity")]
 
     def _prep(self, img, depth):
         nat = PSFNet.native(self)
@@ -214,46 +289,80 @@ class PSFNet(nn.Module):
         depth = depth.detach().to(dev, torch.float32).reshape(N, H, W).contiguous()
         return img, depth, dev
 
-    @torch.no_grad()
-    def render(self, img, depth, foc_dist, mode=None):
+    def _render_grad(self, img, depth, foc, layout, mode):
+        """The differentiable render: conversions to fp32 contiguous tensors on the handle's device as ordinary torch
+        ops (gradients return in each input's own shape, dtype and device), then _RenderStack.  foc is [N] or [N,S]."""
+        nat = PSFNet.native(self)
+        dev = torch.device(f"cuda:{nat.device_index}")
+        img = img.to(dev, torch.float32).contiguous()
+        N, C, H, W = img.shape
+        depth = depth.to(dev, torch.float32).reshape(N, H, W).contiguous()
+        foc = torch.as_tensor(foc).to(dev, torch.float32)
+        # as the no-grad paths: [N], [N,S] or [S] for one image; an empty batch keeps its slice count
+        foc = (foc.reshape(N, -1) if N else foc.reshape(0, foc.shape[-1] if foc.dim() > 1 else 1)).contiguous()
+        params = []
+        for l in _linear_layers(self.psfnet):
+            params += [l.weight.to(dev, torch.float32).contiguous(), l.bias.to(dev, torch.float32).contiguous()]
+        return _RenderStack.apply(nat, PSFNet._mode(self, mode), layout, float(self.d_min), float(self.d_max),
+                                  img, depth, foc, *params)
+
+    def _wants_grad(self, differentiable, *inputs):
+        """differentiable=True, grad mode on, and an input or a parameter of the network requiring grad."""
+        return differentiable and torch.is_grad_enabled() and (
+            any(torch.is_tensor(t) and t.requires_grad for t in inputs) or
+            any(p.requires_grad for p in self.psfnet.parameters()))
+
+    def render(self, img, depth, foc_dist, mode=None, differentiable=False):
         """Render image with aif image and depth map.
 
         img [N,C,H,W], depth [N,1,H,W] (mm, negative), foc_dist [N] (mm, negative) -> [N,C,H,W];
         or img [C,H,W], depth [H,W], scalar foc_dist -> [1,C,H,W].
+
+        The output is detached, as the reference's no_grad render.  With differentiable=True, grad mode on and img,
+        depth, foc_dist or a network parameter requiring grad, it is differentiable in all of them (same values).
         """
         if img.dim() == 3:
             img = img.unsqueeze(0)
             depth = depth.reshape(1, *depth.shape[-2:])
-            foc_dist = torch.as_tensor([float(foc_dist)], dtype=torch.float32)
+            if not (torch.is_tensor(foc_dist) and PSFNet._wants_grad(self, differentiable, img, depth, foc_dist)):
+                foc_dist = torch.as_tensor([float(foc_dist)], dtype=torch.float32)
         elif img.dim() != 4:
             raise ValueError(f"render expects a [N,C,H,W] or [C,H,W] image, got shape {tuple(img.shape)}")
-        img, depth, dev = PSFNet._prep(self, img, depth)
-        N, C, H, W = img.shape
-        foc = torch.as_tensor(foc_dist).detach().to(dev, torch.float32).reshape(N, 1).contiguous()
-        out = torch.empty_like(img)
-        PSFNet._launch(self, img, depth, foc, out.data_ptr(), (C * H * W, H * W, 0, W, 1), mode)
-        return out
+        if PSFNet._wants_grad(self, differentiable, img, depth, foc_dist):
+            return PSFNet._render_grad(self, img, depth, foc_dist, "NCHW", mode)
+        with torch.no_grad():
+            img, depth, dev = PSFNet._prep(self, img, depth)
+            N, C, H, W = img.shape
+            foc = torch.as_tensor(foc_dist).detach().to(dev, torch.float32).reshape(N, 1).contiguous()
+            out = torch.empty_like(img)
+            PSFNet._launch(self, img, depth, foc, out.data_ptr(), (C * H * W, H * W, 0, W, 1), mode)
+            return out
 
-    @torch.no_grad()
-    def render_stack(self, img, depth, foc_dists, layout="BCSHW", mode=None):
+    def render_stack(self, img, depth, foc_dists, layout="BCSHW", mode=None, differentiable=False):
         """All S focal slices in one launch: foc_dists [N,S] (mm, negative) -> [N,C,S,H,W]
-        (== torch.stack([render(img, depth, foc_dists[:, s]) for s], dim=2)), or [N,S,C,H,W]."""
+        (== torch.stack([render(img, depth, foc_dists[:, s]) for s], dim=2)), or [N,S,C,H,W].
+        differentiable=True: as for ``render``."""
         if img.dim() != 4:
             raise ValueError("render_stack expects a [N,C,H,W] image")
-        img, depth, dev = PSFNet._prep(self, img, depth)
-        N, C, H, W = img.shape
-        foc = foc_dists.detach().to(dev, torch.float32).reshape(N, -1).contiguous()
-        S = foc.shape[1]
-        if layout == "BCSHW":
-            out = torch.empty(N, C, S, H, W, device=dev, dtype=torch.float32)
-            strides = (C * S * H * W, S * H * W, H * W, W, 1)
-        elif layout == "BSCHW":
-            out = torch.empty(N, S, C, H, W, device=dev, dtype=torch.float32)
-            strides = (S * C * H * W, H * W, C * H * W, W, 1)
-        else:
-            raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
-        PSFNet._launch(self, img, depth, foc, out.data_ptr(), strides, mode)
-        return out
+        if PSFNet._wants_grad(self, differentiable, img, depth, foc_dists):
+            if layout not in ("BCSHW", "BSCHW"):
+                raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
+            return PSFNet._render_grad(self, img, depth, foc_dists, layout, mode)
+        with torch.no_grad():
+            img, depth, dev = PSFNet._prep(self, img, depth)
+            N, C, H, W = img.shape
+            foc = foc_dists.detach().to(dev, torch.float32).reshape(N, -1).contiguous()
+            S = foc.shape[1]
+            if layout == "BCSHW":
+                out = torch.empty(N, C, S, H, W, device=dev, dtype=torch.float32)
+                strides = (C * S * H * W, S * H * W, H * W, W, 1)
+            elif layout == "BSCHW":
+                out = torch.empty(N, S, C, H, W, device=dev, dtype=torch.float32)
+                strides = (S * C * H * W, H * W, C * H * W, W, 1)
+            else:
+                raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
+            PSFNet._launch(self, img, depth, foc, out.data_ptr(), strides, mode)
+            return out
 
     @torch.no_grad()
     def render_stack_rows(self, img, depth, foc_dists, tile_row_begin, tile_row_end, mode=None):
@@ -352,7 +461,8 @@ class PSFNet(nn.Module):
 
 
 # names install() grafts onto the reference's PSFNet (everything render/pred need, nothing the ray tracer owns)
-PSFNET_GRAFT = ("native", "refresh", "_mlp_eval", "pred", "_launch", "_prep", "render", "render_stack",
+PSFNET_GRAFT = ("native", "refresh", "_mlp_eval", "pred", "_launch", "_mode", "_prep", "_render_grad", "_wants_grad",
+                "render", "render_stack",
                 "render_stack_rows", "simulate_focal_stack", "train_psfnet")
 
 

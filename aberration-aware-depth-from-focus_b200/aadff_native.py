@@ -109,6 +109,13 @@ def _load() -> ctypes.CDLL:
     lib.aadff_psfnet_backward_f32.argtypes = [ctypes.c_void_p] * 4 + [ctypes.POINTER(c_f32p)] * 2 + \
                                              [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p]
     lib.aadff_psfnet_backward_f32.restype = ctypes.c_int
+    lib.aadff_render_stack_backward_work_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int]
+    lib.aadff_render_stack_backward_work_bytes.restype = ctypes.c_int64
+    lib.aadff_render_stack_backward_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.POINTER(ctypes.c_int64)] + \
+                                                   [ctypes.c_void_p] * 3 + [ctypes.POINTER(c_f32p)] * 2 + \
+                                                   [ctypes.c_int] * 5 + [ctypes.c_float, ctypes.c_float, ctypes.c_int,
+                                                                         ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
+    lib.aadff_render_stack_backward_f32.restype = ctypes.c_int
     lib.aadff_local_psf_render_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
     lib.aadff_local_psf_render_backward_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
     lib.aadff_render_psf_map_backward_work_bytes.argtypes = [ctypes.c_int] * 6 + [ctypes.POINTER(ctypes.c_int)] * 2

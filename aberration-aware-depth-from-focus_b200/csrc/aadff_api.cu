@@ -26,6 +26,7 @@
 #include "psf_conv_grad_kernel.cuh"
 #include "train_kernels.cuh"
 #include "mlp_grad_kernel.cuh"
+#include "render_grad_kernel.cuh"
 #include "preprocess_kernel.cuh"
 #include "spline_rotate_kernel.cuh"
 #include "econ_calib.h"
@@ -867,6 +868,65 @@ static MlpGradLayout mlp_grad_layout(const aadff_psfnet* h, long long M) {
     return g;
 }
 
+static int grid_blocks(long long n, long long per, long long cap) { return (int)std::min<long long>((n + per - 1) / per, cap); }
+
+// One chunk of the MLP backward below the head, shared by aadff_psfnet_backward_f32 and
+// aadff_render_stack_backward_f32.  dZ of the head is in ws + g.dz[0], acts holds the chunk's recomputed activations
+// and inp its probes [valid][4].  From the head down to layer `lowest`: each requested dW_l / db_l (partial sums over
+// MG_SLICE probes, added to the running total of the earlier chunks unless `first`) and, when grad_inp is not NULL,
+// dX = dZ_0 W_0 into grad_inp [valid][4].
+static int mlp_backward_layers(const aadff_psfnet* h, const MlpGradLayout& g, float* ws, const MlpActs& acts,
+                               const float* inp, int valid, int cp, int lowest, int first, float* const* grad_weights,
+                               float* const* grad_biases, float* grad_inp, cudaStream_t st) {
+    auto dW = [&](int l) { return grad_weights ? grad_weights[l] : nullptr; };
+    auto dB = [&](int l) { return grad_biases ? grad_biases[l] : nullptr; };
+    float* part_w = ws + g.part_w;
+    float* part_b = ws + g.part_b;
+    const int slices = (valid + MG_SLICE - 1) / MG_SLICE;
+    int cur = 0;                                     // dz[cur] holds dZ of the layer being processed
+    float* dz = ws + g.dz[cur];
+    for (int l = h->n_layers - 1; l >= lowest; --l) {
+        const int K = h->dims[l], N = h->dims[l + 1], ldz = (N + 3) / 4 * 4;
+        const float* act = l ? acts.act[l] : inp;
+        if (dW(l)) {                                 // dW_l = dZ_l^T A_l, one partial per probe slice
+            const long long n = (long long)N * K;
+            if (int rc = launch(mlp_grad_gemm_kernel<false, MG_PLAIN>,
+                                dim3((K + MG_BN - 1) / MG_BN, (N + MG_BM - 1) / MG_BM, slices), MG_NT, 0, st,
+                                (const float*)dz, (long long)ldz, act, (long long)K, part_w, (long long)K, N, K, valid,
+                                MG_SLICE, n, (const float*)nullptr))
+                return rc;
+            if (int rc = launch(mlp_grad_reduce_kernel, grid_blocks(n, 256, (long long)h->num_sms * 8), 256, 0, st,
+                                (const float*)part_w, n, slices, dW(l), first))
+                return rc;
+        }
+        if (dB(l)) {                                 // db_l = column sums of dZ_l, one partial per probe slice
+            if (int rc = launch(mlp_colsum_kernel, dim3((N + 255) / 256, slices), 256, 0, st, (const float*)dz, ldz, N,
+                                valid, part_b))
+                return rc;
+            if (int rc = launch(mlp_grad_reduce_kernel, grid_blocks(N, 256, (long long)h->num_sms * 8), 256, 0, st,
+                                (const float*)part_b, (long long)N, slices, dB(l), first))
+                return rc;
+        }
+        if (l > lowest) {                            // dZ_{l-1} = (dZ_l W_l) masked by A_l > 0
+            float* dz_next = ws + g.dz[cur ^ 1];
+            if (int rc = launch(mlp_grad_gemm_kernel<true, MG_RELU_MASK>,
+                                dim3((K + MG_BN - 1) / MG_BN, (cp + MG_BM - 1) / MG_BM, 1), MG_NT, 0, st,
+                                (const float*)dz, (long long)ldz, h->w_row[l], (long long)K, dz_next, (long long)K,
+                                cp, K, N, 0, 0ll, (const float*)acts.act[l]))
+                return rc;
+            cur ^= 1;
+            dz = dz_next;
+        } else if (l == 0 && grad_inp) {             // dX = dZ_0 W_0, rows of this chunk
+            if (int rc = launch(mlp_grad_gemm_kernel<true, MG_PLAIN>,
+                                dim3((K + MG_BN - 1) / MG_BN, (valid + MG_BM - 1) / MG_BM, 1), MG_NT, 0, st,
+                                (const float*)dz, (long long)ldz, h->w_row[0], (long long)K, grad_inp, (long long)K,
+                                valid, K, N, 0, 0ll, (const float*)nullptr))
+                return rc;
+        }
+    }
+    return AADFF_OK;
+}
+
 extern "C" {
 
 int64_t aadff_psfnet_backward_work_bytes(aadff_psfnet_t h, int64_t M) {
@@ -915,63 +975,162 @@ int aadff_psfnet_backward_f32(aadff_psfnet_t h, const float* inp, const float* g
     acts.s = ws + g.s;
     acts.ssum = ws + g.ssum;
     acts.lds = g.lds;
-    float* part_w = ws + g.part_w;
-    float* part_b = ws + g.part_b;
-    auto blocks = [](long long n, long long per, long long cap) { return (int)std::min<long long>((n + per - 1) / per, cap); };
+    auto blocks = grid_blocks;
     for (long long m0 = 0; m0 < M; m0 += MG_CHUNK) {
         const int valid = (int)std::min<long long>(MG_CHUNK, M - m0);
         const int cp = (valid + F32_TP - 1) / F32_TP * F32_TP;
-        const int slices = (valid + MG_SLICE - 1) / MG_SLICE;
         const int first = m0 == 0;
         acts.cp = cp;
         if (int rc = launch(mlp_fp32_store_kernel, blocks(cp, F32_TP, (long long)h->num_sms * 8), F32_NT, F32_SMEM, st,
                             h->f32, inp, m0, (long long)M, acts))
             return rc;
-        int cur = 0;                                 // dz[cur] holds dZ of the layer being processed
-        float* dz = ws + g.dz[cur];
+        float* dz = ws + g.dz[0];
         if (int rc = launch(mlp_head_backward_kernel, blocks(cp, 8, 1ll << 30), 256, 0, st, (const float*)acts.s, g.lds,
                             (const float*)acts.ssum, grad_psf, m0, valid, cp, h->kk, dz, (h->kk + 3) / 4 * 4))
             return rc;
-        for (int l = L - 1; l >= lowest; --l) {
-            const int K = h->dims[l], N = h->dims[l + 1], ldz = (N + 3) / 4 * 4;
-            const float* act = l ? acts.act[l] : inp + m0 * 4;
-            if (dW(l)) {                             // dW_l = dZ_l^T A_l, one partial per probe slice
-                const long long n = (long long)N * K;
-                if (int rc = launch(mlp_grad_gemm_kernel<false, MG_PLAIN>,
-                                    dim3((K + MG_BN - 1) / MG_BN, (N + MG_BM - 1) / MG_BM, slices), MG_NT, 0, st,
-                                    (const float*)dz, (long long)ldz, act, (long long)K, part_w, (long long)K, N, K, valid,
-                                    MG_SLICE, n, (const float*)nullptr))
-                    return rc;
-                if (int rc = launch(mlp_grad_reduce_kernel, blocks(n, 256, (long long)h->num_sms * 8), 256, 0, st,
-                                    (const float*)part_w, n, slices, dW(l), first))
-                    return rc;
-            }
-            if (dB(l)) {                             // db_l = column sums of dZ_l, one partial per probe slice
-                if (int rc = launch(mlp_colsum_kernel, dim3((N + 255) / 256, slices), 256, 0, st, (const float*)dz, ldz, N,
-                                    valid, part_b))
-                    return rc;
-                if (int rc = launch(mlp_grad_reduce_kernel, blocks(N, 256, (long long)h->num_sms * 8), 256, 0, st,
-                                    (const float*)part_b, (long long)N, slices, dB(l), first))
-                    return rc;
-            }
-            if (l > lowest) {                        // dZ_{l-1} = (dZ_l W_l) masked by A_l > 0
-                float* dz_next = ws + g.dz[cur ^ 1];
-                if (int rc = launch(mlp_grad_gemm_kernel<true, MG_RELU_MASK>,
-                                    dim3((K + MG_BN - 1) / MG_BN, (cp + MG_BM - 1) / MG_BM, 1), MG_NT, 0, st,
-                                    (const float*)dz, (long long)ldz, h->w_row[l], (long long)K, dz_next, (long long)K,
-                                    cp, K, N, 0, 0ll, (const float*)acts.act[l]))
-                    return rc;
-                cur ^= 1;
-                dz = dz_next;
-            } else if (l == 0 && grad_inp) {         // dX = dZ_0 W_0, rows of this chunk
-                if (int rc = launch(mlp_grad_gemm_kernel<true, MG_PLAIN>,
-                                    dim3((K + MG_BN - 1) / MG_BN, (valid + MG_BM - 1) / MG_BM, 1), MG_NT, 0, st,
-                                    (const float*)dz, (long long)ldz, h->w_row[0], (long long)K, grad_inp + m0 * K,
-                                    (long long)K, valid, K, N, 0, 0ll, (const float*)nullptr))
-                    return rc;
-            }
-        }
+        if (int rc = mlp_backward_layers(h, g, ws, acts, inp + m0 * 4, valid, cp, lowest, first, grad_weights, grad_biases,
+                                         grad_inp ? grad_inp + m0 * h->dims[0] : nullptr, st))
+            return rc;
     }
+    return AADFF_OK;
+}
+
+}  // extern "C"
+
+// Workspace of aadff_render_stack_backward_f32 for bands of rows * W pixels: the band's probes, its PSFs (for dimg),
+// dX, then the MLP backward's buffers for one chunk of that size (float offsets, 256-byte aligned).
+struct RenderGradLayout {
+    int rows = 0;
+    size_t probes = 0, psf = 0, dx = 0, mlp = 0, floats = 0;
+    MlpGradLayout g;
+};
+
+static RenderGradLayout render_grad_layout(const aadff_psfnet* h, int H, int W) {
+    RenderGradLayout r;
+    r.rows = std::min(H, MG_CHUNK / W);
+    const size_t px = (size_t)r.rows * W;
+    size_t off = 0;
+    auto take = [&](size_t n) { const size_t o = off; off += (n + 63) / 64 * 64; return o; };
+    r.probes = take(px * 4);
+    r.psf = take(px * h->kk);
+    r.dx = take(px * 4);
+    r.mlp = off;
+    r.g = mlp_grad_layout(h, (long long)px);
+    r.floats = off + r.g.floats;
+    return r;
+}
+
+extern "C" {
+
+int64_t aadff_render_stack_backward_work_bytes(aadff_psfnet_t h, int H, int W) {
+    if (H < 1 || W < 1) return fail(AADFF_E_INVALID, "H and W must be >= 1");
+    if (W > MG_CHUNK) return fail(AADFF_E_INVALID, "W must be <= 16384");
+    if (!h) return fail(AADFF_E_INVALID, "net is NULL");
+    return (int64_t)(render_grad_layout(h, H, W).floats * sizeof(float));
+}
+
+int aadff_render_stack_backward_f32(aadff_psfnet_t h, const float* img, const float* depth, const float* foc,
+                                    const float* grad_out, const int64_t grad_out_strides[5], float* grad_img,
+                                    float* grad_depth, float* grad_foc, float* const* grad_weights,
+                                    float* const* grad_biases, int N, int C, int S, int H, int W, float d_min,
+                                    float d_max, int mode, void* work, int64_t work_bytes, void* stream) {
+    // the checks that need no handle first: they are testable without a device
+    if (N < 0) return fail(AADFF_E_INVALID, "N must be >= 0");
+    if (C < 1) return fail(AADFF_E_INVALID, "C must be >= 1");
+    if (S < 1) return fail(AADFF_E_INVALID, "S must be >= 1");
+    if (H < 1 || W < 1) return fail(AADFF_E_INVALID, "H and W must be >= 1");
+    if (W > MG_CHUNK) return fail(AADFF_E_INVALID, "W must be <= 16384");
+    if (mode < 0 || mode > AADFF_MODE_ECON8) return fail(AADFF_E_INVALID, "mode is unknown");
+    if (!(d_max != d_min)) return fail(AADFF_E_INVALID, "d_max must differ from d_min");
+    if (!img) return fail(AADFF_E_INVALID, "img is NULL");
+    if (!depth) return fail(AADFF_E_INVALID, "depth is NULL");
+    if (!foc) return fail(AADFF_E_INVALID, "foc is NULL");
+    if (!grad_out) return fail(AADFF_E_INVALID, "grad_out is NULL");
+    if (!grad_out_strides) return fail(AADFF_E_INVALID, "grad_out_strides is NULL");
+    if (!grad_img && !grad_depth && !grad_foc && !grad_weights && !grad_biases)
+        return fail(AADFF_E_INVALID,
+                    "no output requested: grad_img, grad_depth, grad_foc, grad_weights and grad_biases are all NULL");
+    // the band buffers inside `work` sit at multiples of 256 bytes from it (float4 probes, tensor-core pred input)
+    if (reinterpret_cast<uintptr_t>(work) % 256) return fail(AADFF_E_INVALID, "work must be 256-byte aligned");
+    if (!h) return fail(AADFF_E_INVALID, "net is NULL");
+    const int L = h->n_layers;
+    int lowest = (grad_depth || grad_foc) ? 0 : L;   // the lowest layer whose dZ is needed (L: no MLP backward)
+    for (int l = 0; l < L; ++l)
+        if ((grad_weights && grad_weights[l]) || (grad_biases && grad_biases[l])) lowest = std::min(lowest, l);
+    if (lowest == L && !grad_img)
+        return fail(AADFF_E_INVALID, "no output requested: grad_img, grad_depth, grad_foc and every grad_weights / "
+                                     "grad_biases entry are NULL");
+    const RenderGradLayout rl = render_grad_layout(h, H, W);
+    if (N > 0 && !work) return fail(AADFF_E_INVALID, "work is NULL");
+    if (N > 0 && work_bytes < (int64_t)(rl.floats * sizeof(float)))
+        return fail(AADFF_E_INVALID, "work_bytes is smaller than aadff_render_stack_backward_work_bytes(net, H, W)");
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return fail(AADFF_E_CUDA, "cannot select device");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    auto dW = [&](int l) { return grad_weights ? grad_weights[l] : nullptr; };
+    auto dB = [&](int l) { return grad_biases ? grad_biases[l] : nullptr; };
+    if (N == 0) {                                    // no pixel: the parameter gradients are 0
+        for (int l = 0; l < L; ++l) {
+            if (dW(l)) CUDA_TRY(cudaMemsetAsync(dW(l), 0, (size_t)h->dims[l] * h->dims[l + 1] * sizeof(float), st));
+            if (dB(l)) CUDA_TRY(cudaMemsetAsync(dB(l), 0, (size_t)h->dims[l + 1] * sizeof(float), st));
+        }
+        return AADFF_OK;
+    }
+    const int64_t* os = grad_out_strides;
+    const float d_range = d_max - d_min;
+    const float step_x = (W > 1) ? (1.0f - (-1.0f)) / (float)(W - 1) : 0.f;      // as render_stack_impl
+    const float step_y = (H > 1) ? (-1.0f - 1.0f) / (float)(H - 1) : 0.f;
+    const int r = (h->ks - 1) / 2;
+    float* ws = static_cast<float*>(work);
+    float* probes = ws + rl.probes;
+    float* psf = ws + rl.psf;
+    float* dx = ws + rl.dx;
+    float* mws = ws + rl.mlp;
+    MlpActs acts{};
+    for (int l = 1; l < L; ++l) acts.act[l] = mws + rl.g.act[l];
+    acts.s = mws + rl.g.s;
+    acts.ssum = mws + rl.g.ssum;
+    acts.lds = rl.g.lds;
+    if (grad_img) CUDA_TRY(cudaMemsetAsync(grad_img, 0, (size_t)N * C * H * W * sizeof(float), st));
+    const long long cap = (long long)h->num_sms * 8;
+    int first = 1;                                   // first band of the whole call (dW / db start from 0)
+    for (int n = 0; n < N; ++n)
+        for (int s = 0; s < S; ++s)
+            for (int b0 = 0; b0 < H; b0 += rl.rows) {
+                const int b1 = std::min(H, b0 + rl.rows), valid = (b1 - b0) * W;
+                const int cp = (valid + F32_TP - 1) / F32_TP * F32_TP;
+                if (int rc = launch(rg_probe_kernel, grid_blocks(valid, 256, 1ll << 30), 256, 0, st, depth, foc, n, s, S,
+                                    H, W, b0, valid, d_min, d_range, step_x, step_y, probes))
+                    return rc;
+                if (grad_img) {                      // PSFs in the forward's mode, then the transposed gather
+                    if (int rc = aadff_psfnet_pred_tc_f32(h, probes, psf, valid, mode, st)) return rc;
+                    const long long targets = (long long)(std::min(H, b1 + r) - std::max(0, b0 - r)) * W;
+                    if (int rc = launch(rg_grad_img_band_kernel, grid_blocks(targets, 256, cap), 256, 0, st,
+                                        (const float*)psf, grad_out, (long long)os[0], (long long)os[1], (long long)os[2],
+                                        (long long)os[3], (long long)os[4], grad_img, n, s, C, H, W, h->ks, b0, b1))
+                        return rc;
+                }
+                if (lowest == L) continue;
+                acts.cp = cp;
+                if (int rc = launch(mlp_fp32_store_kernel, grid_blocks(cp, F32_TP, cap), F32_NT, F32_SMEM, st, h->f32,
+                                    (const float*)probes, 0ll, (long long)valid, acts))
+                    return rc;
+                if (int rc = launch(rg_head_kernel, grid_blocks(cp, 8, 1ll << 30), 256, 0, st, (const float*)acts.s,
+                                    rl.g.lds, (const float*)acts.ssum, img, grad_out, (long long)os[0], (long long)os[1],
+                                    (long long)os[2], (long long)os[3], (long long)os[4], n, s, C, H, W, h->ks, b0,
+                                    valid, cp, mws + rl.g.dz[0], (h->kk + 3) / 4 * 4))
+                    return rc;
+                const bool need_dx = grad_depth || grad_foc;
+                if (int rc = mlp_backward_layers(h, rl.g, mws, acts, probes, valid, cp, lowest, first, grad_weights,
+                                                 grad_biases, need_dx ? dx : nullptr, st))
+                    return rc;
+                if (need_dx)
+                    if (int rc = launch(rg_depth_focus_kernel, 1, RG_DF_NT, 0, st, (const float*)dx, depth, foc,
+                                        grad_depth, grad_foc, n, s, S, H, W, b0, valid, d_min, d_range, (int)(b0 == 0),
+                                        (int)(b1 == H)))
+                        return rc;
+                first = 0;
+            }
     return AADFF_OK;
 }
 

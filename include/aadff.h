@@ -115,6 +115,32 @@ int aadff_psfnet_backward_f32(aadff_psfnet_t net, const float* inp, const float*
                               float* const* grad_weights, float* const* grad_biases, void* work, int64_t work_bytes,
                               int64_t M, void* stream);
 
+/* Backward of aadff_render_stack_f32 (what autograd does through the reference's PSFNet.render, times S): given
+ * grad_out = dL/dout in the forward's (n, c, s, h, w) element strides grad_out_strides (HOST array; [N,C,H,W] with
+ * stride 0 for s, BCSHW and BSCHW all work without a copy) -> grad_img [N,C,H,W], grad_depth [N,H,W], grad_foc [N,S]
+ * and the gradient of each weight and bias (grad_weights / grad_biases as for aadff_psfnet_backward_f32).  img, depth,
+ * foc, mode, d_min and d_max are those of the forward.  Any subset of outputs may be NULL (not computed), but at least
+ * one must be requested; a layer without a requested weight gradient costs no dW GEMM, and when only grad_img is
+ * requested no MLP backward runs.  Outputs are overwritten, not accumulated.  The gradient of the (x, y) probe columns
+ * is dropped (the grid is a constant); depth and focus distances get d depth2z / dd = 1 / (d_max - d_min) where
+ * 0 <= (d - d_min) / (d_max - d_min) <= 1 and 0 elsewhere (torch.clamp's rule: invalid and out-of-range depths get 0).
+ * The work runs in bands of floor(16384 / W) whole image rows of one (image, slice), in (n, s, band) order (W > 16384
+ * is refused).  Per band: the probes; for grad_img the PSFs in the forward's `mode` (AADFF_MODE_FP32: the fp32 kernel)
+ * and their transposed gather with the replicate-border folds; for the other outputs the fp32 recompute of
+ * aadff_psfnet_backward_f32, dZ of the head straight from the image taps and grad_out, and the MLP backward down to the
+ * probes.  grad_img never depends on which other outputs are requested.  `work` is 256-byte aligned device memory of
+ * at least aadff_render_stack_backward_work_bytes(net, H, W) bytes, bounded whatever N*S*H*W is; the size query returns a
+ * negative AADFF_E_* code for arguments the backward would refuse.  Arguments are checked before any device call.  No
+ * atomics: every element has one writer per band and a fixed summation order, so two calls give bit-identical results.
+ * Stream-ordered, no allocation, no synchronisation, CUDA-graph capturable (AADFF_MODE_ECON calibrates on its first
+ * use of a handle, synchronously: warm it up before capturing).                                                       */
+int64_t aadff_render_stack_backward_work_bytes(aadff_psfnet_t net, int H, int W);
+int aadff_render_stack_backward_f32(aadff_psfnet_t net, const float* img, const float* depth, const float* foc,
+                                    const float* grad_out, const int64_t grad_out_strides[5], float* grad_img,
+                                    float* grad_depth, float* grad_foc, float* const* grad_weights,
+                                    float* const* grad_biases, int N, int C, int S, int H, int W, float d_min,
+                                    float d_max, int mode, void* work, int64_t work_bytes, void* stream);
+
 /* Replaces local_psf_render (deeplens/render_psf.py:76-107) for a PSF tensor in memory:
  *   img [N,C,H,W], psf [N,H,W,ks,ks] -> out [N,C,H,W]; device pointers.                        */
 int aadff_local_psf_render_f32(const float* img, const float* psf, float* out, int N, int C, int H, int W, int ks,
