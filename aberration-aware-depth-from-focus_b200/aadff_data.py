@@ -81,18 +81,14 @@ def preprocess_rgbd(bgr_u8, depth_u16, size, depth_div=4000.0, depth_mode="antia
         planes = torch.empty(B, P, H, W, device=dev, dtype=torch.float32)
         work = torch.empty(2, B, P, H, W, device=dev, dtype=torch.float32)
         rotated = torch.empty_like(planes)
-        with torch.cuda.device(dev):
-            st = torch.cuda.current_stream().cuda_stream
-            _nat.check(_nat.lib.aadff_prepare_planes_u8(ptr(bgr_u8), ptr(depth_u16), planes.data_ptr(), B, H, W, float(depth_div),
-                                                        ptr(jit), ptr(flp), st))
-            _nat.check(_nat.lib.aadff_spline_affine_f32(planes.data_ptr(), work.data_ptr(), rotated.data_ptr(), B, P, H, W,
-                                                        xf.data_ptr(), P - 1 if depth_u16 is not None else -1, st))
-            _nat.check(_nat.lib.aadff_resize_planes_f32(rotated.data_ptr(), ptr(aif), ptr(depth), B, P, H, W, h, w,
-                                                        {"antialias": 0, "cv2": 1}[depth_mode], st))
+        _nat.call("aadff_prepare_planes_u8", ptr(bgr_u8), ptr(depth_u16), planes.data_ptr(), B, H, W, float(depth_div),
+                  ptr(jit), ptr(flp), device=dev)
+        _nat.call("aadff_spline_affine_f32", planes.data_ptr(), work.data_ptr(), rotated.data_ptr(), B, P, H, W,
+                  xf.data_ptr(), P - 1 if depth_u16 is not None else -1, device=dev)
+        _nat.call("aadff_resize_planes_f32", rotated.data_ptr(), ptr(aif), ptr(depth), B, P, H, W, h, w,
+                  {"antialias": 0, "cv2": 1}[depth_mode], device=dev)
         return aif, depth
     if B:
-        with torch.cuda.device(dev):
-            _nat.check(_nat.lib.aadff_preprocess_rgbd_u8(ptr(bgr_u8), ptr(depth_u16), ptr(aif), ptr(depth), B, H, W, h, w,
-                                                         float(depth_div), {"antialias": 0, "cv2": 1}[depth_mode],
-                                                         ptr(jit), ptr(flp), torch.cuda.current_stream().cuda_stream))
+        _nat.call("aadff_preprocess_rgbd_u8", ptr(bgr_u8), ptr(depth_u16), ptr(aif), ptr(depth), B, H, W, h, w,
+                  float(depth_div), {"antialias": 0, "cv2": 1}[depth_mode], ptr(jit), ptr(flp), device=dev)
     return aif, depth

@@ -18,9 +18,8 @@ def select_focus_dist(depth, num, mode='linear', center=True):
         flat = depth.detach().reshape(B, -1).contiguous()
         out = torch.empty(B, num, device=depth.device, dtype=torch.float32)
         if B:
-            with torch.cuda.device(depth.device):
-                _nat.check(_nat.lib.aadff_select_focus_f32(flat.data_ptr(), B, flat.shape[1], num, out.data_ptr(),
-                                                           torch.cuda.current_stream().cuda_stream))
+            _nat.call("aadff_select_focus_f32", flat.data_ptr(), B, flat.shape[1], num, out.data_ptr(),
+                      device=depth.device)
         return out
     flat = depth.reshape(B, -1)
     valid = flat > 0

@@ -57,9 +57,8 @@ class _PSFNetMLP(torch.autograd.Function):
     def forward(ctx, nat, flat, *params):
         out = torch.empty(flat.shape[0], nat.ks ** 2, device=flat.device, dtype=torch.float32)
         if flat.shape[0]:
-            with torch.cuda.device(flat.device):
-                _nat.check(_nat.lib.aadff_psfnet_pred_f32(nat.handle, flat.data_ptr(), out.data_ptr(), flat.shape[0],
-                                                          torch.cuda.current_stream().cuda_stream))
+            _nat.call("aadff_psfnet_pred_f32", nat.handle, flat.data_ptr(), out.data_ptr(), flat.shape[0],
+                      device=flat.device)
         ctx.nat = nat
         ctx.save_for_backward(flat, *params)
         return out
@@ -72,25 +71,14 @@ class _PSFNetMLP(torch.autograd.Function):
         grads = [torch.empty_like(p) if n else None for p, n in zip(params, need_p)]
         grad_inp = torch.empty_like(flat) if need_inp else None
         M = flat.shape[0]
-        if not (need_inp or any(need_p)):
-            return (None, None) + tuple(grads)
         if M == 0:          # no probe: the parameter gradients are 0 (data_ptr() of an empty tensor is NULL)
             return (None, grad_inp) + tuple(g.zero_() if g is not None else None for g in grads)
         nat = ctx.nat
         g = grad_psf.to(torch.float32).contiguous()
-        c_f32p = _nat.ctypes.POINTER(_nat.ctypes.c_float)
-        ptr = lambda t: _nat.ctypes.cast(_nat.ctypes.c_void_p(t.data_ptr()), c_f32p) if t is not None else None
-        n = nat.n_layers
-        wp = (c_f32p * n)(*[ptr(t) for t in grads[0::2]])
-        bp = (c_f32p * n)(*[ptr(t) for t in grads[1::2]])
-        with torch.cuda.device(flat.device):
-            work_bytes = _nat.lib.aadff_psfnet_backward_work_bytes(nat.handle, M)
-            if work_bytes < 0:
-                _nat.check(int(work_bytes))
-            work = torch.empty(work_bytes, dtype=torch.uint8, device=flat.device)
-            _nat.check(_nat.lib.aadff_psfnet_backward_f32(
-                nat.handle, flat.data_ptr(), g.data_ptr(), grad_inp.data_ptr() if need_inp else None, wp, bp,
-                work.data_ptr(), work_bytes, M, torch.cuda.current_stream().cuda_stream))
+        work = _nat.workspace(_nat.lib.aadff_psfnet_backward_work_bytes(nat.handle, M), flat.device)
+        _nat.call("aadff_psfnet_backward_f32", nat.handle, flat.data_ptr(), g.data_ptr(),
+                  grad_inp.data_ptr() if need_inp else None, _nat.f32_ptrs(grads[0::2]), _nat.f32_ptrs(grads[1::2]),
+                  work.data_ptr(), work.numel(), M, device=flat.device)
         return (None, grad_inp) + tuple(grads)
 
 
@@ -100,47 +88,63 @@ def _launch_stack(nat, img, depth, foc, out_ptr, strides, m, d_min, d_max, rows=
     S = foc.shape[1]
     if N * C * S * H * W == 0:      # empty batch: nothing to launch (data_ptr() of an empty tensor is NULL)
         return
-    arr = (_nat.ctypes.c_int64 * 5)(*strides)
-    with torch.cuda.device(img.device):
-        st = torch.cuda.current_stream().cuda_stream
-        if rows is None:
-            _nat.check(_nat.lib.aadff_render_stack_f32(
-                nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, arr,
-                N, C, S, H, W, d_min, d_max, m, st))
-        else:
-            _nat.check(_nat.lib.aadff_render_stack_rows_f32(
-                nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, arr,
-                N, C, S, H, W, d_min, d_max, m, int(rows[0]), int(rows[1]), st))
+    args = (nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), out_ptr, (_nat.ctypes.c_int64 * 5)(*strides),
+            N, C, S, H, W, d_min, d_max, m)
+    if rows is None:
+        _nat.call("aadff_render_stack_f32", *args, device=img.device)
+    else:
+        _nat.call("aadff_render_stack_rows_f32", *args, int(rows[0]), int(rows[1]), device=img.device)
 
 
-# element strides (n, c, s, h, w) of each output layout of render / render_stack
+def _render_inputs(nat, img, depth, foc, S=-1):
+    """img [N,C,H,W], depth [N,H,W] and foc [N,S] as fp32 contiguous tensors on the device of the handle `nat`.  These
+    are ordinary torch ops, so on the differentiable path the gradients return in each input's own shape, dtype and
+    device.  foc is [N] or [N,S], or [S] for one image; S = -1 takes the slice count from foc."""
+    dev = torch.device(f"cuda:{nat.device_index}")
+    img = img.to(dev, torch.float32).contiguous()
+    N, C, H, W = img.shape
+    depth = depth.to(dev, torch.float32).reshape(N, H, W).contiguous()
+    foc = torch.as_tensor(foc).to(dev, torch.float32)
+    # an empty batch keeps its slice count
+    foc = (foc.reshape(N, S) if N else foc.reshape(0, foc.shape[-1] if foc.dim() > 1 else 1)).contiguous()
+    return img, depth, foc
+
+
+def _fp32_params(layers, dev):
+    """(w0, b0, w1, b1, ...) of the nn.Linear modules `layers` as fp32 contiguous tensors on `dev` (differentiable)."""
+    return [t.to(dev, torch.float32).contiguous() for l in layers for t in (l.weight, l.bias)]
+
+
+# element strides (n, c, s, h, w) of each output layout: render's "NCHW" (S = 1), render_stack's "BCSHW" and "BSCHW"
 def _layout_strides(layout, N, C, S, H, W):
     if layout == "NCHW":
         return (N, C, H, W), (C * H * W, H * W, 0, W, 1)
     if layout == "BCSHW":
         return (N, C, S, H, W), (C * S * H * W, S * H * W, H * W, W, 1)
-    if layout == "BSCHW":
-        return (N, S, C, H, W), (S * C * H * W, H * W, C * H * W, W, 1)
-    raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
+    return (N, S, C, H, W), (S * C * H * W, H * W, C * H * W, W, 1)
+
+
+def _render_stack(nat, m, layout, d_min, d_max, img, depth, foc):
+    """The output of render / render_stack in `layout` from one aadff_render_stack_f32 launch; inputs as
+    _render_inputs returns them."""
+    N, C, H, W = img.shape
+    shape, strides = _layout_strides(layout, N, C, foc.shape[1], H, W)
+    out = torch.empty(shape, device=img.device, dtype=torch.float32)
+    _launch_stack(nat, img, depth, foc, out.data_ptr(), strides, m, d_min, d_max)
+    return out
 
 
 class _RenderStack(torch.autograd.Function):
-    """out = render_stack(img, depth, foc) with the network (w0, b0, w1, b1, ...) of the handle `nat`: fp32 contiguous
-    img [N,C,H,W], depth [N,H,W], foc [N,S] on the handle's device, `layout` one of _layout_strides'.  The forward is
-    the launch of the no-grad path, so the output is bit-identical to it; the backward
-    (aadff_render_stack_backward_f32) recomputes the PSFs and activations band by band and reads the weights of the
-    same handle, which the graph keeps alive.  The saved inputs make autograd refuse a backward after an in-place change
-    to them."""
+    """out = _render_stack(nat, m, layout, d_min, d_max, img, depth, foc) with the network (w0, b0, w1, b1, ...) of the
+    handle `nat`, so the output is bit-identical to the no-grad path's; the backward (aadff_render_stack_backward_f32)
+    recomputes the PSFs and activations band by band and reads the weights of the same handle, which the graph keeps
+    alive.  The saved inputs make autograd refuse a backward after an in-place change to them."""
 
     @staticmethod
     def forward(ctx, nat, m, layout, d_min, d_max, img, depth, foc, *params):
-        N, C, H, W = img.shape
-        shape, strides = _layout_strides(layout, N, C, foc.shape[1], H, W)
-        out = torch.empty(shape, device=img.device, dtype=torch.float32)
-        _launch_stack(nat, img, depth, foc, out.data_ptr(), strides, m, d_min, d_max)
         ctx.nat, ctx.m, ctx.layout, ctx.d_min, ctx.d_max = nat, m, layout, d_min, d_max
         ctx.save_for_backward(img, depth, foc, *params)
-        return out
+        return _render_stack(nat, m, layout, d_min, d_max, img, depth, foc)
 
     @staticmethod
     @once_differentiable
@@ -155,29 +159,17 @@ class _RenderStack(torch.autograd.Function):
         head = (None,) * 5
         N, C, H, W = img.shape
         S = foc.shape[1]
-        if not (need_img or need_depth or need_foc or any(need_p)):
-            return head + (None, None, None) + tuple(grads)
         if N * C * S * H * W == 0:      # no pixel: the parameter gradients are 0, the other gradients are empty
             return head + (grad_img, grad_depth, grad_foc) + tuple(g.zero_() if g is not None else None for g in grads)
         nat = ctx.nat
         g = grad_out.to(torch.float32).contiguous()
         _, strides = _layout_strides(ctx.layout, N, C, S, H, W)
-        arr = (_nat.ctypes.c_int64 * 5)(*strides)
-        c_f32p = _nat.ctypes.POINTER(_nat.ctypes.c_float)
-        ptr = lambda t: _nat.ctypes.cast(_nat.ctypes.c_void_p(t.data_ptr()), c_f32p) if t is not None else None
-        n = nat.n_layers
-        wp = (c_f32p * n)(*[ptr(t) for t in grads[0::2]])
-        bp = (c_f32p * n)(*[ptr(t) for t in grads[1::2]])
         dp = lambda t: t.data_ptr() if t is not None else None
-        with torch.cuda.device(img.device):
-            work_bytes = _nat.lib.aadff_render_stack_backward_work_bytes(nat.handle, H, W)
-            if work_bytes < 0:
-                _nat.check(int(work_bytes))
-            work = torch.empty(work_bytes, dtype=torch.uint8, device=img.device)
-            _nat.check(_nat.lib.aadff_render_stack_backward_f32(
-                nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(), g.data_ptr(), arr, dp(grad_img),
-                dp(grad_depth), dp(grad_foc), wp, bp, N, C, S, H, W, ctx.d_min, ctx.d_max, ctx.m, work.data_ptr(),
-                work_bytes, torch.cuda.current_stream().cuda_stream))
+        work = _nat.workspace(_nat.lib.aadff_render_stack_backward_work_bytes(nat.handle, H, W), img.device)
+        _nat.call("aadff_render_stack_backward_f32", nat.handle, img.data_ptr(), depth.data_ptr(), foc.data_ptr(),
+                  g.data_ptr(), (_nat.ctypes.c_int64 * 5)(*strides), dp(grad_img), dp(grad_depth), dp(grad_foc),
+                  _nat.f32_ptrs(grads[0::2]), _nat.f32_ptrs(grads[1::2]), N, C, S, H, W, ctx.d_min, ctx.d_max, ctx.m,
+                  work.data_ptr(), work.numel(), device=img.device)
         return head + (grad_img, grad_depth, grad_foc) + tuple(grads)
 
 
@@ -251,20 +243,15 @@ class PSFNet(nn.Module):
         MLP.forward when autograd needs it) the result is differentiable in inp and in their parameters."""
         nat = PSFNet.native(self)
         kk = self.kernel_size ** 2
+        dev = torch.device(f"cuda:{nat.device_index}")
         if layers is not None:
-            dev = torch.device(f"cuda:{nat.device_index}")
             flat = inp.reshape(-1, 4).to(dev, torch.float32).contiguous()
-            params = []
-            for l in layers:
-                params += [l.weight.to(dev, torch.float32).contiguous(), l.bias.to(dev, torch.float32).contiguous()]
-            return _PSFNetMLP.apply(nat, flat, *params).reshape(*inp.shape[:-1], kk)
-        flat = inp.detach().reshape(-1, 4).to(f"cuda:{nat.device_index}", torch.float32).contiguous()
-        out = torch.empty(flat.shape[0], kk, device=flat.device, dtype=torch.float32)
-        if flat.shape[0] == 0:
-            return out.reshape(*inp.shape[:-1], kk)
-        with torch.cuda.device(flat.device):
-            _nat.check(_nat.lib.aadff_psfnet_pred_tc_f32(nat.handle, flat.data_ptr(), out.data_ptr(), flat.shape[0],
-                                                         _nat.MODES[mode], torch.cuda.current_stream().cuda_stream))
+            return _PSFNetMLP.apply(nat, flat, *_fp32_params(layers, dev)).reshape(*inp.shape[:-1], kk)
+        flat = inp.detach().reshape(-1, 4).to(dev, torch.float32).contiguous()
+        out = torch.empty(flat.shape[0], kk, device=dev, dtype=torch.float32)
+        if flat.shape[0]:
+            _nat.call("aadff_psfnet_pred_tc_f32", nat.handle, flat.data_ptr(), out.data_ptr(), flat.shape[0],
+                      _nat.MODES[mode], device=dev)
         return out.reshape(*inp.shape[:-1], kk)
 
     @torch.no_grad()
@@ -274,37 +261,19 @@ class PSFNet(nn.Module):
         psf = PSFNet._mlp_eval(self, inp, "fp32" if mode is None else mode)
         return psf.reshape(*psf.shape[:-1], self.kernel_size, self.kernel_size)
 
-    def _launch(self, img, depth, foc, out_ptr, strides, mode, rows=None):
-        _launch_stack(PSFNet.native(self), img, depth, foc, out_ptr, strides, PSFNet._mode(self, mode),
-                      float(self.d_min), float(self.d_max), rows)
-
     def _mode(self, mode):
         return _nat.MODES[mode or getattr(self, "mode", None) or os.environ.get("AADFF_MODE", "parity")]
 
-    def _prep(self, img, depth):
+    def _render(self, img, depth, foc, layout, mode, differentiable):
+        """render / render_stack into `layout`: differentiable when _wants_grad says so, with the same output."""
         nat = PSFNet.native(self)
-        dev = torch.device(f"cuda:{nat.device_index}")
-        img = img.detach().to(dev, torch.float32).contiguous()
-        N, C, H, W = img.shape
-        depth = depth.detach().to(dev, torch.float32).reshape(N, H, W).contiguous()
-        return img, depth, dev
-
-    def _render_grad(self, img, depth, foc, layout, mode):
-        """The differentiable render: conversions to fp32 contiguous tensors on the handle's device as ordinary torch
-        ops (gradients return in each input's own shape, dtype and device), then _RenderStack.  foc is [N] or [N,S]."""
-        nat = PSFNet.native(self)
-        dev = torch.device(f"cuda:{nat.device_index}")
-        img = img.to(dev, torch.float32).contiguous()
-        N, C, H, W = img.shape
-        depth = depth.to(dev, torch.float32).reshape(N, H, W).contiguous()
-        foc = torch.as_tensor(foc).to(dev, torch.float32)
-        # as the no-grad paths: [N], [N,S] or [S] for one image; an empty batch keeps its slice count
-        foc = (foc.reshape(N, -1) if N else foc.reshape(0, foc.shape[-1] if foc.dim() > 1 else 1)).contiguous()
-        params = []
-        for l in _linear_layers(self.psfnet):
-            params += [l.weight.to(dev, torch.float32).contiguous(), l.bias.to(dev, torch.float32).contiguous()]
-        return _RenderStack.apply(nat, PSFNet._mode(self, mode), layout, float(self.d_min), float(self.d_max),
-                                  img, depth, foc, *params)
+        args = (nat, PSFNet._mode(self, mode), layout, float(self.d_min), float(self.d_max))
+        S = 1 if layout == "NCHW" else -1
+        if PSFNet._wants_grad(self, differentiable, img, depth, foc):
+            img, depth, foc = _render_inputs(nat, img, depth, foc, S)
+            return _RenderStack.apply(*args, img, depth, foc, *_fp32_params(_linear_layers(self.psfnet), img.device))
+        with torch.no_grad():       # the default path calls the launch directly: no autograd node, no extra host cost
+            return _render_stack(*args, *_render_inputs(nat, img, depth, foc, S))
 
     def _wants_grad(self, differentiable, *inputs):
         """differentiable=True, grad mode on, and an input or a parameter of the network requiring grad."""
@@ -328,15 +297,7 @@ class PSFNet(nn.Module):
                 foc_dist = torch.as_tensor([float(foc_dist)], dtype=torch.float32)
         elif img.dim() != 4:
             raise ValueError(f"render expects a [N,C,H,W] or [C,H,W] image, got shape {tuple(img.shape)}")
-        if PSFNet._wants_grad(self, differentiable, img, depth, foc_dist):
-            return PSFNet._render_grad(self, img, depth, foc_dist, "NCHW", mode)
-        with torch.no_grad():
-            img, depth, dev = PSFNet._prep(self, img, depth)
-            N, C, H, W = img.shape
-            foc = torch.as_tensor(foc_dist).detach().to(dev, torch.float32).reshape(N, 1).contiguous()
-            out = torch.empty_like(img)
-            PSFNet._launch(self, img, depth, foc, out.data_ptr(), (C * H * W, H * W, 0, W, 1), mode)
-            return out
+        return PSFNet._render(self, img, depth, foc_dist, "NCHW", mode, differentiable)
 
     def render_stack(self, img, depth, foc_dists, layout="BCSHW", mode=None, differentiable=False):
         """All S focal slices in one launch: foc_dists [N,S] (mm, negative) -> [N,C,S,H,W]
@@ -344,44 +305,28 @@ class PSFNet(nn.Module):
         differentiable=True: as for ``render``."""
         if img.dim() != 4:
             raise ValueError("render_stack expects a [N,C,H,W] image")
-        if PSFNet._wants_grad(self, differentiable, img, depth, foc_dists):
-            if layout not in ("BCSHW", "BSCHW"):
-                raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
-            return PSFNet._render_grad(self, img, depth, foc_dists, layout, mode)
-        with torch.no_grad():
-            img, depth, dev = PSFNet._prep(self, img, depth)
-            N, C, H, W = img.shape
-            foc = foc_dists.detach().to(dev, torch.float32).reshape(N, -1).contiguous()
-            S = foc.shape[1]
-            if layout == "BCSHW":
-                out = torch.empty(N, C, S, H, W, device=dev, dtype=torch.float32)
-                strides = (C * S * H * W, S * H * W, H * W, W, 1)
-            elif layout == "BSCHW":
-                out = torch.empty(N, S, C, H, W, device=dev, dtype=torch.float32)
-                strides = (S * C * H * W, H * W, C * H * W, W, 1)
-            else:
-                raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
-            PSFNet._launch(self, img, depth, foc, out.data_ptr(), strides, mode)
-            return out
+        if layout not in ("BCSHW", "BSCHW"):
+            raise ValueError("layout must be 'BCSHW' or 'BSCHW'")
+        return PSFNet._render(self, img, depth, foc_dists, layout, mode, differentiable)
 
     @torch.no_grad()
     def render_stack_rows(self, img, depth, foc_dists, tile_row_begin, tile_row_end, mode=None):
         """One contiguous run of tile rows (8 image rows each) of the flattened (image, slice, row) stack -- the
         unit of the multi-GPU partition (sharding.py).  Returns the rows in [flat_rows, C, W] layout, where
         flat row = (n*S + s)*H + h; bit-identical to the same rows of ``render_stack``."""
-        img, depth, dev = PSFNet._prep(self, img, depth)
+        nat = PSFNet.native(self)
+        img, depth, foc = _render_inputs(nat, img, depth, foc_dists)
         N, C, H, W = img.shape
-        foc = foc_dists.detach().to(dev, torch.float32).reshape(N, -1).contiguous()
         S = foc.shape[1]
         th = _nat.lib.aadff_tile_row_height()
         ty = -(-H // th)
         fr = [(R // ty) * H + min((R % ty) * th, H) for R in (int(tile_row_begin), int(tile_row_end))]
-        out = torch.empty(fr[1] - fr[0], C, W, device=dev, dtype=torch.float32)
+        out = torch.empty(fr[1] - fr[0], C, W, device=img.device, dtype=torch.float32)
         # element strides of a virtual [N,S,H,C,W] tensor whose flat row fr[0] sits at out[0]
         strides = (S * H * C * W, W, H * C * W, C * W, 1)
         if out.numel():
-            PSFNet._launch(self, img, depth, foc, out.data_ptr() - fr[0] * C * W * 4, strides, mode,
-                           rows=(tile_row_begin, tile_row_end))
+            _launch_stack(nat, img, depth, foc, out.data_ptr() - fr[0] * C * W * 4, strides, PSFNet._mode(self, mode),
+                          float(self.d_min), float(self.d_max), rows=(tile_row_begin, tile_row_end))
         return out
 
     @torch.no_grad()
@@ -434,8 +379,8 @@ class PSFNet(nn.Module):
                         raise ValueError(f"train_psfnet: data returned PSFs of {psf.shape[-1]} taps per probe; "
                                          f"kernel_size {self.kernel_size} needs {self.kernel_size ** 2}")
                     lr_i = 0.5 * lr * (1.0 + math.cos(math.pi * i / iters)) if iters > 0 else lr   # CosineAnnealingLR, eta_min 0
-                    _nat.check(_nat.lib.aadff_trainer_step(trainer.handle, inp.data_ptr(), psf.data_ptr(), lr_i,
-                                                           loss_dev.data_ptr(), torch.cuda.current_stream().cuda_stream))
+                    _nat.call("aadff_trainer_step", trainer.handle, inp.data_ptr(), psf.data_ptr(), lr_i,
+                              loss_dev.data_ptr(), device=dev)
                     if (i + 1) % evaluate_every == 0:
                         history.append((i + 1, float(loss_dev)))
                 ws, bs_ = trainer.read(0, torch.cuda.current_stream().cuda_stream)
@@ -461,8 +406,7 @@ class PSFNet(nn.Module):
 
 
 # names install() grafts onto the reference's PSFNet (everything render/pred need, nothing the ray tracer owns)
-PSFNET_GRAFT = ("native", "refresh", "_mlp_eval", "pred", "_launch", "_mode", "_prep", "_render_grad", "_wants_grad",
-                "render", "render_stack",
+PSFNET_GRAFT = ("native", "refresh", "_mlp_eval", "pred", "_mode", "_render", "_wants_grad", "render", "render_stack",
                 "render_stack_rows", "simulate_focal_stack", "train_psfnet")
 
 
@@ -512,13 +456,10 @@ class ThinLens(nn.Module):
         if out.numel() == 0:
             return out
         flag = torch.empty(1, dtype=torch.uint8, device=img.device)
-        with torch.cuda.device(img.device):
-            st = torch.cuda.current_stream().cuda_stream
-            _nat.check(_nat.lib.aadff_any_negative_f32(dep.data_ptr(), dep.numel(), flag.data_ptr(), st))
-            _nat.check(_nat.lib.aadff_thinlens_render_f32(
-                img.data_ptr(), dep.data_ptr(), foc.data_ptr(), out.data_ptr(), N, C, H, W, int(self.kernel_size),
-                float(self.foc_len), float(self.fnum), float(self.ps), float(self.d_min), float(self.d_max), 0,
-                flag.data_ptr(), st))
+        _nat.call("aadff_any_negative_f32", dep.data_ptr(), dep.numel(), flag.data_ptr(), device=img.device)
+        _nat.call("aadff_thinlens_render_f32", img.data_ptr(), dep.data_ptr(), foc.data_ptr(), out.data_ptr(),
+                  N, C, H, W, int(self.kernel_size), float(self.foc_len), float(self.fnum), float(self.ps),
+                  float(self.d_min), float(self.d_max), 0, flag.data_ptr(), device=img.device)
         return out
 
     @torch.no_grad()

@@ -8,8 +8,11 @@ from __future__ import annotations
 
 import ctypes
 import os
+import re
 import shutil
 import subprocess
+
+import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _REPO = os.path.dirname(_HERE)
@@ -48,97 +51,47 @@ def build(force: bool = False, verbose: bool = False) -> str:
     return LIB_PATH
 
 
-def _header_symbols():
-    import re
-    with open(HEADER) as f:
-        return sorted(set(re.findall(r"\b(aadff_[a-z0-9_]+)\s*\(", f.read())))
+# C types of include/aadff.h's scalar parameters and return values.  Every pointer or array parameter is c_void_p, which
+# takes data_ptr() ints, None, ctypes arrays and byref(); a type outside this map fails the import instead of falling
+# back to ctypes' default (a 32-bit int).
+_CTYPES = {"int": ctypes.c_int, "int64_t": ctypes.c_int64, "float": ctypes.c_float, "double": ctypes.c_double,
+           "const char*": ctypes.c_char_p, "aadff_psfnet_t": ctypes.c_void_p, "aadff_trainer_t": ctypes.c_void_p}
+
+
+def _ctype(decl):
+    t = " ".join(decl.replace("*", " * ").split()).replace(" *", "*")
+    if t not in _CTYPES:
+        raise TypeError(f"include/aadff.h: no ctypes mapping for C type '{t}'")
+    return _CTYPES[t]
+
+
+def _prototypes(text=None):
+    """{name: (restype, argtypes)} of each prototype `ret aadff_name(params);` in include/aadff.h (or in `text`)."""
+    if text is None:
+        with open(HEADER) as f:
+            text = f.read()
+    text = re.sub(r"^\s*#.*$", "", re.sub(r"/\*.*?\*/", " ", text, flags=re.S), flags=re.M)
+    protos = {}
+    for ret, name, params in re.findall(r"(\w[\w\s*]*?)\s*\b(aadff_\w+)\s*\(([^()]*)\)\s*;", text):
+        params = [p for p in params.split(",") if p.strip() not in ("", "void")]
+        protos[name] = (_ctype(ret), [ctypes.c_void_p if "*" in p or "[" in p else _ctype(p.rsplit(None, 1)[0])
+                                      for p in params])
+    return protos
 
 
 def _load() -> ctypes.CDLL:
     if not os.path.exists(LIB_PATH):
         build()
     lib = ctypes.CDLL(LIB_PATH)
-    if any(not hasattr(lib, name) for name in _header_symbols()):     # stale binary: rebuild once
+    protos = _prototypes()
+    if any(not hasattr(lib, name) for name in protos):     # stale binary: rebuild once
         import _ctypes
         _ctypes.dlclose(lib._handle)
         build(force=True)
         lib = ctypes.CDLL(LIB_PATH)
-    c_f32p = ctypes.POINTER(ctypes.c_float)
-    lib.aadff_version.restype = ctypes.c_int
-    lib.aadff_last_error.restype = ctypes.c_char_p
-    lib.aadff_launch_count.restype = ctypes.c_int64
-    lib.aadff_psfnet_create.argtypes = [ctypes.POINTER(c_f32p), ctypes.POINTER(c_f32p),
-                                        ctypes.POINTER(ctypes.c_int), ctypes.c_int, ctypes.c_int, ctypes.c_int,
-                                        ctypes.POINTER(ctypes.c_void_p)]
-    lib.aadff_psfnet_destroy.argtypes = [ctypes.c_void_p]
-    lib.aadff_render_stack_f32.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
-                                           ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)] + [ctypes.c_int] * 5 + \
-                                          [ctypes.c_float, ctypes.c_float, ctypes.c_int, ctypes.c_void_p]
-    lib.aadff_render_stack_rows_f32.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
-                                                ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)] + [ctypes.c_int] * 5 + \
-                                               [ctypes.c_float, ctypes.c_float, ctypes.c_int, ctypes.c_int64,
-                                                ctypes.c_int64, ctypes.c_void_p]
-    lib.aadff_tile_row_height.restype = ctypes.c_int
-    lib.aadff_econ_first_group.restype = ctypes.c_int
-    lib.aadff_render_psf_map_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 6 + \
-                                            [ctypes.POINTER(ctypes.c_int)] * 2 + [ctypes.c_void_p]
-    lib.aadff_trainer_create.argtypes = [ctypes.POINTER(c_f32p), ctypes.POINTER(c_f32p), ctypes.POINTER(ctypes.c_int),
-                                         ctypes.c_int, ctypes.c_int] + [ctypes.c_float] * 4 + \
-                                        [ctypes.c_int, ctypes.POINTER(ctypes.c_void_p)]
-    lib.aadff_trainer_step.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p,
-                                       ctypes.c_void_p]
-    lib.aadff_trainer_read.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(c_f32p), ctypes.POINTER(c_f32p),
-                                       ctypes.c_void_p]
-    lib.aadff_trainer_destroy.argtypes = [ctypes.c_void_p]
-    lib.aadff_preprocess_rgbd_u8.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_int] * 5 + [ctypes.c_float, ctypes.c_int,
-                                             ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
-    lib.aadff_prepare_planes_u8.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 3 + [ctypes.c_float, ctypes.c_void_p,
-                                            ctypes.c_void_p, ctypes.c_void_p]
-    lib.aadff_spline_affine_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 4 + [ctypes.c_void_p, ctypes.c_int,
-                                            ctypes.c_void_p]
-    lib.aadff_resize_planes_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 6 + [ctypes.c_int, ctypes.c_void_p]
-    lib.aadff_any_negative_f32.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p]
-    lib.aadff_render_stack_host_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int] * 5 + \
-                                               [ctypes.c_float, ctypes.c_float, ctypes.c_int]
-    lib.aadff_psfnet_pred_f32.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
-                                          ctypes.c_void_p]
-    lib.aadff_psfnet_pred_tc_f32.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
-                                             ctypes.c_int, ctypes.c_void_p]
-    lib.aadff_psfnet_backward_work_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int64]
-    lib.aadff_psfnet_backward_work_bytes.restype = ctypes.c_int64
-    lib.aadff_psfnet_backward_f32.argtypes = [ctypes.c_void_p] * 4 + [ctypes.POINTER(c_f32p)] * 2 + \
-                                             [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p]
-    lib.aadff_psfnet_backward_f32.restype = ctypes.c_int
-    lib.aadff_render_stack_backward_work_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int]
-    lib.aadff_render_stack_backward_work_bytes.restype = ctypes.c_int64
-    lib.aadff_render_stack_backward_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.POINTER(ctypes.c_int64)] + \
-                                                   [ctypes.c_void_p] * 3 + [ctypes.POINTER(c_f32p)] * 2 + \
-                                                   [ctypes.c_int] * 5 + [ctypes.c_float, ctypes.c_float, ctypes.c_int,
-                                                                         ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
-    lib.aadff_render_stack_backward_f32.restype = ctypes.c_int
-    lib.aadff_local_psf_render_f32.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
-    lib.aadff_local_psf_render_backward_f32.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int] * 5 + [ctypes.c_void_p]
-    lib.aadff_render_psf_map_backward_work_bytes.argtypes = [ctypes.c_int] * 6 + [ctypes.POINTER(ctypes.c_int)] * 2
-    lib.aadff_render_psf_map_backward_work_bytes.restype = ctypes.c_int64
-    lib.aadff_render_psf_map_backward_f32.argtypes = [ctypes.c_void_p] * 6 + [ctypes.c_int64] + [ctypes.c_int] * 6 + \
-                                                     [ctypes.POINTER(ctypes.c_int)] * 2 + [ctypes.c_void_p]
-    lib.aadff_debug_umma_gemm.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 3
-    lib.aadff_thinlens_render_f32.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_int] * 5 + [ctypes.c_float] * 5 + \
-                                             [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
-    lib.aadff_debug_set_desc_swap.argtypes = [ctypes.c_int]
-    lib.aadff_debug_econ_round.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_int,
-                                           ctypes.c_void_p]
-    lib.aadff_debug_econ_round.restype = ctypes.c_int
-    lib.aadff_select_focus_f32.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_int, ctypes.c_void_p,
-                                           ctypes.c_void_p]
-    for fn in ("aadff_psfnet_create", "aadff_psfnet_destroy", "aadff_render_stack_f32", "aadff_render_stack_rows_f32",
-               "aadff_any_negative_f32", "aadff_render_psf_map_f32", "aadff_preprocess_rgbd_u8", "aadff_prepare_planes_u8",
-               "aadff_spline_affine_f32", "aadff_resize_planes_f32", "aadff_trainer_create", "aadff_trainer_step",
-               "aadff_trainer_read", "aadff_trainer_destroy",
-               "aadff_render_stack_host_f32", "aadff_psfnet_pred_f32", "aadff_psfnet_pred_tc_f32", "aadff_local_psf_render_f32",
-               "aadff_local_psf_render_backward_f32", "aadff_render_psf_map_backward_f32", "aadff_thinlens_render_f32", "aadff_select_focus_f32",
-               "aadff_debug_umma_gemm", "aadff_debug_set_desc_swap"):
-        getattr(lib, fn).restype = ctypes.c_int
+    for name, (restype, argtypes) in protos.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     return lib
 
 
@@ -161,7 +114,30 @@ def econ_first_group() -> int:
 
 def exported_symbols():
     """Names declared in include/aadff.h (used by the CPU test that checks the library exports them)."""
-    return _header_symbols()
+    return sorted(_prototypes())
+
+
+def call(fn_name: str, *args, device: torch.device) -> None:
+    """lib.<fn_name>(*args, stream) on `device` with its current stream; raises AadffError on a non-zero return."""
+    # by index: resolving the torch.device in both torch calls would cost more host time than the rest of this helper
+    idx = device.index
+    with torch.cuda.device(idx):
+        check(getattr(lib, fn_name)(*args, torch.cuda.current_stream(idx).cuda_stream))
+
+
+def workspace(nbytes: int, device) -> torch.Tensor:
+    """The device workspace an aadff_*_work_bytes query asked for; a negative size is the query's refusal and raises.
+    The caching allocator hands out blocks aligned to at least 256 bytes, as the render backward requires."""
+    if nbytes < 0:
+        check(nbytes)
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)
+
+
+def f32_ptrs(seq):
+    """Host array of float* for the C ABI's per-layer pointer arrays: one per tensor or numpy array, NULL for None.
+    The caller keeps the arrays alive for the duration of the call."""
+    return (ctypes.c_void_p * len(seq))(*[None if t is None else t.data_ptr() if torch.is_tensor(t) else t.ctypes.data
+                                          for t in seq])
 
 
 class NativePSFNet:
@@ -169,20 +145,16 @@ class NativePSFNet:
 
     def __init__(self, weights, biases, ks: int, device_index: int):
         import numpy as np
-        self._np = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
-        self._nb = [np.ascontiguousarray(b, dtype=np.float32) for b in biases]
-        n = len(self._np)
-        dims = [self._np[0].shape[1]] + [w.shape[0] for w in self._np]
-        c_f32p = ctypes.POINTER(ctypes.c_float)
-        wp = (c_f32p * n)(*[w.ctypes.data_as(c_f32p) for w in self._np])
-        bp = (c_f32p * n)(*[b.ctypes.data_as(c_f32p) for b in self._nb])
-        dm = (ctypes.c_int * (n + 1))(*dims)
+        ws = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
+        bs = [np.ascontiguousarray(b, dtype=np.float32) for b in biases]
+        n = len(ws)
+        dims = [ws[0].shape[1]] + [w.shape[0] for w in ws]
         self.handle = ctypes.c_void_p()
         self.ks = ks
         self.n_layers = n
         self.device_index = device_index
-        check(lib.aadff_psfnet_create(wp, bp, dm, n, ks, device_index, ctypes.byref(self.handle)))
-        self._np = self._nb = None
+        check(lib.aadff_psfnet_create(f32_ptrs(ws), f32_ptrs(bs), (ctypes.c_int * (n + 1))(*dims), n, ks, device_index,
+                                      ctypes.byref(self.handle)))
 
     def close(self):
         if getattr(self, "handle", None):
@@ -202,25 +174,21 @@ class NativeTrainer:
     def __init__(self, weights, biases, batch: int, device_index: int, betas=(0.9, 0.999), eps=1e-8,
                  weight_decay=1e-2):
         import numpy as np
-        self._np = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
-        self._nb = [np.ascontiguousarray(b, dtype=np.float32) for b in biases]
-        n = len(self._np)
-        if n < 1 or len(self._nb) != n:
-            raise ValueError(f"NativeTrainer: need as many biases as weights (>= 1), got {n} and {len(self._nb)}")
-        self.dims = [self._np[0].shape[-1]] + [w.shape[0] for w in self._np]
-        for l, (w, b) in enumerate(zip(self._np, self._nb)):
+        ws = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
+        bs = [np.ascontiguousarray(b, dtype=np.float32) for b in biases]
+        n = len(ws)
+        if n < 1 or len(bs) != n:
+            raise ValueError(f"NativeTrainer: need as many biases as weights (>= 1), got {n} and {len(bs)}")
+        self.dims = [ws[0].shape[-1]] + [w.shape[0] for w in ws]
+        for l, (w, b) in enumerate(zip(ws, bs)):
             # the library copies dims[l+1] * dims[l] weights and dims[l+1] biases of each layer from these buffers
             if w.shape != (self.dims[l + 1], self.dims[l]) or b.shape != (self.dims[l + 1],):
                 raise ValueError(f"NativeTrainer: layer {l} has weight {tuple(w.shape)} and bias {tuple(b.shape)}; "
                                  f"expected ({self.dims[l + 1]}, {self.dims[l]}) and ({self.dims[l + 1]},)")
         self.batch, self.device_index = int(batch), device_index
-        c_f32p = ctypes.POINTER(ctypes.c_float)
-        wp = (c_f32p * n)(*[w.ctypes.data_as(c_f32p) for w in self._np])
-        bp = (c_f32p * n)(*[b.ctypes.data_as(c_f32p) for b in self._nb])
-        dm = (ctypes.c_int * (n + 1))(*self.dims)
         self.handle = ctypes.c_void_p()
-        check(lib.aadff_trainer_create(wp, bp, dm, n, self.batch, betas[0], betas[1], eps, weight_decay, device_index,
-                                       ctypes.byref(self.handle)))
+        check(lib.aadff_trainer_create(f32_ptrs(ws), f32_ptrs(bs), (ctypes.c_int * (n + 1))(*self.dims), n, self.batch,
+                                       betas[0], betas[1], eps, weight_decay, device_index, ctypes.byref(self.handle)))
 
     def read(self, which: int, stream=None):
         """which 0: parameters, 1: gradients of the last step -> (weights, biases) as numpy arrays."""
@@ -228,10 +196,7 @@ class NativeTrainer:
         n = len(self.dims) - 1
         ws = [np.empty((self.dims[l + 1], self.dims[l]), np.float32) for l in range(n)]
         bs = [np.empty((self.dims[l + 1],), np.float32) for l in range(n)]
-        c_f32p = ctypes.POINTER(ctypes.c_float)
-        wp = (c_f32p * n)(*[w.ctypes.data_as(c_f32p) for w in ws])
-        bp = (c_f32p * n)(*[b.ctypes.data_as(c_f32p) for b in bs])
-        check(lib.aadff_trainer_read(self.handle, which, wp, bp, stream))
+        check(lib.aadff_trainer_read(self.handle, which, f32_ptrs(ws), f32_ptrs(bs), stream))
         return ws, bs
 
     def close(self):

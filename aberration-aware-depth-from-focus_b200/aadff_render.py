@@ -8,8 +8,8 @@ import aadff_native as _nat
 __all__ = ["local_psf_render", "render_psf", "render_psf_map", "local_psf_render_high_res"]
 
 
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
+def _ptr(t):
+    return None if t is None else t.data_ptr()
 
 
 class _LocalPSFRender(torch.autograd.Function):
@@ -19,9 +19,8 @@ class _LocalPSFRender(torch.autograd.Function):
     def forward(ctx, img, taps, ks):
         n, c, h, w = img.shape
         out = torch.empty_like(img)
-        with torch.cuda.device(img.device):
-            _nat.check(_nat.lib.aadff_local_psf_render_f32(img.data_ptr(), taps.data_ptr(), out.data_ptr(), n, c, h, w,
-                                                           ks, _stream()))
+        _nat.call("aadff_local_psf_render_f32", img.data_ptr(), taps.data_ptr(), out.data_ptr(), n, c, h, w, ks,
+                  device=img.device)
         ctx.save_for_backward(img, taps)
         ctx.ks = ks
         return out
@@ -31,16 +30,12 @@ class _LocalPSFRender(torch.autograd.Function):
     def backward(ctx, grad_out):
         img, taps = ctx.saved_tensors
         need_img, need_psf = ctx.needs_input_grad[:2]
-        if not (need_img or need_psf):
-            return None, None, None
         g = grad_out.contiguous()
         grad_img = torch.empty_like(img) if need_img else None
         grad_psf = torch.empty_like(taps) if need_psf else None
         n, c, h, w = img.shape
-        with torch.cuda.device(img.device):
-            _nat.check(_nat.lib.aadff_local_psf_render_backward_f32(
-                img.data_ptr(), taps.data_ptr(), g.data_ptr(), grad_img.data_ptr() if need_img else None,
-                grad_psf.data_ptr() if need_psf else None, n, c, h, w, ctx.ks, _stream()))
+        _nat.call("aadff_local_psf_render_backward_f32", img.data_ptr(), taps.data_ptr(), g.data_ptr(), _ptr(grad_img),
+                  _ptr(grad_psf), n, c, h, w, ctx.ks, device=img.device)
         return grad_img, grad_psf, None
 
 
@@ -77,9 +72,8 @@ class _PSFConv(torch.autograd.Function):
     def forward(ctx, x, taps, ks, grid):
         B, C, H, W = x.shape
         out = torch.zeros_like(x)            # the reference starts from zeros (rows past the last patch stay 0)
-        with torch.cuda.device(x.device):
-            _nat.check(_nat.lib.aadff_render_psf_map_f32(x.data_ptr(), taps.data_ptr(), out.data_ptr(), B, C, H, W, ks,
-                                                         grid, _bounds(grid, H), _bounds(grid, W), _stream()))
+        _nat.call("aadff_render_psf_map_f32", x.data_ptr(), taps.data_ptr(), out.data_ptr(), B, C, H, W, ks, grid,
+                  _bounds(grid, H), _bounds(grid, W), device=x.device)
         ctx.save_for_backward(x, taps)
         ctx.ks, ctx.grid = ks, grid
         return out
@@ -89,25 +83,19 @@ class _PSFConv(torch.autograd.Function):
     def backward(ctx, grad_out):
         x, taps = ctx.saved_tensors
         need_img, need_psf = ctx.needs_input_grad[:2]
-        if not (need_img or need_psf):
-            return None, None, None, None
         g = grad_out.contiguous()
         B, C, H, W = x.shape
         ks, grid = ctx.ks, ctx.grid
         hb, wb = _bounds(grid, H), _bounds(grid, W)
         grad_img = torch.empty_like(x) if need_img else None
         grad_psf = torch.empty_like(taps) if need_psf else None
-        work, work_bytes = None, 0
+        work = None         # only grad_psf_map needs a workspace
         if need_psf:
-            work_bytes = _nat.lib.aadff_render_psf_map_backward_work_bytes(B, C, H, W, ks, grid, hb, wb)
-            if work_bytes < 0:
-                _nat.check(int(work_bytes))
-            work = torch.empty((work_bytes + 3) // 4, dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _nat.check(_nat.lib.aadff_render_psf_map_backward_f32(
-                x.data_ptr(), taps.data_ptr(), g.data_ptr(), grad_img.data_ptr() if need_img else None,
-                grad_psf.data_ptr() if need_psf else None, work.data_ptr() if need_psf else None, work_bytes,
-                B, C, H, W, ks, grid, hb, wb, _stream()))
+            work = _nat.workspace(_nat.lib.aadff_render_psf_map_backward_work_bytes(B, C, H, W, ks, grid, hb, wb),
+                                  x.device)
+        _nat.call("aadff_render_psf_map_backward_f32", x.data_ptr(), taps.data_ptr(), g.data_ptr(), _ptr(grad_img),
+                  _ptr(grad_psf), _ptr(work), 0 if work is None else work.numel(), B, C, H, W, ks, grid, hb, wb,
+                  device=x.device)
         return grad_img, grad_psf, None, None
 
 

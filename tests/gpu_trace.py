@@ -22,7 +22,6 @@ def main():
     mode = sys.argv[1] if len(sys.argv) > 1 else "parity"
     ks = int(sys.argv[2]) if len(sys.argv) > 2 else 11
     nat = aadff_b200.native
-    nat.lib.aadff_debug_trace_entries.restype = int
     n = nat.lib.aadff_debug_trace_entries()
     lens = aadff_b200.PSFNet(kernel_size=ks, device="cuda", mode=mode)
     if ks == 11:
@@ -32,7 +31,6 @@ def main():
     img, dep = img.cuda(), -dm.cuda() * 1e3
     lens.render_stack(img, dep, foc)
     buf = torch.zeros(4 * n, dtype=torch.int64, device="cuda")
-    nat.lib.aadff_debug_set_trace.argtypes = [nat.ctypes.c_void_p]
     nat.lib.aadff_debug_set_trace(buf.data_ptr())
     lens.render_stack(img, dep, foc)
     torch.cuda.synchronize()
