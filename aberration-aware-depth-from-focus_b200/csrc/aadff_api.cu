@@ -37,7 +37,6 @@ namespace {
 
 thread_local std::string g_err;
 std::atomic<long long> g_launches{0};
-std::atomic<int> g_desc_swap{0};
 std::atomic<int> g_dbg_flags{0};
 std::atomic<unsigned long long*> g_trace{nullptr};
 
@@ -53,13 +52,12 @@ int fail(int code, const std::string& msg) {
             return fail(AADFF_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));      \
     } while (0)
 
-// Bits of aadff_debug_set_flags (include/aadff.h documents them).  Bit 1, the fused kernel's what-if without weight
-// copies, is read on the device (TcParams::dbg).
+// Bits of aadff_debug_set_flags (include/aadff.h documents them): cross-check paths that keep results valid, all read
+// on the host.
 constexpr int DBG_THINLENS_NO_TMA = 16;
 constexpr int DBG_ECON_PLAIN_ROUNDING = 256;
 constexpr int DBG_NO_STRIP_GATHER = 512;
 constexpr int DBG_STRIP_PLAN1 = 1024, DBG_STRIP_PLAN2 = 4096, DBG_STRIP_PLAN0 = 8192;
-constexpr int DBG_ECON_FIRST_SHIFT = 16;           // bits 16..19: first two-term group of AADFF_MODE_ECON
 constexpr int DBG_SMEM_A_OPERANDS = 1 << 20;
 
 template <int V> constexpr std::integral_constant<int, V> ic{};
@@ -381,10 +379,6 @@ extern "C" {
 int aadff_version(void) { return AADFF_VERSION; }
 const char* aadff_last_error(void) { return g_err.c_str(); }
 int64_t aadff_launch_count(void) { return g_launches.load(); }
-int aadff_debug_set_desc_swap(int swap) {
-    g_desc_swap.store(swap ? 1 : 0);
-    return AADFF_OK;
-}
 
 int aadff_debug_set_trace(void* device_buffer) {
     g_trace.store(static_cast<unsigned long long*>(device_buffer));
@@ -613,9 +607,6 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
     TermPattern tp = TERM_PATTERNS[0];
     for (const TermPattern& p : TERM_PATTERNS)
         if (p.mode == mode) tp = p;
-    // debug flags bits 16..19: first two-term group of AADFF_MODE_ECON for this launch (0 = the shipped pattern, L5 =
-    // group 4; later groups trade speed for accuracy -- tests/gpu_econ_certificate.py sweeps it)
-    if (mode == AADFF_MODE_ECON) tp.first = std::max(tp.first, (dbg >> DBG_ECON_FIRST_SHIFT) & 15);
     if (tp.first >= h->n_groups) tp = TERM_PATTERNS[0];       // no group reduced: the network runs as in parity mode
     bool any_lo = false, all2 = true, aligned = true;
     for (int i = 0; i < h->n_groups; ++i) {
@@ -643,7 +634,6 @@ static int launch_tc(aadff_psfnet_t h, RenderArgs ra, int mode, cudaStream_t st,
         P.n_tiles = (n_probes + TC_M - 1) / TC_M;
     }
     P.trace = g_trace.load();
-    P.dbg = (uint32_t)dbg;
     uint32_t halo_bytes = (uint32_t)(TC_TILE_H + ra.ks - 1) * TC_HALO_PITCH * 16;          // float4 per pixel
     if (probes != nullptr) halo_bytes = std::max<uint32_t>(halo_bytes, 8 * 32 * 9 * 4);        // pred mode: the store staging lives there
     const uint32_t bias_bytes = (uint32_t)(h->n_bias - h->head_bias0) * 4;                 // head bias only
@@ -1641,7 +1631,7 @@ int aadff_debug_umma_gemm(const float* A, const float* B, float* D, int K, int N
     CUDA_TRY(cudaMemcpy(dA, A, (size_t)128 * K * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(cudaMemcpy(dB, pack_hi.data(), pack_hi.size() * 2, cudaMemcpyHostToDevice));
     if (int rc = launch(debug_umma_gemm_kernel, 1, 128, TC_A_PART_BYTES + 131072 + 64, nullptr, dA,
-                        reinterpret_cast<const uint8_t*>(dB), dD, K, N, (uint32_t)g_desc_swap.load()))
+                        reinterpret_cast<const uint8_t*>(dB), dD, K, N))
         return rc;
     CUDA_TRY(cudaDeviceSynchronize());
     CUDA_TRY(cudaMemcpy(D, dD, (size_t)128 * N * 4, cudaMemcpyDeviceToHost));
@@ -1655,32 +1645,6 @@ int aadff_debug_econ_round(const float* W, int N, int K, const float* A, int NC,
     std::vector<float> a(A, A + (size_t)NC * K), q;
     if (!gptq_round_fp16(W, N, K, a, NC, q)) return fail(AADFF_E_INVALID, "activation covariance is not positive definite");
     std::memcpy(out, q.data(), q.size() * sizeof(float));
-    return AADFF_OK;
-}
-
-int aadff_debug_mma_timing(const int* mmas_per_commit, int n_patterns, int reps, int N, int epi_load,
-                           uint64_t* out_cycles, int device) {
-    if (!mmas_per_commit || !out_cycles || n_patterns < 1 || n_patterns > 16) return fail(AADFF_E_INVALID, "bad args");
-    DeviceGuard guard(device);
-    if (!guard.ok) return fail(AADFF_E_CUDA, "cannot select device");
-    int* d_m = nullptr;
-    unsigned long long* d_out = nullptr;
-    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d_m), n_patterns * sizeof(int)));
-    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d_out), 64 * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemcpy(d_m, mmas_per_commit, n_patterns * sizeof(int), cudaMemcpyHostToDevice));
-    uint8_t* d_src = nullptr;
-    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d_src), 65536));
-    CUDA_TRY(cudaMemset(d_src, 0, 65536));
-    CUDA_TRY(cudaMemset(d_out, 0, 64 * sizeof(unsigned long long)));
-    const int smem = TC_A_PART_BYTES + 65536 + 128;
-    CUDA_TRY(cudaFuncSetAttribute(debug_mma_timing_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    debug_mma_timing_kernel<<<1, 128, smem>>>(d_out, n_patterns, d_m, reps, N, epi_load, d_src);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaDeviceSynchronize());
-    CUDA_TRY(cudaMemcpy(out_cycles, d_out, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    cudaFree(d_src);
-    cudaFree(d_m);
-    cudaFree(d_out);
     return AADFF_OK;
 }
 

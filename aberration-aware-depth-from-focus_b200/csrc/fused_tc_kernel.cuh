@@ -97,7 +97,6 @@ struct TcParams {
     uint32_t off_bslab;     // bias-slab slot: [256 x 8] halves (K columns 0..7) + a shared [256 x 8] block of zeros (K 8..15)
     uint32_t off_stg;       // TA: raw head accumulator of the tile being gathered, [head columns / 4][128 rows] float4
     uint32_t halo_bytes;    // TA: one of the two halo slots (tile t is gathered while tile t+1's halo is fetched)
-    uint32_t dbg;           // debug flags (include/aadff.h); the kernel reads bit 0: what-if, no weight copies
     // pred mode (kernel instantiated with PRED = true): probes [M,4] in, L1-normalised PSFs [M, ks*ks] out
     const float* probes;
     float* psf_out;
@@ -124,10 +123,6 @@ struct TcTrace {
         }
     }
 };
-
-__device__ __forceinline__ uint64_t tc_desc(uint32_t addr, uint32_t lbo, uint32_t sbo, uint32_t swap) {
-    return swap ? umma_smem_desc(addr, sbo, lbo) : umma_smem_desc(addr, lbo, sbo);
-}
 
 __device__ __forceinline__ uint32_t pack_half2(float a, float b) {
     __half2 h = __floats2half2_rn(a, b);
@@ -330,12 +325,8 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                     // a compile-time constant in the specialised kernels)
                     mbar_wait(bar_bempty(), bphase ^ 1);
                     if (elect_one_sync()) {
-                        if (P.dbg & 1) {
-                            mbar_arrive(bar_bfull());
-                        } else {
-                            mbar_arrive_expect_tx(bar_bfull(), TC_BSLAB_BYTES);
-                            bulk_g2s(sbase + P.off_bslab, src, TC_BSLAB_BYTES, bar_bfull());
-                        }
+                        mbar_arrive_expect_tx(bar_bfull(), TC_BSLAB_BYTES);
+                        bulk_g2s(sbase + P.off_bslab, src, TC_BSLAB_BYTES, bar_bfull());
                     }
                     __syncwarp();
                     bphase ^= 1;
@@ -351,9 +342,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
                         tr.ev(0x100 + gi);                       // stage load issued
                         if (part == 0) pair_bar = bar_full(stage);
                         if (elect_one_sync()) {
-                            if (P.dbg & 1) {                     // what-if: no copies (lo stages of a pair have no barrier use)
-                                if (!(nparts == 2 && P.n_stages >= 4 && part == 1)) mbar_arrive(bar_full(stage));
-                            } else if (nparts == 2 && P.n_stages >= 4) {
+                            if (nparts == 2 && P.n_stages >= 4) {
                                 if (part == 0) mbar_arrive_expect_tx(pair_bar, 2 * bytes);
                                 bulk_g2s(stage_addr(stage), src + (size_t)(it * 2 + part) * bytes, bytes, pair_bar);
                             } else {
@@ -1055,7 +1044,7 @@ __global__ void __launch_bounds__(TC_NT, 1) fused_psfnet_render_kernel(const __g
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128, 1)
 debug_umma_gemm_kernel(const float* __restrict__ A, const uint8_t* __restrict__ bpack, float* __restrict__ D,
-                       int K, int N, uint32_t swap) {
+                       int K, int N) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1086,8 +1075,8 @@ debug_umma_gemm_kernel(const float* __restrict__ A, const uint8_t* __restrict__ 
         const uint32_t lbo_b = (uint32_t)N * 16;
         for (int ks16 = 0; ks16 < K / 16; ++ks16) {
             const uint32_t slab = b_sm + (ks16 / 2) * (N * 64);
-            umma_f16_ss(tmem_base, tc_desc(a_hi + ks16 * 2 * TC_A_LBO, TC_A_LBO, 128, swap),
-                        tc_desc(slab + (ks16 & 1) * 2 * lbo_b, lbo_b, 128, swap), idesc, ks16 > 0);
+            umma_f16_ss(tmem_base, umma_smem_desc(a_hi + ks16 * 2 * TC_A_LBO, TC_A_LBO, 128),
+                        umma_smem_desc(slab + (ks16 & 1) * 2 * lbo_b, lbo_b, 128), idesc, ks16 > 0);
         }
         umma_commit(bar);
     }
@@ -1104,116 +1093,6 @@ debug_umma_gemm_kernel(const float* __restrict__ A, const uint8_t* __restrict__ 
     tc_fence_before_sync();
     __syncthreads();
     if (warp == 0) tmem_dealloc<256>(tmem_base);
-}
-
-
-// ------------------------------------------------------------------------------------------
-// Debug microbenchmark: cost of issuing tcgen05.mma / tcgen05.commit from one converged warp.
-// Pattern p: `reps` x [ mmas_per_commit[p] MMAs (M128 x N x K16, smem operands) ; commit ].
-// out[p*2+0] = cycles until the issuing thread is done, out[p*2+1] = cycles until all MMAs retired.
-// ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128, 1)
-debug_mma_timing_kernel(unsigned long long* out, int n_patterns, const int* mmas_per_commit, int reps, int N,
-                        int epi_load, const uint8_t* __restrict__ gsrc) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t sbase = smem_u32(smem);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t a_sm = sbase, b_sm = sbase + TC_A_PART_BYTES;
-    const uint32_t bar_done = sbase + TC_A_PART_BYTES + 65536, bar_slab = bar_done + 8;
-    volatile uint32_t* slot = reinterpret_cast<volatile uint32_t*>(smem + TC_A_PART_BYTES + 65536 + 32);
-    for (int i = threadIdx.x; i < (TC_A_PART_BYTES + 65536) / 4; i += 128) reinterpret_cast<uint32_t*>(smem)[i] = 0;
-    // epi_load: low 16 bits = competing TMEM reads; bit 16 = warp 1 streams 16 KB bulk copies (3 in flight)
-    // into smem like the weight producer; bit 17 = warps 2-3 stream 16-byte st.shared like the epilogue.
-    const int tmem_reads = epi_load & 0xFFFF;
-    const bool do_copy = (epi_load >> 16) & 1, do_sts = (epi_load >> 17) & 1;
-    const uint32_t bar_copy = bar_done + 64;                 // 4 barriers
-    volatile uint32_t* stop = slot + 1;
-    if (threadIdx.x == 0) {
-        mbar_init(bar_done, 1); mbar_init(bar_slab, 1);
-        for (int i = 0; i < 4; ++i) mbar_init(bar_copy + 8 * i, 1);
-        fence_mbar_init();
-    }
-    if (warp == 0) tmem_alloc<512>(smem_u32(const_cast<uint32_t*>(slot)));
-    fence_proxy_async_smem();
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem_base = *slot;
-    uint32_t done_phase = 0, cph = 0;
-    for (int p = 0; p < n_patterns; ++p) {
-        const int m = mmas_per_commit[p];
-        if (threadIdx.x == 0) *stop = 0;
-        __syncthreads();
-        if (warp == 0) {
-            const uint32_t idesc = umma_idesc_f16_f32(128, N);
-            const uint64_t da = umma_smem_desc(a_sm, TC_A_LBO, 128);
-            const uint64_t db = umma_smem_desc(b_sm, (uint32_t)N * 16, 128);
-            const long long t0 = clock64();
-            for (int r = 0; r < reps; ++r) {
-                if (elect_one_sync()) {
-                    for (int i = 0; i < m; ++i)
-                        umma_f16_ss(tmem_base, da + (uint32_t)((r * m + i) & 15) * 256u,
-                                    db + (uint32_t)(i & 1) * (uint32_t)(2 * N), idesc, 1);
-                    umma_commit(bar_slab);
-                }
-                __syncwarp();
-            }
-            if (elect_one_sync()) umma_commit(bar_done);
-            __syncwarp();
-            const long long t1 = clock64();
-            mbar_wait(bar_done, done_phase);
-            const long long t2 = clock64();
-            if (lane == 0) { out[p * 2] = t1 - t0; out[p * 2 + 1] = t2 - t0; *stop = 1; }
-        } else if (warp == 1 && do_copy) {
-            // 16 KB copies into the upper 48 KB of the B region, three in flight; `cph` (one parity bit per barrier)
-            // lives across patterns, and every copy is waited for before the pattern ends
-            unsigned long long n = 0;
-            if (lane == 0) {
-                for (int i = 0; i < 3; ++i) {
-                    mbar_arrive_expect_tx(bar_copy + 8 * i, 16384);
-                    bulk_g2s(b_sm + 16384 + 16384 * i, gsrc + 16384 * i, 16384, bar_copy + 8 * i);
-                }
-                while (!*stop) {
-                    for (int i = 0; i < 3; ++i) {
-                        mbar_wait(bar_copy + 8 * i, (cph >> i) & 1);
-                        cph ^= 1u << i;
-                        mbar_arrive_expect_tx(bar_copy + 8 * i, 16384);
-                        bulk_g2s(b_sm + 16384 + 16384 * i, gsrc + 16384 * i, 16384, bar_copy + 8 * i);
-                        ++n;
-                    }
-                }
-                for (int i = 0; i < 3; ++i) {
-                    mbar_wait(bar_copy + 8 * i, (cph >> i) & 1);
-                    cph ^= 1u << i;
-                }
-                out[32 + p] = n * 16384ull;
-            }
-            __syncwarp();
-        } else if (warp >= 2 && do_sts) {
-            unsigned long long n = 0;
-            const uint32_t dst = a_sm + 32768 + (uint32_t)(threadIdx.x - 64) * 16;
-            while (!*stop) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i)
-                    asm volatile("st.shared.v4.u32 [%0], {%1,%1,%1,%1};" :: "r"(dst + (uint32_t)i * 1024u), "r"(0u) : "memory");
-                n += 8;
-            }
-            if (threadIdx.x == 64) out[48 + p] = n * 64ull * 16ull;
-        } else if (tmem_reads) {
-            // competing TMEM reads from the other accumulator half, like a concurrent epilogue
-            uint32_t rr[32];
-            for (int it = 0; it < tmem_reads; ++it) {
-                tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + 256 + (it & 7) * 32, rr);
-                tmem_ld_wait();
-            }
-            if (rr[0] == 0x12345678u) out[63] = rr[1];
-        }
-        done_phase ^= 1;
-        tc_fence_before_sync();
-        __syncthreads();
-        tc_fence_after_sync();
-    }
-    if (warp == 0) tmem_dealloc<512>(tmem_base);
 }
 
 }  // namespace aadff

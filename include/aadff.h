@@ -242,32 +242,25 @@ int aadff_trainer_destroy(aadff_trainer_t t);
 int64_t aadff_launch_count(void);
 
 /* Test hooks (used by tests/ only): a single-tile tcgen05 GEMM through the same operand
- * packing, descriptors and TMEM read-back as the fused kernel (host pointers, synchronous),
- * and the descriptor-convention probe it controls.                                            */
+ * packing, descriptors and TMEM read-back as the fused kernel (host pointers, synchronous). */
 int aadff_debug_umma_gemm(const float* A, const float* B, float* D, int K, int N, int device);
-int aadff_debug_set_desc_swap(int swap);
 /* Event trace of CTA 0 of the fused kernel: device buffer of 4 * aadff_debug_trace_entries()
  * uint64 (zero-filled by the caller), NULL switches tracing off.  See tests/gpu_trace.py.    */
 int aadff_debug_set_trace(void* device_buffer);
 int aadff_debug_trace_entries(void);
-/* Debug switches, 0 restores normal operation.  What-if timing of the fused kernel (results become invalid):
- * 1 = skip the weight copies.  16 = aadff_thinlens_render_f32 fetches every halo tile with clamped cp.async instead of
- * TMA tensor tiles for interior tiles (results unchanged).  Cross-check paths (results stay valid): 256 =
- * AADFF_MODE_ECON with plainly rounded fp16 weights instead of the calibrated ones, 512 = aadff_local_psf_render_f32
- * through the register-streaming kernel also where the strip-walking kernel would run (ks <= 15, W % 4 == 0);
- * 8192 / 1024 / 4096 = the strip-walking kernel with its shared-memory plan 0 / 1 / 2 forced (default: the widest
- * strips that divide W well).  Bits 16..19 (value g > 4): AADFF_MODE_ECON starts its two-term evaluation at layer group
- * g instead of 4 (L5) -- accuracy / speed sweep, generic kernel.  1 << 20 = the fused kernel keeps its A operands in
- * shared memory also where it would keep them in tensor memory (results unchanged).                                 */
+/* Debug switches, 0 restores normal operation.  Each selects a cross-check path; results stay valid:
+ *   16 = aadff_thinlens_render_f32 fetches every halo tile with clamped cp.async instead of TMA tensor tiles for
+ *        interior tiles;
+ *   256 = AADFF_MODE_ECON with plainly rounded fp16 weights instead of the calibrated ones;
+ *   512 = aadff_local_psf_render_f32 through the register-streaming kernel also where the strip-walking kernel would
+ *        run (ks <= 15, W % 4 == 0);
+ *   8192 / 1024 / 4096 = the strip-walking kernel with its shared-memory plan 0 / 1 / 2 forced (default: the widest
+ *        strips that divide W well);
+ *   1 << 20 = the fused kernel keeps its A operands in shared memory also where it would keep them in tensor memory. */
 int aadff_debug_set_flags(int flags);
 /* Host-only: the output-error-calibrated fp16 rounding used by AADFF_MODE_ECON (csrc/econ_calib.h) for one layer.
  * W [N][K], A [NC][K] = sample input activations of the layer, out [N][K] = fp16-representable values.  No GPU. */
 int aadff_debug_econ_round(const float* W, int N, int K, const float* A, int NC, float* out);
-/* Issue-cost microbenchmark of tcgen05.mma / tcgen05.commit (see tests/gpu_diag.py mma_timing);
- * epi_load: low 16 bits = competing TMEM reads, bit 16 = competing bulk copies into smem, bit 17 =
- * competing st.shared stream.  out_cycles must hold 64 entries.                                   */
-int aadff_debug_mma_timing(const int* mmas_per_commit, int n_patterns, int reps, int N, int epi_load,
-                           uint64_t* out_cycles, int device);
 
 #ifdef __cplusplus
 }

@@ -19,20 +19,17 @@ def stage_umma():
     import aadff_b200
     nat = aadff_b200.native
     rng = np.random.default_rng(0)
-    for swap in (0, 1):
-        nat.lib.aadff_debug_set_desc_swap(swap)
-        for K, N in [(32, 16), (64, 256), (256, 256), (256, 128), (256, 208)]:
-            A = rng.standard_normal((128, K)).astype(np.float32)
-            B = rng.standard_normal((N, K)).astype(np.float32)
-            D = np.zeros((128, N), np.float32)
-            rc = nat.lib.aadff_debug_umma_gemm(A.ctypes.data, B.ctypes.data, D.ctypes.data, K, N, 0)
-            if rc:
-                print(f"swap={swap} K={K} N={N}: rc={rc} {nat.lib.aadff_last_error().decode()}")
-                continue
-            ref = A.astype(np.float16).astype(np.float32) @ B.astype(np.float16).astype(np.float32).T
-            err = np.abs(D - ref).max()
-            print(f"swap={swap} K={K} N={N}: max|D-ref|={err:.3e}  (|ref|max={np.abs(ref).max():.2f})", flush=True)
-    nat.lib.aadff_debug_set_desc_swap(0)
+    for K, N in [(32, 16), (64, 256), (256, 256), (256, 128), (256, 208)]:
+        A = rng.standard_normal((128, K)).astype(np.float32)
+        B = rng.standard_normal((N, K)).astype(np.float32)
+        D = np.zeros((128, N), np.float32)
+        rc = nat.lib.aadff_debug_umma_gemm(A.ctypes.data, B.ctypes.data, D.ctypes.data, K, N, 0)
+        if rc:
+            print(f"K={K} N={N}: rc={rc} {nat.lib.aadff_last_error().decode()}")
+            continue
+        ref = A.astype(np.float16).astype(np.float32) @ B.astype(np.float16).astype(np.float32).T
+        err = np.abs(D - ref).max()
+        print(f"K={K} N={N}: max|D-ref|={err:.3e}  (|ref|max={np.abs(ref).max():.2f})", flush=True)
 
 
 def _lens(ks=11, mode="parity"):
@@ -67,18 +64,16 @@ def stage_fp32():
     _check("gather kat_d_0", out, torch.from_numpy(g["out"]))
 
 
-def _tc(mode, swap=0):
+def _tc(mode):
     import torch
-    import aadff_b200
     from conftest import analytic_rgbd, load_golden
-    aadff_b200.native.lib.aadff_debug_set_desc_swap(swap)
     lens = _lens(mode=mode)
     for N, H, W in [(1, 48, 64), (2, 64, 64)]:
         g = load_golden(f"kat_b_{N}x{H}x{W}.npz")
         img, dm = analytic_rgbd(N, H, W)
         out = lens.render(img.cuda(), -dm.cuda() * 1e3, torch.from_numpy(g["foc"]).cuda())
         torch.cuda.synchronize()
-        _check(f"{mode} (swap={swap}) render kat_b {N}x{H}x{W}", out, torch.from_numpy(g["out"]))
+        _check(f"{mode} render kat_b {N}x{H}x{W}", out, torch.from_numpy(g["out"]))
     g = load_golden("kat_e_stack_2x40x56.npz")
     out = lens.render_stack(torch.from_numpy(g["img"]).cuda(), -torch.from_numpy(g["depth_m"]).cuda() * 1e3,
                             -torch.from_numpy(g["foc_m"]).cuda() * 1e3)
@@ -87,10 +82,6 @@ def _tc(mode, swap=0):
 
 def stage_tc_parity():
     _tc("parity")
-
-
-def stage_tc_parity_swap():
-    _tc("parity", swap=1)
 
 
 def stage_tc_fast():
@@ -224,53 +215,6 @@ def stage_speed():
                   flush=True)
 
 
-def stage_whatif():
-    """Timing with parts of the kernel switched off (results invalid) to locate the bottleneck."""
-    import torch
-    import aadff_b200
-    from oracle import focal_stack_oracle as orc
-    nat = aadff_b200.native
-    img, dm = orc.synthetic_rgbd(1, 512, 512, seed=1234)
-    foc = -orc.synthetic_focus(dm, 5).cuda() * 1e3
-    img, dep = img.cuda(), -dm.cuda() * 1e3
-    for mode in ("parity", "fast"):
-        lens = _lens(mode=mode)
-        for flags in (0, 1):
-            nat.lib.aadff_debug_set_flags(flags)
-            for _ in range(2):
-                lens.render_stack(img, dep, foc)
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(10):
-                lens.render_stack(img, dep, foc)
-            e1.record()
-            torch.cuda.synchronize()
-            print(f"whatif {mode} flags={flags}: {e0.elapsed_time(e1) / 10:.3f} ms", flush=True)
-    nat.lib.aadff_debug_set_flags(0)
-
-
-def stage_mma_timing():
-    import ctypes
-    import numpy as np
-    import aadff_b200
-    nat = aadff_b200.native
-    pats = np.array([1, 2, 4, 6, 8, 16, 64], dtype=np.int32)
-    reps = 16
-    # epi_load: low 16 bits = competing TMEM reads, bit 16 = bulk copies into smem, bit 17 = st.shared stream
-    for N in (256, 128):
-        for epi in (0, 4000, 1 << 16, 1 << 17, 3 << 16):
-            out = np.zeros(64, dtype=np.uint64)
-            nat.check(nat.lib.aadff_debug_mma_timing(ctypes.c_void_p(pats.ctypes.data), len(pats), reps, N, epi,
-                                                     ctypes.c_void_p(out.ctypes.data), 0))
-            for i, m in enumerate(pats):
-                tot = int(m) * reps
-                cyc = float(out[2 * i + 1])
-                print(f"N={N} epi_load={epi:#x} [{m:2d} MMA + commit] x{reps}: issue {out[2*i]/tot:7.1f} cyc/MMA, "
-                      f"retire {out[2*i+1]/tot:7.1f} cyc/MMA; competing copy {out[32+i]/cyc:5.1f} B/clk, "
-                      f"st.shared {out[48+i]/cyc:5.1f} B/clk", flush=True)
-
-
 def stage_rows():
     """Throughput of the stand-alone rows: local_psf_render (HBM-bound on the PSF read) and pred."""
     import torch
@@ -394,7 +338,7 @@ if __name__ == "__main__":
     if len(sys.argv) > 2 and sys.argv[1] == "--run":
         STAGES[sys.argv[2]]()
         sys.exit(0)
-    names = sys.argv[1:] or ["umma", "fp32", "tc_parity", "tc_fast", "tc_ks31", "speed", "rows", "mma_timing", "econ"]
+    names = sys.argv[1:] or ["umma", "fp32", "tc_parity", "tc_fast", "tc_ks31", "speed", "rows", "econ"]
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     log = open(os.path.join(ROOT, "gpurun_out", "diag.log"), "a")
     for name in names:

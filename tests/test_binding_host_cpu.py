@@ -20,11 +20,16 @@ def nat():
     return aadff_b200.native
 
 
-def header_prototypes():
-    """[(return type, name, [parameter declarations])], read statement by statement from the header."""
+def header_text():
+    """include/aadff.h without comments and preprocessor lines."""
     with open(os.path.join(ROOT, "include", "aadff.h")) as f:
         text = re.sub(r"/\*.*?\*/", "", f.read(), flags=re.S)
-    text = "\n".join(line for line in text.splitlines() if not line.lstrip().startswith("#"))
+    return "\n".join(line for line in text.splitlines() if not line.lstrip().startswith("#"))
+
+
+def header_prototypes():
+    """[(return type, name, [parameter declarations])], read statement by statement from the header."""
+    text = header_text()
     protos = []
     for stmt in text.split(";"):
         if "(" not in stmt:
@@ -39,10 +44,12 @@ def header_prototypes():
     return protos
 
 
-def test_argtypes_and_restype_follow_the_header(nat):
+def test_argtypes_and_restype_follow_every_header_prototype(nat):
     protos = header_prototypes()
-    assert sorted(name for _, name, _ in protos) == nat.exported_symbols()
-    assert len(protos) >= 39
+    names = sorted(name for _, name, _ in protos)
+    assert names == nat.exported_symbols()
+    # every function the header declares, found by a plain scan: neither parse may drop a prototype
+    assert names == sorted(set(re.findall(r"\b(aadff_\w+)\s*\(", header_text()))) and "aadff_version" in names
     for ret, name, params in protos:
         fn = getattr(nat.lib, name)
         assert fn.restype is RETURNS[ret], (name, ret, fn.restype)
